@@ -2,7 +2,7 @@
 """Headline benchmark: all-observation infinitesimal-jackknife sensitivities for
 logistic regression, N = 10M, D = 1024, float64 (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" is the whole hot path over the whole data set:
     GLM statistics pass  ->  H = X^T diag(s) X  (-> all-reduce of H)  ->
@@ -67,7 +67,18 @@ def parse():
     ap.add_argument('--engine-rows-only', action='store_true', help=argparse.SUPPRESS)   # child mode, see main()
     ap.add_argument('--engines', action='store_true', help='also measure the other engines when --gpus > 1 '
                     '(by default they are measured on 1 GPU only)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed as float64 .npy files in DIR: '
+                         'hessian_at_opt (D, D) and dopt_dhyper_sample, the columns of the (D, N) sensitivities at a '
+                         'fixed seeded sample of observations (see dump_outputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
+    if args.dump_outputs and dump_columns(args.n_total, args.dim) < 1:
+        ap.error('--dump-outputs: the {0} x {0} Hessian alone exceeds {1} bytes'.format(args.dim, DUMP_BYTES))
+    return args
 
 
 # ---------------------------------------------------------------------------
@@ -292,7 +303,8 @@ def main():
     barrier()
     e0.record()
     for _ in range(args.steps):
-        s_ = one_step(); del s_
+        s_ = None             # release the previous step's (D, N) result before the next one is allocated
+        s_ = one_step()
     e1.record()
     barrier()
     launches = ops.launch_count() - launches0
@@ -302,6 +314,9 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_per_step = float(ms.item()) / args.steps
     value = N / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s_, torch, dist, world, rank, r0, N, dev)
+    del s_
 
     # ---- per-kernel timing (same stream, CUDA events) -> roofline ------------
     def timed(fn, reps):
@@ -633,6 +648,35 @@ def engine_row(prec, vt, ops, torch, dist, world, group, dev, X, y, theta, w, st
     t_sy, _h = timed(lambda: ops.syrk_weighted(X, st['s'], precision=prec), reps)
     row.update({'syrk_ms': t_sy, 'syrk_fp64_equiv_tflops_algorithmic': float(D) * (D + 1) * n_loc / (t_sy * 1e-3) / 1e12})
     return row
+
+
+DUMP_BYTES = 60 << 20          # the whole --dump-outputs directory stays under 64 MB
+DUMP_MAX_COLUMNS = 4096
+
+
+def dump_columns(n, d):
+    """How many columns of the (D, N) sensitivity matrix --dump-outputs keeps: all up to 4096, fewer when D is so
+    wide that they and the D x D Hessian would not fit in DUMP_BYTES."""
+    return min(n, DUMP_MAX_COLUMNS, (DUMP_BYTES - 8 * d * d) // (8 * d))
+
+
+def dump_outputs(out_dir, sens, torch, dist, world, rank, r0, n, dev):
+    """--dump-outputs: what the caller of the last timed step receives, in float64.  hessian_at_opt.npy is the whole
+    D x D Hessian; dopt_dhyper_sample.npy holds the columns of the (D, N) sensitivity matrix at dump_columns(N, D)
+    observations drawn without replacement by numpy's RandomState(SEED), in increasing order, gathered from the ranks
+    that hold them.  The inputs depend only on the arguments, so two builds can be compared file by file."""
+    S = sens.get_dopt_dhyper()                   # this rank's (D, n_loc) block, on the device
+    d, n_loc = S.shape
+    cols = np.sort(np.random.RandomState(SEED).choice(n, dump_columns(n, d), replace=False))
+    mine = (cols >= r0) & (cols < r0 + n_loc)
+    sample = torch.zeros((d, len(cols)), dtype=torch.float64, device=dev)
+    sample[:, torch.from_numpy(np.flatnonzero(mine)).to(dev)] = S[:, torch.from_numpy(cols[mine] - r0).to(dev)]
+    if world > 1:
+        dist.all_reduce(sample)                  # every column comes from exactly one rank; the others add zeros
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, 'hessian_at_opt.npy'), sens.get_hessian_at_opt().double().cpu().numpy())
+        np.save(os.path.join(out_dir, 'dopt_dhyper_sample.npy'), sample.cpu().numpy())
 
 
 def memlog(tag):

@@ -7,7 +7,7 @@ timed CPU baseline.  ``vittles_b200`` never imports it: the product path fails
 loudly when its CUDA library is missing.
 
 What it is: a float64 restatement of the reference's algorithms
-(``/root/reference/vittles``), module by module, with
+(the ``vittles`` package of rgiordan/vittles), module by module, with
 ``autograd.{grad,jacobian,hessian,make_jvp}`` replaced by
 ``torch.func.{grad,jacrev,hessian,jvp}`` on CPU and the reference's scipy calls
 (``cho_factor``/``cho_solve``, ``factorized``, ``cg``) kept verbatim.  Each
@@ -15,7 +15,7 @@ function cites the reference ``file:line`` it follows.
 
 Pinning (SURVEY.md section 8c): the reference itself cannot be imported here
 (``autograd``/``paragami`` are not installed).  ``oracle/make_golden.py`` runs
-the UNMODIFIED reference sources from ``/root/reference`` on top of the
+the UNMODIFIED reference sources from a checkout of it on top of the
 ``oracle/refshim`` stand-ins for those two packages, checks this restatement
 against the reference's outputs, and stores them under ``tests/golden/``.
 The reference's own closed-form test fixtures (QuadraticModel, MVN KL, block

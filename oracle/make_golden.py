@@ -1,19 +1,19 @@
 #!/usr/bin/env python3
 """Generate ``tests/golden/*.npz`` by running the UNMODIFIED reference.
 
-TEST INFRASTRUCTURE ONLY.  Run in the build container (it needs
-``/root/reference``; the GPU box does not have it, which is why the outputs are
-committed):
+TEST INFRASTRUCTURE ONLY.  It needs a checkout of the reference
+(rgiordan/vittles, the directory that holds the ``vittles`` package); the
+tests do not, which is why the outputs are committed:
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py PATH/TO/VITTLES_CHECKOUT
 
 How the reference runs here: ``autograd`` and ``paragami`` are not installed,
 so ``oracle/refshim`` provides ``torch.func``-backed stand-ins for the handful
 of names the reference imports, and ``scipy.sparse.linalg.cg`` is wrapped to
 accept the removed ``atol='legacy'`` (``solver_lib.py:93``) with its documented
 meaning (``rtol=tol, atol=0``).  The reference's SOURCE is untouched: every
-golden value below is produced by ``vittles.*`` code imported from
-``/root/reference``.  Each case is also evaluated with the oracle restatement
+golden value below is produced by ``vittles.*`` code imported from that
+checkout.  Each case is also evaluated with the oracle restatement
 and the two must agree to 1e-12 relative before anything is written.
 """
 import os
@@ -29,9 +29,12 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 OUT = os.path.join(ROOT, 'tests', 'golden')
+if len(sys.argv) != 2:
+    sys.exit('usage: python oracle/make_golden.py PATH/TO/VITTLES_CHECKOUT')
+REF = os.path.abspath(sys.argv[1])
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(HERE, 'refshim'))
-sys.path.insert(0, '/root/reference')
+sys.path.insert(0, REF)
 
 # ---- environment shim for the removed scipy keyword (not a source change) ----
 _scipy_cg = sp.sparse.linalg.cg
@@ -47,14 +50,14 @@ def _cg_legacy(A, b, x0=None, tol=None, maxiter=None, M=None, callback=None, ato
 
 sp.sparse.linalg.cg = _cg_legacy
 
-import vittles  # noqa: E402  (the reference, from /root/reference)
+import vittles  # noqa: E402  (the reference, from REF)
 from vittles import solver_lib as ref_solver_lib  # noqa: E402
 from vittles import sensitivity_lib as ref_sens  # noqa: E402
 
 import oracle  # noqa: E402
 from oracle import models, fixtures, bivariate  # noqa: E402,F401
 
-assert vittles.__file__.startswith('/root/reference'), vittles.__file__
+assert vittles.__file__.startswith(REF + os.sep), vittles.__file__
 
 
 def close(a, b, what, rtol=1e-12):

@@ -1,7 +1,7 @@
 """Stand-in for HIPS ``autograd`` backed by ``torch.func`` (float64, CPU).
 
-TEST INFRASTRUCTURE ONLY.  ``autograd`` is not installed in this image, so the
-unmodified reference (``/root/reference/vittles``) cannot be imported as is.
+TEST INFRASTRUCTURE ONLY.  Without ``autograd`` installed, the unmodified
+reference (the ``vittles`` package of rgiordan/vittles) cannot be imported as is.
 ``oracle/make_golden.py`` puts this directory on ``sys.path`` so that the
 reference's own code runs here and its outputs can be stored as golden
 fixtures under ``tests/golden/``.  Nothing in ``vittles_b200`` imports this.

@@ -235,3 +235,21 @@ def test_bench_host_memory_accounting():
     assert bench.host_reserve_bytes() >= 16 * GB
     room = bench.host_headroom_bytes()
     assert room is None or room > 0
+    # --dump-outputs: the headline shape keeps 4096 sampled columns, and no accepted --dim goes over 64 MB
+    assert bench.dump_columns(10_000_000, 1024) == 4096 and bench.dump_columns(1000, 16) == 1000
+    for d in (1, 1024, 2048, 2700, 2800):
+        k = bench.dump_columns(10_000_000, d)
+        assert k < 1 or 8 * d * (d + k) + 2 * 128 <= 64 * 10 ** 6
+
+
+def test_bench_rejects_bad_arguments(tmp_path):
+    """--steps is the number of timed steps, so at least one; --dump-outputs belongs to the GPU path and needs room
+    for the Hessian.  Each is refused before any work starts."""
+    import subprocess
+    import sys
+    for extra in (['--steps', '0'], ['--impl', 'reference', '--dump-outputs', str(tmp_path)],
+                  ['--dim', '4096', '--dump-outputs', str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, capture_output=True, text=True,
+                             timeout=120)
+        assert out.returncode == 2 and 'error:' in out.stderr, (extra, out.stderr[-300:])
+    assert os.listdir(str(tmp_path)) == []
