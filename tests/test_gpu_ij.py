@@ -221,22 +221,25 @@ def test_quadratic_model_through_patterns_vs_golden(vt, golden, key):
 
 def test_streamed_host_input_matches_resident(vt):
     """Pinned host X goes through the chunked-copy path (copies overlapped with
-    the statistics + Hessian sweep); results must equal the resident path."""
+    the statistics + Hessian sweep); results must equal the resident path.  With odd D and n = 4100 the chunk that
+    starts at row 1025 begins 8 bytes off the 16-byte alignment: the statistics pass stages it with plain loads."""
     from oracle import models
-    n, d = 4096, 64
-    X, y, _ = models.synth_logistic(3, n, d)
-    w = np.random.RandomState(0).uniform(0.5, 1.5, size=n)
-    theta = models.glm_newton(X, y, w, l2=0.2)
-    Xh = torch.as_tensor(X).pin_memory()
-    obj_s = vt.objectives.GLMObjective(Xh, y, l2=0.2, stream_chunks=8)
-    assert obj_s._host_src is not None
-    sens_s = vt.HyperparameterSensitivityLinearApproximation(obj_s, theta, w, validate_optimum=True)
-    assert not obj_s._pending and obj_s._host_src is None
-    sens_r = vt.HyperparameterSensitivityLinearApproximation(vt.objectives.GLMObjective(X, y, l2=0.2), theta, w)
-    assert_close(sens_s.get_hessian_at_opt(), sens_r.get_hessian_at_opt(), rtol=1e-12)
-    assert_close(sens_s.get_dopt_dhyper(), sens_r.get_dopt_dhyper(), rtol=1e-9, atol_scale=1e-13)
-    cf = models.glm_closed_form(X, y, theta, w, l2=0.2)
-    assert_close(sens_s.get_dopt_dhyper(), -np.linalg.solve(cf['hessian'], cf['cross_hessian']))
+    for n, d in ((4096, 64), (4100, 65)):
+        X, y, _ = models.synth_logistic(3, n, d)
+        w = np.random.RandomState(0).uniform(0.5, 1.5, size=n)
+        theta = models.glm_newton(X, y, w, l2=0.2)
+        Xh = torch.as_tensor(X).pin_memory()
+        obj_s = vt.objectives.GLMObjective(Xh, y, l2=0.2, stream_chunks=8)
+        assert obj_s._host_src is not None
+        if d % 2:
+            assert any((obj_s.X[r0:].data_ptr() % 16) == 8 for r0 in (n * c // 8 for c in range(8)))
+        sens_s = vt.HyperparameterSensitivityLinearApproximation(obj_s, theta, w, validate_optimum=True)
+        assert not obj_s._pending and obj_s._host_src is None
+        sens_r = vt.HyperparameterSensitivityLinearApproximation(vt.objectives.GLMObjective(X, y, l2=0.2), theta, w)
+        assert_close(sens_s.get_hessian_at_opt(), sens_r.get_hessian_at_opt(), rtol=1e-12)
+        assert_close(sens_s.get_dopt_dhyper(), sens_r.get_dopt_dhyper(), rtol=1e-9, atol_scale=1e-13)
+        cf = models.glm_closed_form(X, y, theta, w, l2=0.2)
+        assert_close(sens_s.get_dopt_dhyper(), -np.linalg.solve(cf['hessian'], cf['cross_hessian']))
 
 
 @pytest.mark.parametrize('kappa', [1e2, 1e6, 1e9])

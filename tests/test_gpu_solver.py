@@ -60,7 +60,8 @@ def test_not_positive_definite_raises(vt):
         vt.solver_lib.get_dense_cholesky_solver(h)
 
 
-@pytest.mark.parametrize('d,k', [(1, 1), (7, 3), (128, 5), (129, 130), (300, 1), (1024, 64), (1500, 257)])
+@pytest.mark.parametrize('d,k', [(1, 1), (7, 3), (128, 5), (129, 130), (300, 1), (1024, 64), (1500, 257), (1023, 9),
+                                 (1025, 1300), (2049, 1100)])
 def test_cholesky_vs_scipy(vt, d, k):
     rng = np.random.RandomState(d * 7 + k)
     a = rng.normal(size=(d, d + 5))

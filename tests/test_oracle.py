@@ -239,3 +239,30 @@ def test_extended_precision_oracle_agrees_with_scipy_when_well_conditioned():
     G_ld = ((1 / (1 + np.exp(-(X.astype(np.longdouble) @ theta.astype(np.longdouble)))) - y)[:, None] * X).T
     resid = np.abs(H_ld @ S_ld + G_ld).max() / np.abs(G_ld).max()
     assert float(resid) < 1e-17
+
+
+def test_integer_designs_are_exact_in_float64_and_in_the_int8_model():
+    """oracle/exact.py: on the integer designs float64 is exact (numpy's BLAS product equals the Python-integer
+    product), the largest shapes the GPU tests use stay below 2^53, and the INT8 engine's arithmetic model reproduces
+    the exact product too - so the GPU tests may demand torch.equal of every engine."""
+    from oracle import exact, slicing
+    assert exact.hessian_bound(exact.MAX_N) < exact.EXACT_LIMIT
+    assert exact.apply_bound(exact.MAX_D) < exact.EXACT_LIMIT
+    for n, d in [(300, 37), (1001, 64)]:
+        X = exact.integer_design(1, n, d)
+        s = exact.square_weights(2, n)
+        r = exact.integer_vector(3, n)
+        Hinv = exact.integer_design(4, d, d, vmax=exact.HMAX)
+        assert np.abs(X).max() == exact.XMAX and np.abs(r).max() == exact.RMAX and np.all(np.sqrt(s) % 1 == 0)
+        H = (X * s[:, None]).T @ X
+        S = -Hinv @ (X * r[:, None]).T
+        assert np.array_equal(H.astype(np.int64).astype(object), exact.weighted_gram_int(X, s))
+        assert np.array_equal(S.astype(np.int64).astype(object), exact.apply_int(Hinv, X, r))
+        # the engine's model: the transposed weighted operand of the Hessian, the residual folded into the scale
+        W = (X * np.sqrt(s)[:, None]).T.copy()
+        dW, sW = slicing.slice_rows(W, 7)
+        assert np.array_equal(slicing.digits_gemm(dW, sW, dW, sW), H)
+        assert np.all(dW[2:] == 0)                            # two digits carry every entry: nothing is dropped
+        dH, sH = slicing.slice_rows(Hinv, 7)
+        dX, sX = slicing.slice_rows(X, 7)
+        assert np.array_equal(-slicing.digits_gemm(dH, sH, dX, sX * r), S)
