@@ -117,6 +117,16 @@ size_t vt_glm_dirderiv_workspace_bytes(int64_t N, int D);
 int vt_glm_dirderiv(const double* X, int64_t ldx, int64_t N, int D, const double* z, const double* w, int family,
                     const double* dirs, int q, double* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Per-observation influence on quantities of interest -----------------
+ * out[k * ldo + n] = alpha * c[n] * (x_n . V[k, :]) for k < K, n < N: with c = resid, V = rows of H^{-1} A^T and
+ * alpha = -1, row k of out is a_k^T S, the influence of every observation on the quantity of interest a_k, without
+ * forming S (D x N).  One pass over X (ldx >= D), K values written per row, no workspace; V (K x D) row-major and
+ * contiguous, out (K x N) row-major with ldo >= N.  K <= vt_glm_influence_max_directions(D): 8 up to D = 2048, 2 up
+ * to 4096, 1 up to 8192, 0 beyond (D > 8192 is refused with VT_ERR_INVALID).  Bitwise reproducible.              */
+int vt_glm_influence_max_directions(int D);
+int vt_glm_influence(const double* X, int64_t ldx, int64_t N, int D, const double* c, const double* V, int K,
+                     double alpha, double* out, int64_t ldo, void* stream);
+
 /* ---- Dense Cholesky solver -------------------------------------------------
  * vt_potrf / vt_potrs replace scipy.linalg.cho_factor / cho_solve behind
  * get_dense_cholesky_solver (solver_lib.py:27,29).  A is overwritten by its

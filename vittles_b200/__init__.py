@@ -10,6 +10,8 @@ from .sensitivity_lib import \
 
 from .sparse_hessian_lib import SparseBlockHessian
 from .lr_cov_lib import LinearResponseCovariances
+from .influence_lib import ObservationInfluence, AMIPResult
+from . import influence_lib
 from . import solver_lib
 from . import bivariate_sensitivity_lib
 from . import objectives

@@ -41,6 +41,8 @@ SIGNATURES = {
     'vt_glm_hvp': (_I, [_P, _I64, _I64, _I, _P, _P, _D, _P, _P, _SZ, _P]),
     'vt_glm_dirderiv_workspace_bytes': (_SZ, [_I64, _I]),
     'vt_glm_dirderiv': (_I, [_P, _I64, _I64, _I, _P, _P, _I, _P, _I, _P, _P, _SZ, _P]),
+    'vt_glm_influence_max_directions': (_I, [_I]),
+    'vt_glm_influence': (_I, [_P, _I64, _I64, _I, _P, _P, _I, _D, _P, _I64, _P]),
     'vt_potrf_dinv_doubles': (_SZ, [_I]),
     'vt_potrf': (_I, [_P, _I64, _I, _P, _P, _P]),
     'vt_potrs': (_I, [_P, _I64, _I, _P, _P, _I64, _I, _P]),

@@ -172,6 +172,12 @@ int vt_glm_hvp(const double* X, int64_t ldx, int64_t N, int D, const double* s, 
   return glm_hvp(X, ldx, N, D, s, v, ridge, out, static_cast<double*>(workspace), workspace_bytes, S(stream));
 }
 
+int vt_glm_influence_max_directions(int D) { return glm_influence_max_directions(D); }
+int vt_glm_influence(const double* X, int64_t ldx, int64_t N, int D, const double* c, const double* V, int K,
+                     double alpha, double* out, int64_t ldo, void* stream) {
+  return glm_influence(X, ldx, N, D, c, V, K, alpha, out, ldo, S(stream));
+}
+
 size_t vt_glm_dirderiv_workspace_bytes(int64_t N, int D) { return glm_dirderiv_workspace_bytes(N, D); }
 
 int vt_glm_dirderiv(const double* X, int64_t ldx, int64_t N, int D, const double* z, const double* w, int family,

@@ -164,10 +164,21 @@ struct DirDerivOp {
   }
 };
 
+// out[j * ldo + n] = alpha * c_n * (x_n . v_j): the per-observation influence of Q quantities of interest
+struct InfluenceOp {
+  const double* c;
+  double* out;
+  long ldo;
+  double alpha;
+  struct Aux { double c; };
+  __device__ Aux load(long n) const { return Aux{c[n]}; }
+  __device__ void store(long n, int j, double t, const Aux& a) const { out[(long)j * ldo + n] = alpha * (a.c * t); }
+};
+
 template <class RowOp, int Q, int CPT, int NOUT = 1, bool CMAX = false>
 int launch_xtfx(const XtfxParams& p, const RowOp& op, cudaStream_t stream, int* grid_out) {
   constexpr int R = (CPT <= 8) ? 8 / CPT : 1;
-  constexpr int CTAS_PER_SM = (R * CPT <= 8 && NOUT == 1) ? 2 : 1;
+  constexpr int CTAS_PER_SM = xt_ctas_per_sm<Q, CPT, R, NOUT>();
   const size_t smem = xtfx_smem_bytes(p.Dp, R, Q);
   VT_CUDA(cudaFuncSetAttribute(xtfx_kernel<RowOp, Q, CPT, R, NOUT, CMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long nblocks = (p.N + R - 1) / R;
@@ -304,6 +315,57 @@ int glm_hvp_multi(const double* X, long ldx, long N, int D, const double* s, con
     case 2: return hvp_multi_q<2>(p, s, V, ridge, out, stream);
     case 3: return hvp_multi_q<3>(p, s, V, ridge, out, stream);
     default: return hvp_multi_q<4>(p, s, V, ridge, out, stream);
+  }
+}
+
+// Directions per influence pass: the Q x CPT direction registers of a thread bound Q (no spills, -Xptxas -v)
+int glm_influence_max_directions(int D) {
+  if (D < 1) return 0;
+  if (D <= 2048) return GLM_INFLUENCE_MAXQ;
+  if (D <= 4096) return 2;
+  if (D <= 8192) return 1;
+  return 0;
+}
+
+namespace {
+template <int Q>
+int influence_q(const XtfxParams& p, const InfluenceOp& op, cudaStream_t stream) {
+  int grid = 0;
+  const int D = p.D;
+  if (D <= 512) return launch_xtfx<InfluenceOp, Q, 1, 0>(p, op, stream, &grid);
+  if (D <= 1024) return launch_xtfx<InfluenceOp, Q, 2, 0>(p, op, stream, &grid);
+  if (D <= 2048) return launch_xtfx<InfluenceOp, Q, 4, 0>(p, op, stream, &grid);
+  if constexpr (Q <= 2) {
+    if (D <= 4096) return launch_xtfx<InfluenceOp, Q, 8, 0>(p, op, stream, &grid);
+  }
+  if constexpr (Q == 1) {
+    if (D <= 8192) return launch_xtfx<InfluenceOp, 1, 16, 0>(p, op, stream, &grid);
+  }
+  set_error("glm_influence: %d directions at D = %d exceed the per-pass limit", Q, D);
+  return VT_ERR_INVALID;
+}
+}  // namespace
+
+int glm_influence(const double* X, long ldx, long N, int D, const double* c, const double* V, int q, double alpha,
+                  double* out, long ldo, cudaStream_t stream) {
+  VT_REQUIRE(c && out, "glm_influence: null pointer");
+  VT_REQUIRE(D >= 1 && D <= 8192, "glm_influence: D = %d is not supported (1 <= D <= 8192)", D);
+  const int qmax = glm_influence_max_directions(D);
+  VT_REQUIRE(q >= 1 && q <= qmax, "glm_influence: 1..%d directions per pass at D = %d, got %d", qmax, D, q);
+  VT_REQUIRE(ldo >= N, "glm_influence: ldo = %ld < N = %ld", ldo, N);
+  XtfxParams p;
+  int st = make_params(p, X, ldx, N, D, V, nullptr, 0, false);
+  if (st != VT_OK) return st;
+  const InfluenceOp op{c, out, ldo, alpha};
+  switch (q) {
+    case 1: return influence_q<1>(p, op, stream);
+    case 2: return influence_q<2>(p, op, stream);
+    case 3: return influence_q<3>(p, op, stream);
+    case 4: return influence_q<4>(p, op, stream);
+    case 5: return influence_q<5>(p, op, stream);
+    case 6: return influence_q<6>(p, op, stream);
+    case 7: return influence_q<7>(p, op, stream);
+    default: return influence_q<8>(p, op, stream);
   }
 }
 

@@ -31,6 +31,13 @@ int glm_dirderiv(const double* X, long ldx, long N, int D, const double* z, cons
                  const double* dirs, int q, double* out, double* workspace, size_t workspace_bytes,
                  cudaStream_t stream);
 
+// out[j * ldo + n] = alpha * c[n] * (x_n . V[j, :]) for j < q, n < N (V (q, D) row-major): one pass over X that
+// writes q values per row and no column sums.  q <= glm_influence_max_directions(D) (0 for D > 8192).
+constexpr int GLM_INFLUENCE_MAXQ = 8;
+int glm_influence_max_directions(int D);
+int glm_influence(const double* X, long ldx, long N, int D, const double* c, const double* V, int q, double alpha,
+                  double* out, long ldo, cudaStream_t stream);
+
 size_t gemv_workspace_bytes(int M, long N);
 // y = alpha * A x + beta * y0, A (M x N) row-major with leading dimension lda
 int gemv_rows(const double* A, long lda, int M, long N, const double* x, double alpha, const double* y0, double beta,

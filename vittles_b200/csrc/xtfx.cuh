@@ -6,6 +6,7 @@
 //   * Hessian-vector product         (Q=1; u = s_n * t)            -> CG solver
 //   * Q Hessian-vector products      (Q=NOUT<=4; u_j = s_n * t_j)  -> multi-RHS CG: one read of X for Q columns
 //   * Taylor directional derivatives (Q=m; u = c_n * prod_j t_j)   -> dirderiv
+//   * per-row outputs only           (NOUT=0, Q<=8; out_jn = op.store(n, j, t_j)) -> observation influence
 //
 // Structure (B200): persistent CTAs, two per SM, 256 threads.  A block of
 // R = 8/CPT rows (32 KB for D = 512*CPT) is staged in shared memory by ONE
@@ -88,8 +89,47 @@ __device__ __forceinline__ uint32_t xt_himax(uint32_t m, double v) {
   const uint32_t h = (uint32_t)__double2hiint(v);
   return h > m ? h : m;
 }
+// NOUT = 0: no transposed pass at all - the row functor stores the Q dot products of each row (op.store(n, j, t_j)).
+// The directions then take the registers the accumulators would, so two CTAs fit an SM only while Q * CPT <= 8.
+template <int Q, int CPT, int R, int NOUT>
+constexpr int xt_ctas_per_sm() {
+  return (R * CPT <= 8 && (NOUT == 1 || (NOUT == 0 && Q * CPT <= 8))) ? 2 : 1;
+}
+
+// Sum over the warp of each of the Q values s[0..Q-1] by a transpose-reduce: every step halves the values a lane
+// holds, the lanes of the pair exchanging the halves they drop (Q/2 + Q/4 + ... shuffles, then a plain butterfly over
+// the remaining lanes), instead of Q separate 5-step reductions.  Afterwards lane l holds the sum of value
+// j = l / (32 / QP) (QP = Q rounded up to a power of two).  Each lane adds its values in a fixed order, so the result
+// is bitwise reproducible.
+__host__ __device__ constexpr int xt_pow2_ceil(int q) { return q <= 1 ? 1 : 2 * xt_pow2_ceil((q + 1) / 2); }
+
+template <int Q>
+__device__ __forceinline__ double xt_transpose_reduce(double (&s)[Q], int lane) {
+  static_assert(Q >= 1 && Q <= 32, "one value per lane at most");
+  constexpr int QP = xt_pow2_ceil(Q);
+  double v[QP];
+#pragma unroll
+  for (int j = 0; j < QP; ++j) v[j] = j < Q ? s[j] : 0.0;
+#pragma unroll
+  for (int m = QP, o = 16; o >= 1; o >>= 1) {
+    if (m > 1) {
+      const bool upper = (lane & o) != 0;        // this lane keeps the upper half of its values
+#pragma unroll
+      for (int j = 0; j < m / 2; ++j) {
+        const double keep = upper ? v[j + m / 2] : v[j];
+        const double send = upper ? v[j] : v[j + m / 2];
+        v[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+      }
+      m /= 2;
+    } else {
+      v[0] += __shfl_xor_sync(0xffffffffu, v[0], o);
+    }
+  }
+  return v[0];
+}
+
 template <class RowOp, int Q, int CPT, int R, int NOUT = 1, bool CMAX = false>
-__global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 1) xtfx_kernel(const XtfxParams p, const RowOp op) {
+__global__ void __launch_bounds__(XT_THREADS, (xt_ctas_per_sm<Q, CPT, R, NOUT>())) xtfx_kernel(const XtfxParams p, const RowOp op) {
   extern __shared__ __align__(128) unsigned char xt_raw[];
   const int Dp = p.Dp;
   double* bufs = reinterpret_cast<double*>(xt_raw);
@@ -133,9 +173,10 @@ __global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 
       v[j][i].x = (c < p.D) ? p.V[(long)j * p.D + c] : 0.0;
       v[j][i].y = (c + 1 < p.D) ? p.V[(long)j * p.D + c + 1] : 0.0;
     }
-  double2 acc[NOUT][CPT];
+  constexpr int NACC = NOUT > 0 ? NOUT : 1;
+  double2 acc[NACC][CPT];
 #pragma unroll
-  for (int o = 0; o < NOUT; ++o)
+  for (int o = 0; o < NACC; ++o)
 #pragma unroll
     for (int i = 0; i < CPT; ++i) acc[o][i] = make_double2(0.0, 0.0);
   uint32_t cmx[CMAX ? 2 * CPT : 1];
@@ -168,8 +209,10 @@ __global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 
     // per-row operands of the row functor (y, w, z, s ...): issue the global loads
     // now so that their latency overlaps the dot products instead of sitting in
     // the serial functor step
+    // (NOUT = 0: thread tid stores output tid / R of row tid % R)
+    constexpr int NAUX = NOUT == 0 ? R * Q : R;
     typename RowOp::Aux aux;
-    if (tid < R && tid < rows) aux = op.load(row0 + tid);
+    if (tid < NAUX && tid % R < rows) aux = op.load(row0 + tid % R);
     double2 x[R][CPT];
 #pragma unroll
     for (int r = 0; r < R; ++r)
@@ -186,18 +229,44 @@ __global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 
       if (nb < nblocks) issue(nb, buf);
     }
     // ---- phase 1: row dot products --------------------------------------
+    if constexpr (NOUT == 0) {
+      constexpr int LPV = 32 / xt_pow2_ceil(Q);                  // lanes that end up holding the same direction's sum
 #pragma unroll
-    for (int r = 0; r < R; ++r)
+      for (int r = 0; r < R; ++r) {
+        double s[Q];
 #pragma unroll
-      for (int j = 0; j < Q; ++j) {
+        for (int j = 0; j < Q; ++j) {
+          s[j] = 0.0;
+#pragma unroll
+          for (int i = 0; i < CPT; ++i) s[j] = fma(x[r][i].x, v[j][i].x, fma(x[r][i].y, v[j][i].y, s[j]));
+        }
+        const double t = xt_transpose_reduce<Q>(s, lane);
+        const int j = lane / LPV;
+        if (lane % LPV == 0 && j < Q) s_part[(warp * R + r) * Q + j] = t;
+      }
+    } else {
+#pragma unroll
+      for (int r = 0; r < R; ++r)
+#pragma unroll
+        for (int j = 0; j < Q; ++j) {
+          double s = 0.0;
+#pragma unroll
+          for (int i = 0; i < CPT; ++i) s = fma(x[r][i].x, v[j][i].x, fma(x[r][i].y, v[j][i].y, s));
+          s = warp_sum(s);
+          if (lane == 0) s_part[(warp * R + r) * Q + j] = s;
+        }
+    }
+    __syncthreads();
+    if constexpr (NOUT == 0) {
+      // R * Q threads, one output each: consecutive threads store consecutive rows of one direction
+      if (tid < R * Q) {
+        const int r = tid % R, j = tid / R;
         double s = 0.0;
 #pragma unroll
-        for (int i = 0; i < CPT; ++i) s = fma(x[r][i].x, v[j][i].x, fma(x[r][i].y, v[j][i].y, s));
-        s = warp_sum(s);
-        if (lane == 0) s_part[(warp * R + r) * Q + j] = s;
+        for (int w = 0; w < 8; ++w) s += s_part[(w * R + r) * Q + j];
+        if (r < rows) op.store(row0 + r, j, s, aux);
       }
-    __syncthreads();
-    if (tid < R) {
+    } else if (tid < R) {
       double t[Q];
 #pragma unroll
       for (int j = 0; j < Q; ++j) {
@@ -222,7 +291,7 @@ __global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 
         for (int o = 0; o < NOUT; ++o) s_u[tid * NOUT + o] = u[o];
       }
     }
-    if (p.partial) {
+    if (NOUT > 0 && p.partial) {
       __syncthreads();
       // ---- phase 2: rank-R update of the column sums --------------------
 #pragma unroll
@@ -250,7 +319,7 @@ __global__ void __launch_bounds__(XT_THREADS, (R * CPT <= 8 && NOUT == 1) ? 2 : 
     }
     // s_part / s_u are rewritten only after the next block's first barrier
   }
-  if (p.partial) {
+  if (NOUT > 0 && p.partial) {
 #pragma unroll
     for (int o = 0; o < NOUT; ++o)
 #pragma unroll

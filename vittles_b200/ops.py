@@ -393,6 +393,41 @@ def glm_dirderiv(X, z, dirs, w=None, family='logistic', out=None):
     return out
 
 
+def glm_influence_max_directions(D):
+    """Directions one pass of ``glm_influence`` takes at width D: 8 up to 2048, 2 up to 4096, 1 up to 8192, else 0."""
+    return int(_cabi.load().vt_glm_influence_max_directions(int(D)))
+
+
+def glm_influence(X, c, V, alpha=1.0, out=None):
+    """out (K, N) = alpha * c[None, :] * (V @ X.T): row k holds alpha c_n (x_n . V[k]) for every row n of X.  One pass
+    over X (vt_glm_influence) per glm_influence_max_directions(D) rows of V; nothing of size N x D is formed.  ``out``
+    may be a row-major view with a leading dimension >= N."""
+    lib = _cabi.require_cuda()
+    _mat(X, 'X')
+    N, D = X.shape
+    V = _f64(V, 'V')
+    if V.dim() != 2 or V.shape[1] != D or V.shape[0] < 1:
+        raise ValueError('V must have shape (K, D) with K >= 1 and D = {}, got {}'.format(D, tuple(V.shape)))
+    K = V.shape[0]
+    qmax = glm_influence_max_directions(D)
+    if qmax == 0:
+        raise ValueError('glm_influence: D = {} is not supported (D <= 8192)'.format(D))
+    c = _f64(c, 'c').reshape(-1).contiguous()
+    if c.numel() != N:
+        raise ValueError('c must have one entry per row of X ({}), got {}'.format(N, c.numel()))
+    V = V.contiguous()
+    if out is None:
+        out = torch.empty((K, N), dtype=torch.float64, device=X.device)
+    _mat(out, 'out')
+    if tuple(out.shape) != (K, N):
+        raise ValueError('out must have shape ({}, {}), got {}'.format(K, N, tuple(out.shape)))
+    for k0 in range(0, K, qmax):
+        q = min(qmax, K - k0)
+        check(lib.vt_glm_influence(ptr(X), _ld(X), N, D, ptr(c), ptr(V[k0:k0 + q]), q, float(alpha), ptr(out[k0:k0 + q]),
+                                   _ld(out), stream()))
+    return out
+
+
 # --------------------------------------------------------------- Cholesky ----
 class CholeskyFactor:
     """Lower Cholesky factor of a dense SPD matrix, resident on the GPU.
@@ -655,7 +690,7 @@ def _device_scoped(fn):
 
 
 for _name in ('gemm', 'tf32_convert', 'tf32_gemm', 'ozaki_slice', 'ozaki_gemm', 'syrk_weighted', 'glm_stats', 'glm_hvp',
-              'glm_hvp_multi', 'glm_dirderiv', 'potrf', 'ij_apply', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
+              'glm_hvp_multi', 'glm_dirderiv', 'glm_influence', 'potrf', 'ij_apply', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
               'synth_design',
               'synth_theta', 'synth_bernoulli', 'block_potrf', 'block_trsm', 'block_solve', 'tall_gemv', 'tall_colsum',
               'gmm_blocks'):
