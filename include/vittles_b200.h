@@ -17,11 +17,10 @@
  *     last failure on the calling thread is returned by vt_last_error();
  *   - the library never allocates device memory: workspaces are sized by the
  *     *_workspace_bytes queries and owned by the caller, and it keeps no state
- *     between calls.  (One experimental exception, off by default: with
- *     VT_OZAKI_OVERLAP=1 in the environment the chunked INT8 drivers
- *     vt_ij_apply_ozaki / vt_syrk_ozaki slice chunk c+1 on a helper stream -
- *     created once per host thread and device, fenced against `stream` by
- *     events on both sides - while the tensor cores multiply chunk c.)
+ *     between calls.  (One exception: vt_potrf with four or more block
+ *     columns runs its large trailing updates on a helper stream - created
+ *     lazily once per host thread and device, fenced against `stream` by
+ *     events, and joined before the call returns.)
  */
 #ifndef VITTLES_B200_H
 #define VITTLES_B200_H

@@ -4,7 +4,6 @@
 set -x
 # INT8 engine: where the MMA thread and the converter warps spend their clocks (Hessian and apply)
 VT_OGEMM_TIMING=1 python tools/syrk_probe.py 2000000 1024 8000000 320 4000000 512 > gpurun_out/syrk_probe_timing.jsonl
-VT_OZAKI_FUSE=0 python tools/syrk_probe.py 2000000 1024 > gpurun_out/syrk_probe_unfused.jsonl      # same hash as fused
 VT_OGEMM_TIMING=1 python tools/ogemm_probe.py timing > gpurun_out/ogemm_timing.jsonl
 # source-level stall samples of the fused kernel (converter warps) and of the apply GEMM (epilogue)
 ncu --set full --import-source on --clock-control none -k regex:ogemm_kernel --launch-skip 4 --launch-count 1 \

@@ -1,4 +1,4 @@
-# Round 2, job a: INT8 peak probe, stacked-B vs one-product-per-instruction issue, new digit scheme tests.
+# Round 2, job a: INT8 peak probe, stacked-B issue, new digit scheme tests.
 set -x
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,clocks.sm,clocks.max.sm,power.draw,power.limit --format=csv
@@ -6,12 +6,9 @@ VT_PEAK_SECS=0.2 timeout 120 python tools/ogemm_probe.py i8_peak > gpurun_out/i8
 VT_PEAK_SECS=3 timeout 200 python tools/ogemm_probe.py i8_peak > gpurun_out/i8_peak_sustained.jsonl 2>&1
 cat gpurun_out/i8_peak_burst.jsonl gpurun_out/i8_peak_sustained.jsonl
 timeout 600 python -m pytest tests/test_gpu_ozaki.py -x -q 2>&1 | tail -15
-VT_OGEMM_STACK=0 timeout 600 python -m pytest tests/test_gpu_ozaki.py -x -q 2>&1 | tail -5
 for st in one k1024 big ragged s8 apply; do timeout 150 python tools/ogemm_probe.py $st; done > gpurun_out/ogemm_stages.jsonl 2>&1
 cat gpurun_out/ogemm_stages.jsonl
 timeout 150 python tools/ogemm_probe.py time_parts > gpurun_out/ogemm_parts_stack1.jsonl 2>&1
-VT_OGEMM_STACK=0 timeout 150 python tools/ogemm_probe.py time_parts > gpurun_out/ogemm_parts_stack0.jsonl 2>&1
-cat gpurun_out/ogemm_parts_stack1.jsonl gpurun_out/ogemm_parts_stack0.jsonl
 timeout 150 python tools/ogemm_probe.py time_apply > gpurun_out/ogemm_time_apply.jsonl 2>&1
 timeout 150 python tools/ogemm_probe.py time_syrk > gpurun_out/ogemm_time_syrk.jsonl 2>&1
 cat gpurun_out/ogemm_time_apply.jsonl gpurun_out/ogemm_time_syrk.jsonl

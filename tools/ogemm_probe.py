@@ -167,7 +167,7 @@ def run(stage):
         print(json.dumps({'stage': stage, 'rc': rc, 'ms': ms, 'launches_x_ctas': buf[4], 'clk_total': buf[0] / n,
                           'clk_wait_accum': buf[1] / n, 'clk_wait_B': buf[2] / n, 'clk_wait_A': buf[3] / n,
                           'tiles_per_cta': 8 * (nchunk // 64) / 148}), flush=True)
-        # the whole apply (fused slicing of the next chunk unless VT_OZAKI_FUSE=0)
+        # the whole apply (D = 1024: the converter warps of each GEMM slice the next chunk)
         N = 20 * nchunk
         Xb = ops.synth_design(7, 0, N, D, dev)
         resid = rnd(N)

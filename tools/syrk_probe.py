@@ -1,5 +1,4 @@
-"""Weighted SYRK on the INT8 slicing engine: time per call and a hash of the result (the fused and the separate
-slicers must give bit-identical Hessians: run once with VT_OZAKI_FUSE=0 and once without).
+"""Weighted SYRK on the INT8 slicing engine: time per call and a hash of the result.
     python tools/syrk_probe.py [N D [N D ...]]"""
 import hashlib
 import json
@@ -32,7 +31,7 @@ def main():
         s = torch.rand(N, device=dev, dtype=torch.float64, generator=torch.Generator(device=dev).manual_seed(N + D))
         if os.environ.get('VT_PROBE_UNWEIGHTED') == '1':       # X^T X (the Schur complement of config 3)
             s = None
-        row = {'N': N, 'D': D, 'fuse': os.environ.get('VT_OZAKI_FUSE', '1'), 'weighted': s is not None}
+        row = {'N': N, 'D': D, 'weighted': s is not None}
         for prec in ('f64_ozaki', 'f64'):
             ms, H = timed(lambda: ops.syrk_weighted(X, s, precision=prec), 3)
             row[prec + '_ms'] = ms

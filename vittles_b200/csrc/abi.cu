@@ -271,7 +271,7 @@ int vt_ozaki_slice_t(const double* X, int64_t ldx, int64_t rows, int cols, const
                      int8_t* out, int64_t ldo, int64_t slice_stride, int nslices, double* scale_out, int integer_variant,
                      void* stream) {
   return ozaki_slice_t(X, ldx, rows, cols, sq, reinterpret_cast<const unsigned long long*>(colmax), out, ldo, slice_stride,
-                       nslices, scale_out, integer_variant, num_sms() * 6, S(stream));
+                       nslices, scale_out, integer_variant, S(stream));
 }
 
 int vt_ozaki_gemm(int M, int N, int K, const int8_t* A, int64_t lda, int64_t a_slice_stride, const int8_t* B,

@@ -77,11 +77,9 @@ __global__ void __launch_bounds__(128) block_potrf_kernel(double* blocks, long G
 // thread has all M loads of its column in flight before the substitution
 // starts (HBM bound: 16 M Dg bytes per block).
 constexpr int TRSM_BPC = 4;
-#ifndef VT_TRSM_MINB
-#define VT_TRSM_MINB 3
-#endif
+constexpr int TRSM_MINB = 3;           // resident CTAs per SM for blocks of up to 24 rows
 template <int MT, bool TR>
-__global__ void __launch_bounds__(256, MT <= 24 ? VT_TRSM_MINB : 1) block_trsm_kernel(const double* __restrict__ Lb, double* __restrict__ C, long G,
+__global__ void __launch_bounds__(256, MT <= 24 ? TRSM_MINB : 1) block_trsm_kernel(const double* __restrict__ Lb, double* __restrict__ C, long G,
                                                          int M, int Dg) {
   __shared__ double sl[TRSM_BPC][MT * MT];
   __shared__ double sinv[TRSM_BPC][MT];

@@ -19,10 +19,7 @@ constexpr int O_EPI_WARPS = 8, O_CONV_WARPS = 8;
 constexpr int W_EPI0 = O_CONV_WARPS, W_TMA = O_CONV_WARPS + O_EPI_WARPS, W_MMA = W_TMA + 1;   // W_EPI0 % 4 == 0 (TMEM quarters)
 constexpr int A_TILE_BYTES = OBM * OBK;        // 16 KB: one slice of the A tile for one k-block
 constexpr int B_TILE_BYTES = OBN * OBK;        //  8 KB: one slice of the B tile for one k-block
-#ifndef VT_A_RING
-#define VT_A_RING 6
-#endif
-constexpr int A_RING = VT_A_RING;              // A slices stream through a ring of this depth
+constexpr int A_RING = 6;                      // A slices stream through a ring of this depth
 constexpr int B_BUFS = 2;                      // all S slices of the B tile, double buffered over k-blocks
 
 template <int S>
@@ -382,7 +379,7 @@ __device__ __forceinline__ double exact_double(long long u) {
 }
 __device__ __forceinline__ double pair_double(int hi, int lo) { return exact_double((long long)hi * 256 + (long long)lo); }
 
-template <int S, bool STACK>
+template <int S>
 __global__ void __launch_bounds__(O_THREADS, 1)
 ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const OKernelArgs a) {
   constexpr int B_BUF_BYTES = OCfg<S>::B_BUF_BYTES;
@@ -474,39 +471,27 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
             w_a += clock64() - c0;
             tc_fence_after();
             const uint32_t a_lo0 = desc_lo0 + ((sA0 + as * A_TILE_BYTES) >> 4);
-            if constexpr (STACK) {
-              // Slice s of A meets slices 0 .. S-1-s of B, whose tiles are CONTIGUOUS in the B box (64 rows of
-              // 128 bytes each), and product (s, t) belongs to accumulator s + t = columns 64 (s + t): one
-              // tcgen05.mma with N = 64 (S - s) (cut at 256) does them all and reads the A tile once instead of
-              // S - s times - 10 instructions and 96 KB of shared-memory operand reads per k-step for S = 7
-              // instead of 28 instructions and 168 KB (the N = 64 form is bound by those reads).
-              // (measured, bare issue loop: an instruction of N columns costs max(N / 2, 34 + 0.36 N) clocks - 128 for
-              // N = 256, 101 for 192, 80 for 128, 57 for 64 - so 448 columns go as 256 + 192, 384 as 192 + 192, ...)
-              const int NTOT = OBN * (S - s);
-              const int NPART = (NTOT + 255) / 256;
-              const int NFIRST = ((NTOT / NPART) + 63) / 64 * 64;           // balanced parts, multiples of 64
+            // Slice s of A meets slices 0 .. S-1-s of B, whose tiles are CONTIGUOUS in the B box (64 rows of
+            // 128 bytes each), and product (s, t) belongs to accumulator s + t = columns 64 (s + t): one
+            // tcgen05.mma with N = 64 (S - s) (cut at 256) does them all and reads the A tile once instead of
+            // S - s times - 10 instructions and 96 KB of shared-memory operand reads per k-step for S = 7
+            // instead of 28 instructions and 168 KB (the N = 64 form is bound by those reads).
+            // (measured, bare issue loop: an instruction of N columns costs max(N / 2, 34 + 0.36 N) clocks - 128 for
+            // N = 256, 101 for 192, 80 for 128, 57 for 64 - so 448 columns go as 256 + 192, 384 as 192 + 192, ...)
+            const int NTOT = OBN * (S - s);
+            const int NPART = (NTOT + 255) / 256;
+            const int NFIRST = ((NTOT / NPART) + 63) / 64 * 64;           // balanced parts, multiples of 64
 #pragma unroll
-              for (int pn = 0; pn < NPART; ++pn) {
-                const int c0 = pn * NFIRST;
-                const int n = (pn == NPART - 1) ? NTOT - c0 : NFIRST;
-                const uint32_t idesc = idesc0 | ((uint32_t)(n >> 3) << 17);
-                const uint32_t tmem_d = tmem_base + (uint32_t)(s * OBN + c0);
-                const uint32_t b_lo = b_lo0 + (uint32_t)((c0 / OBN) * (B_TILE_BYTES >> 4));
+            for (int pn = 0; pn < NPART; ++pn) {
+              const int c0 = pn * NFIRST;
+              const int n = (pn == NPART - 1) ? NTOT - c0 : NFIRST;
+              const uint32_t idesc = idesc0 | ((uint32_t)(n >> 3) << 17);
+              const uint32_t tmem_d = tmem_base + (uint32_t)(s * OBN + c0);
+              const uint32_t b_lo = b_lo0 + (uint32_t)((c0 / OBN) * (B_TILE_BYTES >> 4));
 #pragma unroll
-                for (int kk = 0; kk < OBK / O_UMMA_K; ++kk)
-                  umma_i8_lohi(tmem_d, a_lo0 + 2u * kk, desc_hi, b_lo + 2u * kk, desc_hi, idesc,
-                               (s == 0 && kk == 0) ? first : 1u);
-              }
-            } else {
-              constexpr uint32_t idesc = idesc0 | ((uint32_t)(OBN >> 3) << 17);
-#pragma unroll
-              for (int t = 0; t < S - s; ++t) {
-                const uint32_t tmem_d = tmem_base + (uint32_t)((s + t) * OBN);
-#pragma unroll
-                for (int kk = 0; kk < OBK / O_UMMA_K; ++kk)
-                  umma_i8_lohi(tmem_d, a_lo0 + 2u * kk, desc_hi, b_lo0 + (uint32_t)(t * (B_TILE_BYTES >> 4)) + 2u * kk,
-                               desc_hi, idesc, (s == 0 && kk == 0) ? first : 1u);
-              }
+              for (int kk = 0; kk < OBK / O_UMMA_K; ++kk)
+                umma_i8_lohi(tmem_d, a_lo0 + 2u * kk, desc_hi, b_lo + 2u * kk, desc_hi, idesc,
+                             (s == 0 && kk == 0) ? first : 1u);
             }
             umma_commit(aempty(as));
             if (++as == A_RING) { as = 0; aph ^= 1u; }
@@ -723,23 +708,6 @@ int make_slice_map(CUtensorMap* map, const int8_t* base, long rows, int K, long 
   return VT_OK;
 }
 
-bool ozaki_fuse_slicing() {
-  static const bool on = [] {
-    const char* e = getenv("VT_OZAKI_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
-// VT_OGEMM_STACK=0 selects the one-product-per-instruction issue loop (N = 64) for A/B measurements.
-bool ogemm_stacked() {
-  static const bool on = [] {
-    const char* e = getenv("VT_OGEMM_STACK");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 // VT_OGEMM_TIMING=1: a device buffer of 8 counters {total, wait accumulators, wait B, wait A, CTAs} that every
 // launch adds to; vt_debug_ogemm_timing() reads and clears it.
 unsigned long long* ogemm_timing_buffer() {
@@ -752,9 +720,9 @@ unsigned long long* ogemm_timing_buffer() {
   return buf;
 }
 
-template <int S, bool STACK>
+template <int S>
 int launch_s(const CUtensorMap& mA, const CUtensorMap& mB, const OKernelArgs& a, cudaStream_t stream) {
-  auto kern = ogemm_kernel<S, STACK>;
+  auto kern = ogemm_kernel<S>;
   VT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OCfg<S>::SMEM_BYTES));
   VT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   const long slots = num_sms();
@@ -766,44 +734,6 @@ int launch_s(const CUtensorMap& mA, const CUtensorMap& mB, const OKernelArgs& a,
 }
 
 inline size_t align_up(size_t x, size_t al) { return (x + al - 1) / al * al; }
-
-// Experimental, off by default (VT_OZAKI_OVERLAP=1): slice chunk c+1 on a helper stream while the tensor
-// cores multiply chunk c - small persistent slicing grids that can share an SM with the resident GEMM CTA,
-// fenced against the caller's stream with events.  Measured on B200 it is not faster (Hessian 30 ms vs 21 ms
-// per 1M observations: the two kernels end up serialised and the small grids are slow on their own), so the
-// default runs everything on the caller's stream with full grids.  The helper stream and its events are
-// created lazily, once per host thread and device, only when the switch is on.
-bool ozaki_overlap() {
-  static const bool on = [] {
-    const char* e = getenv("VT_OZAKI_OVERLAP");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
-
-struct SideLane {
-  int dev = -1;
-  cudaStream_t side = nullptr;
-  cudaEvent_t fork = nullptr, ready[2] = {nullptr, nullptr}, consumed[2] = {nullptr, nullptr};
-};
-int side_lane(SideLane** out) {
-  static thread_local SideLane lane;
-  int dev = 0;
-  VT_CUDA(cudaGetDevice(&dev));
-  if (lane.dev != dev) {
-    SideLane fresh;
-    VT_CUDA(cudaStreamCreateWithFlags(&fresh.side, cudaStreamNonBlocking));
-    VT_CUDA(cudaEventCreateWithFlags(&fresh.fork, cudaEventDisableTiming));
-    for (int i = 0; i < 2; ++i) {
-      VT_CUDA(cudaEventCreateWithFlags(&fresh.ready[i], cudaEventDisableTiming));
-      VT_CUDA(cudaEventCreateWithFlags(&fresh.consumed[i], cudaEventDisableTiming));
-    }
-    fresh.dev = dev;
-    lane = fresh;          // (a lane created for another device is kept alive by the driver until exit)
-  }
-  *out = &lane;
-  return VT_OK;
-}
 
 long ozaki_chunk_rows(long N, int D, int nslices) {
   const long ld = (D + 15) / 16 * 16;
@@ -836,11 +766,9 @@ int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, lon
              "ozaki_slice: bad slice layout");
   VT_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, "ozaki_slice: output must be 16-byte aligned");
   if (rows == 0) return VT_OK;
-  // overlapped (VT_OZAKI_OVERLAP=1): CTAs of 4 warps, two per SM - what fits in the registers the resident GEMM CTA
-  // leaves (320 threads x 96 registers of 64 K)
-  const int bt = ozaki_overlap() ? 128 : 256;
+  const int bt = 256;
   long blocks = (rows + bt / 32 - 1) / (bt / 32);
-  const long cap = (long)num_sms() * (ozaki_overlap() ? 2 : 8);
+  const long cap = (long)num_sms() * 8;
   if (blocks > cap) blocks = cap;
   const int rc = cols <= 1024 ? (cols + 127) / 128 : 0;        // rows of up to 1024 elements stay in registers
   const SliceJob jb{X, ldx, rows, cols, out, ldo, slice_stride, scale_out, fold, nullptr, nullptr};
@@ -877,14 +805,15 @@ int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, lon
 // Transposed digits out[s][feature][observation] of sq_n x_ni (the Hessian's operand) as a launch of its own.
 int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* sq, const unsigned long long* colmax,
                   int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, int integer_variant,
-                  int max_ctas, cudaStream_t stream) {
+                  cudaStream_t stream) {
   VT_REQUIRE(X && colmax && out && scale_out, "ozaki_slice_t: null pointer");      // sq == nullptr: unweighted
   VT_REQUIRE(rows >= 1 && cols >= 1 && ldx >= cols && ldo >= rows && ldo % 16 == 0 && slice_stride >= (long)cols * ldo &&
              slice_stride % 16 == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0, "ozaki_slice_t: bad layout");
   VT_REQUIRE(nslices >= OZAKI_MIN_SLICES && nslices <= OZAKI_MAX_SLICES, "ozaki_slice_t: 5, 6 or 7 slices");
   const SliceJob jb{X, ldx, rows, cols, out, ldo, slice_stride, scale_out, nullptr, sq, colmax};
   const long steps = ((rows + ST_OBS * ST_GROUP - 1) / (ST_OBS * ST_GROUP)) * ((cols + ST_FEAT - 1) / ST_FEAT);
-  const unsigned grid = (unsigned)(steps < max_ctas ? steps : max_ctas);
+  const long cap = (long)num_sms() * 6;
+  const unsigned grid = (unsigned)(steps < cap ? steps : cap);
 #define VT_SLICE_T(SS)                                                                              \
   if (integer_variant) ozaki_slice_t_kernel<SS, true><<<grid, 32 * ST_GROUP, 0, stream>>>(jb);     \
   else ozaki_slice_t_kernel<SS, false><<<grid, 32 * ST_GROUP, 0, stream>>>(jb)
@@ -949,11 +878,10 @@ int ogemm_launch_opts(int M, int N, int K, const int8_t* A, long lda, long a_sli
     VT_REQUIRE((a.next.colmax || a.next.cols <= 1024) && a.next.ldo % 16 == 0,
                "ogemm: in-kernel slicing takes rows of at most 1024 elements");
   a.timing = ogemm_timing_buffer();
-  const bool stk = ogemm_stacked();
   switch (nslices) {
-    case 5: return stk ? launch_s<5, true>(mA, mB, a, stream) : launch_s<5, false>(mA, mB, a, stream);
-    case 6: return stk ? launch_s<6, true>(mA, mB, a, stream) : launch_s<6, false>(mA, mB, a, stream);
-    default: return stk ? launch_s<7, true>(mA, mB, a, stream) : launch_s<7, false>(mA, mB, a, stream);
+    case 5: return launch_s<5>(mA, mB, a, stream);
+    case 6: return launch_s<6>(mA, mB, a, stream);
+    default: return launch_s<7>(mA, mB, a, stream);
   }
 }
 }  // namespace
@@ -1110,34 +1038,18 @@ int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long
     tau[b] = reinterpret_cast<double*>(w);
     w += align_up((size_t)ch * 8, 256);
   }
-  const bool overlap = ozaki_overlap();
-  SideLane* L = nullptr;
-  int st = VT_OK;
-  cudaStream_t slicer = stream;
-  if (overlap) {
-    st = side_lane(&L);
-    if (st != VT_OK) return st;
-    VT_CUDA(cudaEventRecord(L->fork, stream));                  // the inputs are ready once `stream` gets here
-    VT_CUDA(cudaStreamWaitEvent(L->side, L->fork, 0));
-    slicer = L->side;
-  }
-  st = ozaki_slice(Hinv, ldh, D, D, As, ld, (long)D * ld, nslices, sigma, nullptr, stream);
+  int st = ozaki_slice(Hinv, ldh, D, D, As, ld, (long)D * ld, nslices, sigma, nullptr, stream);
   if (st != VT_OK) return st;
-  // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (rows of up to 1024 elements; VT_OZAKI_FUSE=0
-  // or longer rows: a separate slicing launch per chunk).
-  const bool fuse = !overlap && D <= 1024 && ozaki_fuse_slicing();
+  // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (rows of up to 1024 elements; longer rows:
+  // a separate slicing launch per chunk).
+  const bool fuse = D <= 1024;
   long c = 0;
   for (long r0 = 0; r0 < N; r0 += ch, ++c) {
     const int b = (int)(c & 1);
     const long rows = (N - r0 < ch) ? N - r0 : ch;
-    if (overlap && c >= 2) VT_CUDA(cudaStreamWaitEvent(L->side, L->consumed[b], 0));   // GEMM c-2 has read buffer b
     if (!fuse || c == 0) {
-      st = ozaki_slice(X + r0 * ldx, ldx, rows, D, Bs[b], ld, ch * ld, nslices, tau[b], resid + r0, slicer);   // tau_n resid_n
+      st = ozaki_slice(X + r0 * ldx, ldx, rows, D, Bs[b], ld, ch * ld, nslices, tau[b], resid + r0, stream);   // tau_n resid_n
       if (st != VT_OK) return st;
-    }
-    if (overlap) {
-      VT_CUDA(cudaEventRecord(L->ready[b], L->side));
-      VT_CUDA(cudaStreamWaitEvent(stream, L->ready[b], 0));
     }
     OLaunchOpts o;
     const long n0 = r0 + ch;
@@ -1148,7 +1060,6 @@ int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long
     st = ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs[b], ld, ch * ld, nslices, -1.0, sigma, tau[b], S + r0, lds,
                            o, stream);
     if (st != VT_OK) return st;
-    if (overlap) VT_CUDA(cudaEventRecord(L->consumed[b], stream));
   }
   return VT_OK;
 }
@@ -1230,49 +1141,30 @@ int syrk_ozaki(const double* X, long ldx, long N, int D, const double* s, double
     VT_LAUNCH_CHECK();
   }
   VT_CUDA(cudaMemsetAsync(P, 0, (size_t)p.parts * D * D * 8, stream));      // every chunk (and part) accumulates
-  const bool overlap = ozaki_overlap();
-  SideLane* L = nullptr;
-  int st = VT_OK;
-  cudaStream_t slicer = stream;
-  if (overlap) {
-    st = side_lane(&L);
-    if (st != VT_OK) return st;
-    VT_CUDA(cudaEventRecord(L->fork, stream));
-    VT_CUDA(cudaStreamWaitEvent(L->side, L->fork, 0));
-    slicer = L->side;
-  }
-  // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (VT_OZAKI_FUSE=0: a slicing launch per chunk,
-  // which cannot share an SM with the GEMM's 210 KB of shared memory and so runs between the GEMMs).
-  const bool fuse = !overlap && ozaki_fuse_slicing();
+  // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c; only chunk 0 takes a slicing launch.
   auto job = [&](long r0, int b) {
     const long rows = (N - r0 < p.chunk) ? N - r0 : p.chunk;
     return SliceJob{X + r0 * ldx, ldx, rows, D, Xs[b], p.ld, slice_stride, sigma, nullptr, sq_use ? sq_use + r0 : nullptr, cmax_use};
   };
+  int st = VT_OK;
   long c = 0;
   for (long r0 = 0; r0 < N; r0 += p.chunk, ++c) {
     const int b = (int)(c & 1);
     const long rows = (N - r0 < p.chunk) ? N - r0 : p.chunk;
-    if (overlap && c >= 2) VT_CUDA(cudaStreamWaitEvent(L->side, L->consumed[b], 0));
-    if (!fuse || c == 0) {
+    if (c == 0) {
       const SliceJob jb = job(r0, b);
-      st = ozaki_slice_t(jb.X, ldx, jb.rows, D, jb.sq, cmax_use, Xs[b], p.ld, slice_stride, nslices, sigma, 0,
-                         num_sms() * (overlap ? 1 : 6), slicer);
+      st = ozaki_slice_t(jb.X, ldx, jb.rows, D, jb.sq, cmax_use, Xs[b], p.ld, slice_stride, nslices, sigma, 0, stream);
       if (st != VT_OK) return st;
-    }
-    if (overlap) {
-      VT_CUDA(cudaEventRecord(L->ready[b], L->side));
-      VT_CUDA(cudaStreamWaitEvent(stream, L->ready[b], 0));
     }
     OLaunchOpts o;
     o.lower = 1;
     o.parts = p.parts;
     o.accumulate = 1;
     o.part_stride = (long)D * D;
-    if (fuse && r0 + p.chunk < N) o.next = job(r0 + p.chunk, b ^ 1);
+    if (r0 + p.chunk < N) o.next = job(r0 + p.chunk, b ^ 1);
     st = ogemm_launch_opts(D, D, (int)rows, Xs[b], p.ld, slice_stride, Xs[b], p.ld, slice_stride, nslices, 1.0, sigma, sigma,
                            P, D, o, stream);
     if (st != VT_OK) return st;
-    if (overlap) VT_CUDA(cudaEventRecord(L->consumed[b], stream));
   }
   const long total = (long)D * D;
   ozaki_syrk_finish_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(P, p.parts, (long)D * D, D, H, ldh);

@@ -32,7 +32,7 @@ int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, lon
 // integer_variant: the integer-only instruction sequence of the GEMM kernel's converter warps (same digits).
 int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* sq, const unsigned long long* colmax,
                   int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, int integer_variant,
-                  int max_ctas, cudaStream_t stream);
+                  cudaStream_t stream);
 
 // C (M x N, FP64) = alpha * rowscale[m] * colscale[n] * 2^-12 sum_{s+t<S} 2^{-8(s+t)} (A_s B_t^T)(m,n)
 int ogemm_launch(int M, int N, int K, const int8_t* A, long lda, long a_slice_stride, const int8_t* B, long ldb,
