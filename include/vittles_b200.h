@@ -186,19 +186,16 @@ int vt_syrk_tf32(const double* X, int64_t ldx, int64_t N, int D, const double* s
  * ~1e-14 of sigma_m tau_n K (the row scales), inside the rtol 1e-8 parity bar
  * of the FP64 path.  vt_ij_apply_ozaki is vt_ij_apply on this engine; the
  * observations are sliced chunk by chunk by converter warps inside the GEMM
- * kernel, with integer instructions only (FP64 instructions starve while the
- * tensor pipe is saturated).  vt_ozaki_slice_int runs that instruction
- * sequence as a kernel of its own (cols <= 1024; same digits), and
- * vt_ozaki_slice_t writes the Hessian's operand: digits of sq[n] * X[n][i]
- * TRANSPOSED, out[s][i][n], one scale per feature from colmax[i] (the bit
- * pattern of max_n |sq[n] X[n][i]|), integer_variant as above.               */
+ * kernel.  Every slicer, in the GEMM kernel or standing alone, forms the
+ * digits with integer instructions only, from the bit patterns (FP64
+ * instructions starve while the tensor pipe is saturated), so every digit
+ * is formed the same way.  vt_ozaki_slice_t writes the Hessian's operand:
+ * digits of sq[n] * X[n][i] TRANSPOSED, out[s][i][n], one scale per feature
+ * from colmax[i] (the bit pattern of max_n |sq[n] X[n][i]|).               */
 int vt_ozaki_slice(const double* X, int64_t ldx, int64_t rows, int cols, int8_t* out, int64_t ldo, int64_t slice_stride,
                    int nslices, double* scale_out, const double* fold, void* stream);
-int vt_ozaki_slice_int(const double* X, int64_t ldx, int64_t rows, int cols, int8_t* out, int64_t ldo, int64_t slice_stride,
-                       int nslices, double* scale_out, const double* fold, void* stream);
 int vt_ozaki_slice_t(const double* X, int64_t ldx, int64_t rows, int cols, const double* sq, const uint64_t* colmax,
-                     int8_t* out, int64_t ldo, int64_t slice_stride, int nslices, double* scale_out, int integer_variant,
-                     void* stream);
+                     int8_t* out, int64_t ldo, int64_t slice_stride, int nslices, double* scale_out, void* stream);
 int vt_ozaki_gemm(int M, int N, int K, const int8_t* A, int64_t lda, int64_t a_slice_stride, const int8_t* B,
                   int64_t ldb, int64_t b_slice_stride, int nslices, double alpha, const double* rowscale,
                   const double* colscale, double* C, int64_t ldc, void* stream);

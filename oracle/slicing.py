@@ -21,7 +21,7 @@ def _bias(nslices):
 def slice_rows(x, nslices):
     """(digits (S, rows, cols) int8, scale (rows,) float64): per-row power-of-two scale 2^e > max_k |x_rk| and the
     balanced base-256 digits of the fixed-point value q = rint(x 2^(8S-2) / scale): with B = sum_p 128 256^p the
-    bytes of (q + B) ^ B - the computation of ``fixed4_set`` / ``fixed4_digits`` in ``ogemm.cu``."""
+    bytes of (q + B) ^ B - the computation of ``fixed4_set_bits`` / ``fixed4_digits`` in ``ogemm.cu``."""
     assert 1 <= nslices <= 7
     x = np.asarray(x, dtype=np.float64)
     m = np.max(np.abs(x), axis=1)

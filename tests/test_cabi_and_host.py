@@ -20,12 +20,17 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), 'library does not export ' + name
     assert declared == set(_cabi.exported_symbols()), declared ^ set(_cabi.exported_symbols())
-    assert lib.vt_abi_version() == 1
     assert isinstance(lib.vt_last_error(), bytes)
     # inverted 128-blocks + scratch panel + flags + inverted 256-blocks + (D >= 1024) inverted 512-blocks + solve scratch + split-K tiles of the solve (148 SMs assumed without a GPU) + second panel (look-ahead)
     head = 8 * 128 * 128 + 1024 * 128 + 10 + 4 * 256 * 256 + 2 * 512 * 512 + 512 * 512
     assert lib.vt_potrf_dinv_doubles(1024) == (head + 31) // 32 * 32 + 2 * 148 * 128 * 128 + 1024 * 128
     assert lib.vt_potrf_dinv_doubles(130) == 2 * 128 * 128 + 130 * 128 + 4 + 1 * 256 * 256 + 130 * 128
+
+
+def test_abi_version():
+    """Version 2: vt_ozaki_slice_t takes no selector of the instruction sequence, and only vt_ozaki_slice slices rows."""
+    from vittles_b200 import _cabi
+    assert _cabi.load().vt_abi_version() == 2
 
 
 def test_no_cpu_fallback():

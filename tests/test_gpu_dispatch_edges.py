@@ -151,10 +151,10 @@ def _awkward_wide(rows, cols, seed):
 
 
 @pytest.mark.parametrize('cols', [1025, 2048, 3001])
-def test_row_slicer_beyond_1024_columns(vt, cols):
-    """Rows longer than 1024 elements are sliced by the RC = 0 instance, which re-reads the row from global memory:
-    digits and scales bit-identical to the CPU model (the integer variant, which keeps rows in registers, refuses
-    such rows, so this is the only path for them)."""
+def test_row_slicer_rereads_rows_beyond_1024_columns(vt, cols):
+    """Rows longer than 1024 elements are sliced by the RC = 0 instance: the integer maximum of the bit patterns over
+    the lane-strided elements, then the digits of values re-read from global memory.  Digits and scales bit-identical
+    to the CPU model."""
     X = _awkward_wide(203, cols, seed=60)
     d, sc = vt.ops.ozaki_slice(X, S7)
     d_ref, sc_ref = slicing.slice_rows(X.cpu().numpy(), S7)
@@ -164,8 +164,6 @@ def test_row_slicer_beyond_1024_columns(vt, cols):
     fold = _rnd(203, seed=61)
     d2, sc2 = vt.ops.ozaki_slice(X, S7, fold=fold)
     assert torch.equal(d2, d) and torch.equal(sc2, sc * fold)
-    with pytest.raises(ValueError):
-        vt.ops.ozaki_slice(X, S7, integer_variant=True)
 
 
 # ------------------------------------------------------- INT8 apply, many chunks ----

@@ -10,6 +10,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import vittles_b200 as vt  # noqa: E402
 from vittles_b200 import ops  # noqa: E402
+from oracle import slicing  # noqa: E402
 
 dev = torch.device('cuda', 0)
 g = torch.Generator(device=dev).manual_seed(0)
@@ -43,13 +44,19 @@ for (N, D) in ((3001, 77), (90000, 1024), (70000, 515)):
 A = rnd(130, 333)
 B = rnd(70, 333)
 print('ogemm', rel(ops.ozaki_gemm(A, B), A @ B.T))
-# the converter warps' integer-only slicers as kernels of their own, ragged shapes, and an unweighted Hessian
-# whose later chunks are sliced inside the GEMM
+# the stand-alone slicers against the CPU model at ragged shapes (rows held in registers, and rows wider than 1024
+# that are re-read), and an unweighted Hessian whose later chunks are sliced inside the GEMM
+def same_digits(got, ref):
+    return np.array_equal(got[0][:, :, :ref[0].shape[2]].cpu().numpy(), ref[0]) and np.array_equal(got[1].cpu().numpy(), ref[1])
+
+
+for Xr in (rnd(517, 333), rnd(67, 1100)):
+    print('slicer', tuple(Xr.shape), same_digits(ops.ozaki_slice(Xr, 7), slicing.slice_rows(Xr.cpu().numpy(), 7)))
 Xr = rnd(517, 333)
-print('int slicer', torch.equal(ops.ozaki_slice(Xr, 7)[0], ops.ozaki_slice(Xr, 7, integer_variant=True)[0]))
 sqr = torch.rand(517, device=dev, dtype=torch.float64, generator=g).sqrt()
 for sq_ in (sqr, None):
-    print('transposed slicers', torch.equal(ops.ozaki_slice_t(Xr, sq_, 7)[0], ops.ozaki_slice_t(Xr, sq_, 7, integer_variant=True)[0]))
+    W = (Xr if sq_ is None else Xr * sq_[:, None]).T.contiguous().cpu().numpy()
+    print('transposed slicer', same_digits(ops.ozaki_slice_t(Xr, sq_, 7), slicing.slice_rows(W, 7)))
 Xu = ops.synth_design(4, 0, 70001, 650, dev)
 print('syrk unweighted', rel(ops.syrk_weighted(Xu, None, precision='f64_ozaki'), ops.syrk_weighted(Xu, None)))
 # batched CG with a Jacobi preconditioner

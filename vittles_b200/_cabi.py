@@ -55,8 +55,7 @@ SIGNATURES = {
     'vt_syrk_tf32_workspace_bytes': (_SZ, [_I64, _I, _I]),
     'vt_syrk_tf32': (_I, [_P, _I64, _I64, _I, _P, _D, _P, _I64, _I, _P, _SZ, _P]),
     'vt_ozaki_slice': (_I, [_P, _I64, _I64, _I, _P, _I64, _I64, _I, _P, _P, _P]),
-    'vt_ozaki_slice_int': (_I, [_P, _I64, _I64, _I, _P, _I64, _I64, _I, _P, _P, _P]),
-    'vt_ozaki_slice_t': (_I, [_P, _I64, _I64, _I, _P, _P, _P, _I64, _I64, _I, _P, _I, _P]),
+    'vt_ozaki_slice_t': (_I, [_P, _I64, _I64, _I, _P, _P, _P, _I64, _I64, _I, _P, _P]),
     'vt_ozaki_gemm': (_I, [_I, _I, _I, _P, _I64, _I64, _P, _I64, _I64, _I, _D, _P, _P, _P, _I64, _P]),
     'vt_syrk_ozaki_workspace_bytes': (_SZ, [_I64, _I, _I]),
     'vt_syrk_ozaki': (_I, [_P, _I64, _I64, _I, _P, _D, _P, _I64, _I, _P, _P, _P, _SZ, _P]),

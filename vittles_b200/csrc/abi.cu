@@ -44,7 +44,7 @@ static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s)
 extern "C" {
 
 const char* vt_last_error(void) { return vt::last_error(); }
-int vt_abi_version(void) { return 1; }
+int vt_abi_version(void) { return 2; }
 int64_t vt_launch_count(void) { return (int64_t)vt::launch_count(); }
 
 int vt_device_info(int* sm_count, int* cc_major, int* cc_minor) {
@@ -262,16 +262,10 @@ int vt_ozaki_slice(const double* X, int64_t ldx, int64_t rows, int cols, int8_t*
   return ozaki_slice(X, ldx, rows, cols, out, ldo, slice_stride, nslices, scale_out, fold, S(stream));
 }
 
-int vt_ozaki_slice_int(const double* X, int64_t ldx, int64_t rows, int cols, int8_t* out, int64_t ldo, int64_t slice_stride,
-                       int nslices, double* scale_out, const double* fold, void* stream) {
-  return ozaki_slice(X, ldx, rows, cols, out, ldo, slice_stride, nslices, scale_out, fold, S(stream), 1);
-}
-
 int vt_ozaki_slice_t(const double* X, int64_t ldx, int64_t rows, int cols, const double* sq, const uint64_t* colmax,
-                     int8_t* out, int64_t ldo, int64_t slice_stride, int nslices, double* scale_out, int integer_variant,
-                     void* stream) {
+                     int8_t* out, int64_t ldo, int64_t slice_stride, int nslices, double* scale_out, void* stream) {
   return ozaki_slice_t(X, ldx, rows, cols, sq, reinterpret_cast<const unsigned long long*>(colmax), out, ldo, slice_stride,
-                       nslices, scale_out, integer_variant, S(stream));
+                       nslices, scale_out, S(stream));
 }
 
 int vt_ozaki_gemm(int M, int N, int K, const int8_t* A, int64_t lda, int64_t a_slice_stride, const int8_t* B,

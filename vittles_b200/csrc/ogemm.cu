@@ -102,38 +102,24 @@ __device__ __forceinline__ OUnit o_decode(const OKernelArgs& a, long u) {
 // q = sum_p d_p 256^p with every d_p in [-128, 127]: with the bias B = sum_p 128 256^p the ordinary bytes e_p of
 // u = q + B are d_p + 128, i.e. the digits are the bytes of u ^ B.  An int8 digit then carries a full 8 bits
 // (sign-magnitude digits carry 7), so 7 slices hold 54 bits and S (S + 1) / 2 = 28 digit products do the work
-// of the 36 that 8 sign-magnitude slices need.  The scaling by a power of two is exact, rint rounds once, and
-// q is assembled from two 32-bit conversions (hi = rint(t 2^-24), lo = rint(t - hi 2^24), both exact; a 64-bit
-// conversion is emulated in software and made the slicers instruction bound).  Slice `sl` (0 = most significant
+// of the 36 that 8 sign-magnitude slices need.
+// The row maximum, its exponent and q are formed with integer instructions only, from the bit patterns: the
+// converter warps of the GEMM kernel slice next to a saturated tensor pipe, where FP64 instructions of other warps
+// wait ~60 clocks each for their pipe (ncu: stall_math_pipe_throttle on every DMUL / DFMA / DADD of the converters)
+// while the integer pipe is idle, and the stand-alone slicers run the same code so that there is one rounding rule.
+// x = +-M 2^(eb - 1075) with the 53-bit significand M, so t = x 2^(8S-2-e) = 2M >> n with n = k2 - eb,
+// k2 = e + 1078 - 8S, rounded to nearest even by adding half an ulp minus one plus the bit that would become the
+// last (n >= 0 because |x| < 2^e, except in a row whose maximum is subnormal, where the shift goes left).
+// u = q + B is kept as two words, lo = positions 0..3 and hi = positions 4..S-1; slice `sl` (0 = most significant
 // of `nslices`) of four values is packed with PRMT into one word (byte j = value j).
 // (oracle/slicing.py is the CPU model; tests/test_gpu_ozaki.py compares digit for digit.)
 struct Fixed4 {
-  uint32_t lo[4], hi[4];       // biased digits: positions 0..NLO-1 in the low bytes of lo, the rest in the bytes of hi
-                               // (NLO = 3 from fixed4_set, 4 from fixed4_set_bits)
+  uint32_t lo[4], hi[4];       // biased digits: positions 0..3 in the bytes of lo, the rest in the bytes of hi
 };
-// bias of the S - 3 digits kept in the high word
-__host__ __device__ constexpr uint32_t digit_bias_hi(int nslices) { return 0x80808080u >> (8 * (7 - nslices)); }
-// t = x * 2^(8S-2) / sigma, |t| <= 2^(8S-2).  Round-to-nearest-even through the FP64 adder: v + 1.5 2^52 holds
-// rint(v) in the low word of its significand for |v| < 2^51 (no conversion instructions: those issue at a quarter
-// of the FP64 rate).  q = hi 2^24 + lo with |lo| <= 2^23; the balanced digits of lo are the bytes of lo + 0x808080
-// minus 128 each, and what that sum carries beyond 24 bits (0 or 1) goes to hi - everything in 32-bit integers.
-__device__ __forceinline__ void fixed4_set(Fixed4& f, int j, double t, uint32_t bias_hi) {
-  constexpr double MAGIC = 6755399441055744.0;                       // 1.5 * 2^52
-  const double mh = fma(t, 1.0 / 16777216.0, MAGIC);                // rint(t 2^-24), |.| <= 2^30
-  const int hi = __double2loint(mh);
-  const double rem = fma(-(mh - MAGIC), 16777216.0, t);             // exact, |rem| <= 2^23
-  const int lo = __double2loint(rem + MAGIC);
-  const uint32_t ulo = (uint32_t)lo + 0x00808080u;                  // in [0x8080, 0x1008080]
-  f.lo[j] = ulo;
-  f.hi[j] = (uint32_t)hi + (ulo >> 24) + bias_hi;
+// |x| as an unsigned integer orders like the double; Inf and NaN sit above every finite value
+__device__ __forceinline__ unsigned long long abs_bits(double x) {
+  return (unsigned long long)__double_as_longlong(x) & 0x7fffffffffffffffULL;
 }
-// The same digits with integer instructions only, for the converter warps of the GEMM kernel: while the tensor
-// pipe is saturated, FP64 instructions of other warps wait ~60 clocks each for their pipe (ncu: stall_math_pipe_throttle
-// on every DMUL / DFMA / DADD of the converters), the integer pipe is idle.  x = +-M 2^(eb - 1075) with the 53-bit
-// significand M, so t = 2M >> n with n = k2 - eb, k2 = e + 1078 - 8S, rounded to nearest even by adding half an ulp
-// minus one plus the bit that would become the last (n >= 0 because |x| < 2^e, except in a row whose maximum is
-// subnormal, where the shift goes left).  Here lo holds the positions 0..3 and hi the positions 4..S-1 (NLO = 4 in
-// fixed4_digits).
 // frexp exponent of a finite non-negative double given by its bit pattern (0 for zero), in integer instructions
 __device__ __forceinline__ int frexp_exponent_bits(unsigned long long mb) {
   const int eb = (int)(mb >> 52);
@@ -155,13 +141,13 @@ __device__ __forceinline__ void fixed4_set_bits(Fixed4& f, int j, unsigned long 
   f.lo[j] = (uint32_t)u;
   f.hi[j] = (uint32_t)(u >> 32);
 }
-template <int S, int NLO = 3>
+template <int S>
 __device__ __forceinline__ uint32_t fixed4_digits(const Fixed4& f, int sl) {
   const int pos = S - 1 - sl;                      // digit position from the least significant one
-  const uint32_t sel = (uint32_t)(pos < NLO ? pos : pos - NLO);
+  const uint32_t sel = (uint32_t)(pos < 4 ? pos : pos - 4);
   const uint32_t pick = sel | ((4u + sel) << 4);   // PRMT: byte `sel` of the first source, byte `sel` of the second
   uint32_t p01, p23;
-  if (pos < NLO) {
+  if (pos < 4) {
     p01 = __byte_perm(f.lo[0], f.lo[1], pick);
     p23 = __byte_perm(f.lo[2], f.lo[3], pick);
   } else {
@@ -174,15 +160,11 @@ __device__ __forceinline__ uint32_t fixed4_digits(const Fixed4& f, int sl) {
 // One warp per row: row maximum -> power-of-two scale -> S balanced base-256 digits,
 // so that 2^-6 sum_s d_s 2^{-8s} reproduces x / sigma to 8 S - 2 bits (round to nearest).
 // Rows of at most 128 * RC elements are held in registers between the two passes (RC = 0: re-read).
-// INTEGER: maximum and digits with integer instructions only (fixed4_set_bits; same digits).
-template <int S, int RC, bool INTEGER = false>
+template <int S, int RC>
 __device__ __forceinline__ void slice_one_row(const SliceJob& jb, long r, int lane, bool vec) {
-  static_assert(!INTEGER || RC > 0, "the integer slicer keeps the row in registers");
-  constexpr uint32_t bias = digit_bias_hi(S);
   const double* xr = jb.X + r * jb.ldx;
   const int cols = jb.cols;
-  double m = 0.0;
-  bool finite = true;                                // fmax() drops NaNs: track non-finite entries separately
+  unsigned long long mb = 0ULL;                      // bit pattern of the row maximum of |x|
   double xv[RC > 0 ? RC : 1][4];
   if constexpr (RC > 0) {
 #pragma unroll
@@ -196,54 +178,27 @@ __device__ __forceinline__ void slice_one_row(const SliceJob& jb, long r, int la
         for (int j = 0; j < 4; ++j) xv[ch][j] = (c0 + j < cols) ? xr[c0 + j] : 0.0;
       }
     }
-    if constexpr (INTEGER) {
-      // |x| as an unsigned integer orders like the double; Inf and NaN sit above every finite value
-      unsigned long long mb = 0ULL;
 #pragma unroll
-      for (int ch = 0; ch < RC; ++ch)
+    for (int ch = 0; ch < RC; ++ch)
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const unsigned long long b = (unsigned long long)__double_as_longlong(xv[ch][j]) & 0x7fffffffffffffffULL;
-          mb = b > mb ? b : mb;
-        }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        const unsigned long long other = __shfl_xor_sync(0xffffffffu, mb, o);
-        mb = other > mb ? other : mb;
+      for (int j = 0; j < 4; ++j) {
+        const unsigned long long b = abs_bits(xv[ch][j]);
+        mb = b > mb ? b : mb;
       }
-      finite = mb < 0x7ff0000000000000ULL;
-      m = finite ? __longlong_as_double((long long)mb) : 0.0;
-    } else {
-#pragma unroll
-      for (int ch = 0; ch < RC; ++ch)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const double v = fabs(xv[ch][j]);
-          finite = finite && (v <= 1.7976931348623157e308);
-          m = fmax(m, v);
-        }
-    }
   } else {
     for (int c = lane; c < cols; c += 32) {
-      const double v = fabs(xr[c]);
-      finite = finite && (v <= 1.7976931348623157e308);
-      m = fmax(m, v);
+      const unsigned long long b = abs_bits(xr[c]);
+      mb = b > mb ? b : mb;
     }
   }
-  if constexpr (!INTEGER) {
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-    finite = __all_sync(0xffffffffu, finite);
+  for (int o = 16; o > 0; o >>= 1) {
+    const unsigned long long other = __shfl_xor_sync(0xffffffffu, mb, o);
+    mb = other > mb ? other : mb;
   }
+  const bool finite = mb < 0x7ff0000000000000ULL;
   int e = 0;
-  if constexpr (INTEGER) {
-    if (finite) e = frexp_exponent_bits((unsigned long long)__double_as_longlong(m));
-  } else {
-    if (finite && m > 0.0) (void)frexp(m, &e);       // m = f 2^e, f in [0.5, 1)  ->  |x| 2^-e < 1
-  }
-  // |x * up * up2| <= 2^(8S-2); the power of two goes in two factors because rows below ~1e-290 need more than 2^1023
-  const int sh = 8 * S - 2 - e;
-  const double up = ldexp(1.0, sh > 1000 ? 1000 : sh), up2 = ldexp(1.0, sh > 1000 ? sh - 1000 : 0);
+  if (finite) e = frexp_exponent_bits(mb);
   // a row with an Inf or NaN gets a NaN scale: every result that touches it is NaN, as in FP64 arithmetic
   if (lane == 0)
     jb.scale_out[r] = finite ? ldexp(1.0, e) * (jb.fold ? jb.fold[r] : 1.0) : __longlong_as_double(0x7ff8000000000000LL);
@@ -255,27 +210,21 @@ __device__ __forceinline__ void slice_one_row(const SliceJob& jb, long r, int la
       const int c0 = ch * 128 + lane * 4;
       if (c0 < jb.ldo) {
         Fixed4 f;
-        if constexpr (INTEGER) {
 #pragma unroll
-          for (int j = 0; j < 4; ++j)
-            fixed4_set_bits(f, j, (unsigned long long)__double_as_longlong(xv[ch][j]), e + 1078 - 8 * S, digit_bias64(S));
+        for (int j = 0; j < 4; ++j)
+          fixed4_set_bits(f, j, (unsigned long long)__double_as_longlong(xv[ch][j]), e + 1078 - 8 * S, digit_bias64(S));
 #pragma unroll
-          for (int s = 0; s < S; ++s)
-            *reinterpret_cast<uint32_t*>(orow + (long)s * jb.slice_stride + c0) = fixed4_digits<S, 4>(f, s);
-        } else {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) fixed4_set(f, j, xv[ch][j] * up * up2, bias);
-#pragma unroll
-          for (int s = 0; s < S; ++s)
-            *reinterpret_cast<uint32_t*>(orow + (long)s * jb.slice_stride + c0) = fixed4_digits<S>(f, s);
-        }
+        for (int s = 0; s < S; ++s)
+          *reinterpret_cast<uint32_t*>(orow + (long)s * jb.slice_stride + c0) = fixed4_digits<S>(f, s);
       }
     }
   } else {
     for (int c0 = lane * 4; c0 < jb.ldo; c0 += 128) {
       Fixed4 f;
 #pragma unroll
-      for (int j = 0; j < 4; ++j) fixed4_set(f, j, (c0 + j < cols) ? xr[c0 + j] * up * up2 : 0.0, bias);
+      for (int j = 0; j < 4; ++j)
+        fixed4_set_bits(f, j, (c0 + j < cols) ? (unsigned long long)__double_as_longlong(xr[c0 + j]) : 0ULL,
+                        e + 1078 - 8 * S, digit_bias64(S));
 #pragma unroll
       for (int s = 0; s < S; ++s)
         *reinterpret_cast<uint32_t*>(orow + (long)s * jb.slice_stride + c0) = fixed4_digits<S>(f, s);
@@ -283,13 +232,19 @@ __device__ __forceinline__ void slice_one_row(const SliceJob& jb, long r, int la
   }
 }
 
-template <int S, int RC, bool INTEGER = false>
+template <int S, int RC>
 __global__ void __launch_bounds__(256) ozaki_slice_kernel(const SliceJob jb) {
   const int lane = threadIdx.x & 31;
   const long warp0 = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long nwarps = ((long)gridDim.x * blockDim.x) >> 5;
   const bool vec = (jb.ldx % 2 == 0) && (reinterpret_cast<uintptr_t>(jb.X) % 16 == 0);
-  for (long r = warp0; r < jb.rows; r += nwarps) slice_one_row<S, RC, INTEGER>(jb, r, lane, vec);
+  for (long r = warp0; r < jb.rows; r += nwarps) slice_one_row<S, RC>(jb, r, lane, vec);
+}
+// rows of up to 1024 elements stay in registers, narrow rows in an instance with fewer of them
+template <int S>
+void (*row_slicer(int cols))(SliceJob) {
+  return cols <= 128 ? ozaki_slice_kernel<S, 1> : cols <= 256 ? ozaki_slice_kernel<S, 2>
+       : cols <= 512 ? ozaki_slice_kernel<S, 4> : cols <= 1024 ? ozaki_slice_kernel<S, 8> : ozaki_slice_kernel<S, 0>;
 }
 
 // Tile of 32 observations x 32 features per warp, lane = feature: 32 coalesced 256-byte reads (all in flight at
@@ -298,9 +253,8 @@ __global__ void __launch_bounds__(256) ozaki_slice_kernel(const SliceJob jb) {
 // memory, so the converter warps of the GEMM kernel can run it next to the operand ring.  Observations past `rows`
 // are written as zeros up to the next multiple of 16 (the GEMM's tensor map ends at `rows` anyway).
 constexpr int ST_OBS = 32, ST_FEAT = 32, ST_GROUP = 8;      // a CTA step: ST_GROUP consecutive tiles along the observations
-template <int S, bool INTEGER>
+template <int S>
 __device__ __forceinline__ void slice_t_tile(const SliceJob& jb, long n0, int i0, int lane, bool first) {
-  constexpr uint32_t bias = digit_bias_hi(S);
   const int i = i0 + lane;
   const bool live = i < jb.cols;
   int e = 0;
@@ -308,21 +262,15 @@ __device__ __forceinline__ void slice_t_tile(const SliceJob& jb, long n0, int i0
     const unsigned long long mb = jb.colmax[i];
     const double m = __longlong_as_double((long long)mb);
     const bool finite = mb < 0x7ff0000000000000ULL;
-    if constexpr (INTEGER) {
-      if (finite) e = frexp_exponent_bits(mb);
-    } else {
-      if (finite && m > 0.0) (void)frexp(m, &e);
-    }
+    if (finite) e = frexp_exponent_bits(mb);
     if (first) jb.scale_out[i] = finite ? ldexp(1.0, e) : m;   // NaN scale: row and column i of H become NaN
   }
-  const int sh = 8 * S - 2 - e;
-  const double up = ldexp(1.0, sh > 1000 ? 1000 : sh), up2 = ldexp(1.0, sh > 1000 ? sh - 1000 : 0);   // (see slice_one_row)
   double xv[ST_OBS];
   if ((n0 + ST_OBS <= jb.rows) && (i0 + ST_FEAT <= jb.cols)) {
     const double* xp = jb.X + n0 * jb.ldx + i;
 #pragma unroll
     for (int q = 0; q < ST_OBS; ++q) xv[q] = xp[q * jb.ldx];
-    if (jb.sq) {                  // (unweighted: no FP64 instruction per element at all)
+    if (jb.sq) {                  // the one FP64 instruction per element (unweighted: none at all)
 #pragma unroll
       for (int q = 0; q < ST_OBS; ++q) xv[q] *= jb.sq[n0 + q];
     }
@@ -340,21 +288,16 @@ __device__ __forceinline__ void slice_t_tile(const SliceJob& jb, long n0, int i0
 #pragma unroll
     for (int g4 = 0; g4 < 4; ++g4)
 #pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        if constexpr (INTEGER)     // (the product with sqrt(s_n) above is the one FP64 instruction per element left)
-          fixed4_set_bits(f[g4], j, (unsigned long long)__double_as_longlong(xv[16 * h + 4 * g4 + j]), e + 1078 - 8 * S,
-                          digit_bias64(S));
-        else
-          fixed4_set(f[g4], j, xv[16 * h + 4 * g4 + j] * up * up2, bias);
-      }
+      for (int j = 0; j < 4; ++j)
+        fixed4_set_bits(f[g4], j, (unsigned long long)__double_as_longlong(xv[16 * h + 4 * g4 + j]), e + 1078 - 8 * S,
+                        digit_bias64(S));
     if (live && n0 + 16 * h < jb.rows) {
       int8_t* o = jb.out + (long)i * jb.ldo + n0 + 16 * h;
 #pragma unroll
       for (int sl = 0; sl < S; ++sl) {
-        constexpr int NLO = INTEGER ? 4 : 3;
         uint4 w;
-        w.x = fixed4_digits<S, NLO>(f[0], sl); w.y = fixed4_digits<S, NLO>(f[1], sl);
-        w.z = fixed4_digits<S, NLO>(f[2], sl); w.w = fixed4_digits<S, NLO>(f[3], sl);
+        w.x = fixed4_digits<S>(f[0], sl); w.y = fixed4_digits<S>(f[1], sl);
+        w.z = fixed4_digits<S>(f[2], sl); w.w = fixed4_digits<S>(f[3], sl);
         *reinterpret_cast<uint4*>(o + (long)sl * jb.slice_stride) = w;
       }
     }
@@ -362,14 +305,14 @@ __device__ __forceinline__ void slice_t_tile(const SliceJob& jb, long n0, int i0
 }
 
 // CTA steps (feature blocks fastest: a wave reads whole rows of X), `nw` warps of which this one is `w`
-template <int S, bool INTEGER>
+template <int S>
 __device__ __forceinline__ void slice_t_job(const SliceJob& jb, long cta, long nctas, int w, int nw, int lane) {
   const long span = (long)ST_OBS * nw;
   const long steps_x = (jb.rows + span - 1) / span;
   const int tiles_y = (jb.cols + ST_FEAT - 1) / ST_FEAT;
   for (long t = cta; t < steps_x * tiles_y; t += nctas) {
     const long n0 = (t / tiles_y) * span + (long)w * ST_OBS;
-    if (n0 < jb.rows) slice_t_tile<S, INTEGER>(jb, n0, (int)(t % tiles_y) * ST_FEAT, lane, t < tiles_y && w == 0);
+    if (n0 < jb.rows) slice_t_tile<S>(jb, n0, (int)(t % tiles_y) * ST_FEAT, lane, t < tiles_y && w == 0);
   }
 }
 
@@ -596,10 +539,10 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
     const bool vec = (a.next.ldx % 2 == 0) && (reinterpret_cast<uintptr_t>(a.next.X) % 16 == 0);
     const long long t_begin = clock64();
     if (a.next.colmax) {
-      slice_t_job<S, true>(a.next, blockIdx.x, gridDim.x, cw, O_CONV_WARPS, lane);
+      slice_t_job<S>(a.next, blockIdx.x, gridDim.x, cw, O_CONV_WARPS, lane);
     } else {
       for (long r = (long)blockIdx.x * O_CONV_WARPS + cw; r < a.next.rows; r += (long)gridDim.x * O_CONV_WARPS)
-        slice_one_row<S, 8, true>(a.next, r, lane, vec);
+        slice_one_row<S, 8>(a.next, r, lane, vec);
     }
     if (a.timing && lane == 0) {
       atomicAdd(a.timing + 5, (unsigned long long)(clock64() - t_begin));
@@ -667,9 +610,9 @@ __global__ void __launch_bounds__(256) ozaki_colmax_kernel(const double* __restr
   }
 }
 
-template <int S, bool INTEGER = false>
+template <int S>
 __global__ void __launch_bounds__(32 * ST_GROUP) ozaki_slice_t_kernel(const SliceJob jb) {
-  slice_t_job<S, INTEGER>(jb, blockIdx.x, gridDim.x, threadIdx.x >> 5, ST_GROUP, threadIdx.x & 31);
+  slice_t_job<S>(jb, blockIdx.x, gridDim.x, threadIdx.x >> 5, ST_GROUP, threadIdx.x & 31);
 }
 
 // H = sum of the split-K partial buffers over the lower triangle, mirrored (exactly symmetric).
@@ -759,7 +702,7 @@ long ozaki_chunk_rows(long N, int D, int nslices) {
 unsigned long long* ogemm_timing_buffer_public() { return ogemm_timing_buffer(); }
 
 int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, long ldo, long slice_stride, int nslices,
-                double* scale_out, const double* fold, cudaStream_t stream, int integer_variant) {
+                double* scale_out, const double* fold, cudaStream_t stream) {
   VT_REQUIRE(X && out && scale_out, "ozaki_slice: null pointer");
   VT_REQUIRE(rows >= 0 && cols >= 1 && ldx >= cols && ldo >= cols && ldo % 16 == 0, "ozaki_slice: bad shape");
   VT_REQUIRE(nslices >= OZAKI_MIN_SLICES && nslices <= OZAKI_MAX_SLICES && slice_stride >= rows * ldo && slice_stride % 16 == 0,
@@ -770,42 +713,16 @@ int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, lon
   long blocks = (rows + bt / 32 - 1) / (bt / 32);
   const long cap = (long)num_sms() * 8;
   if (blocks > cap) blocks = cap;
-  const int rc = cols <= 1024 ? (cols + 127) / 128 : 0;        // rows of up to 1024 elements stay in registers
   const SliceJob jb{X, ldx, rows, cols, out, ldo, slice_stride, scale_out, fold, nullptr, nullptr};
-  if (integer_variant) {       // the converter warps' instruction sequence as a kernel of its own (tests)
-    VT_REQUIRE(cols <= 1024, "ozaki_slice: the integer variant takes rows of at most 1024 elements");
-    switch (nslices) {
-      case 5: ozaki_slice_kernel<5, 8, true><<<(unsigned)blocks, bt, 0, stream>>>(jb); break;
-      case 6: ozaki_slice_kernel<6, 8, true><<<(unsigned)blocks, bt, 0, stream>>>(jb); break;
-      default: ozaki_slice_kernel<7, 8, true><<<(unsigned)blocks, bt, 0, stream>>>(jb); break;
-    }
-    VT_LAUNCH_CHECK();
-    return VT_OK;
-  }
-#define VT_SLICE_CASE(SS, RR) ozaki_slice_kernel<SS, RR><<<(unsigned)blocks, bt, 0, stream>>>(jb)
-#define VT_SLICE_S(SS)                                                           \
-  switch (rc) {                                                                  \
-    case 1: VT_SLICE_CASE(SS, 1); break;                                         \
-    case 2: VT_SLICE_CASE(SS, 2); break;                                         \
-    case 3: case 4: VT_SLICE_CASE(SS, 4); break;                                 \
-    case 5: case 6: case 7: case 8: VT_SLICE_CASE(SS, 8); break;                 \
-    default: VT_SLICE_CASE(SS, 0); break;                                        \
-  }
-  switch (nslices) {
-    case 5: VT_SLICE_S(5); break;
-    case 6: VT_SLICE_S(6); break;
-    default: VT_SLICE_S(7); break;
-  }
-#undef VT_SLICE_S
-#undef VT_SLICE_CASE
+  const auto kern = nslices == 5 ? row_slicer<5>(cols) : nslices == 6 ? row_slicer<6>(cols) : row_slicer<7>(cols);
+  kern<<<(unsigned)blocks, bt, 0, stream>>>(jb);
   VT_LAUNCH_CHECK();
   return VT_OK;
 }
 
 // Transposed digits out[s][feature][observation] of sq_n x_ni (the Hessian's operand) as a launch of its own.
 int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* sq, const unsigned long long* colmax,
-                  int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, int integer_variant,
-                  cudaStream_t stream) {
+                  int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, cudaStream_t stream) {
   VT_REQUIRE(X && colmax && out && scale_out, "ozaki_slice_t: null pointer");      // sq == nullptr: unweighted
   VT_REQUIRE(rows >= 1 && cols >= 1 && ldx >= cols && ldo >= rows && ldo % 16 == 0 && slice_stride >= (long)cols * ldo &&
              slice_stride % 16 == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0, "ozaki_slice_t: bad layout");
@@ -814,15 +731,8 @@ int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* 
   const long steps = ((rows + ST_OBS * ST_GROUP - 1) / (ST_OBS * ST_GROUP)) * ((cols + ST_FEAT - 1) / ST_FEAT);
   const long cap = (long)num_sms() * 6;
   const unsigned grid = (unsigned)(steps < cap ? steps : cap);
-#define VT_SLICE_T(SS)                                                                              \
-  if (integer_variant) ozaki_slice_t_kernel<SS, true><<<grid, 32 * ST_GROUP, 0, stream>>>(jb);     \
-  else ozaki_slice_t_kernel<SS, false><<<grid, 32 * ST_GROUP, 0, stream>>>(jb)
-  switch (nslices) {
-    case 5: VT_SLICE_T(5); break;
-    case 6: VT_SLICE_T(6); break;
-    default: VT_SLICE_T(7); break;
-  }
-#undef VT_SLICE_T
+  const auto kern = nslices == 5 ? ozaki_slice_t_kernel<5> : nslices == 6 ? ozaki_slice_t_kernel<6> : ozaki_slice_t_kernel<7>;
+  kern<<<grid, 32 * ST_GROUP, 0, stream>>>(jb);
   VT_LAUNCH_CHECK();
   return VT_OK;
 }
@@ -1153,7 +1063,7 @@ int syrk_ozaki(const double* X, long ldx, long N, int D, const double* s, double
     const long rows = (N - r0 < p.chunk) ? N - r0 : p.chunk;
     if (c == 0) {
       const SliceJob jb = job(r0, b);
-      st = ozaki_slice_t(jb.X, ldx, jb.rows, D, jb.sq, cmax_use, Xs[b], p.ld, slice_stride, nslices, sigma, 0, stream);
+      st = ozaki_slice_t(jb.X, ldx, jb.rows, D, jb.sq, cmax_use, Xs[b], p.ld, slice_stride, nslices, sigma, stream);
       if (st != VT_OK) return st;
     }
     OLaunchOpts o;

@@ -27,12 +27,10 @@ constexpr int OZAKI_MAX_K = 16384;      // (K + 128) * 128^2 * S < 2^31
 // digits of every row of X (rows x cols, FP64): out[s][r][k] (int8, row pitch ldo bytes, a multiple of 16; pad bytes
 // are zero), scale_out[r] = sigma_r (* fold[r] if fold != nullptr).
 int ozaki_slice(const double* X, long ldx, long rows, int cols, int8_t* out, long ldo, long slice_stride, int nslices,
-                double* scale_out, const double* fold, cudaStream_t stream, int integer_variant = 0);
+                double* scale_out, const double* fold, cudaStream_t stream);
 // out[s][feature][observation] of sq_n x_ni with one scale per feature from colmax (bit patterns of the maxima).
-// integer_variant: the integer-only instruction sequence of the GEMM kernel's converter warps (same digits).
 int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* sq, const unsigned long long* colmax,
-                  int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, int integer_variant,
-                  cudaStream_t stream);
+                  int8_t* out, long ldo, long slice_stride, int nslices, double* scale_out, cudaStream_t stream);
 
 // C (M x N, FP64) = alpha * rowscale[m] * colscale[n] * 2^-12 sum_{s+t<S} 2^{-8(s+t)} (A_s B_t^T)(m,n)
 int ogemm_launch(int M, int N, int K, const int8_t* A, long lda, long a_slice_stride, const int8_t* B, long ldb,

@@ -171,24 +171,21 @@ def tf32_gemm(A, B, amode='KC', bmode='KC', alpha=1.0, precision='tf32', colscal
 
 
 # ------------------------------------- INT8 error-free slicing (optional) ----
-def ozaki_slice(X, nslices=OZAKI_SLICES, fold=None, integer_variant=False):
+def ozaki_slice(X, nslices=OZAKI_SLICES, fold=None):
     """(digits (nslices, rows, ld) int8, scale (rows,) float64) of a float64 matrix:
     X[r, k] = scale[r] * 2^-6 sum_s digits[s, r, k] 2^{-8 s} up to scale[r] 2^{-(8 nslices - 1)}
-    (``fold`` multiplies the returned scale row by row).  ``integer_variant``: the
-    integer-only instruction sequence that the GEMM kernel's converter warps run
-    (same digits; rows of at most 1024 elements)."""
+    (``fold`` multiplies the returned scale row by row)."""
     lib = _cabi.require_cuda()
     _mat(X, 'X')
     rows, cols = X.shape
     ld = (cols + 15) // 16 * 16
     out = torch.empty((nslices, rows, ld), dtype=torch.int8, device=X.device)
     scale = torch.empty(rows, dtype=torch.float64, device=X.device)
-    fn = lib.vt_ozaki_slice_int if integer_variant else lib.vt_ozaki_slice
-    check(fn(ptr(X), _ld(X), rows, cols, ptr(out), ld, rows * ld, nslices, ptr(scale), ptr(fold), stream()))
+    check(lib.vt_ozaki_slice(ptr(X), _ld(X), rows, cols, ptr(out), ld, rows * ld, nslices, ptr(scale), ptr(fold), stream()))
     return out, scale
 
 
-def ozaki_slice_t(X, sq, nslices=OZAKI_SLICES, integer_variant=False):
+def ozaki_slice_t(X, sq, nslices=OZAKI_SLICES):
     """The Hessian's operand: (digits (nslices, cols, ld) int8, scale (cols,) float64) of
     sq[n] * X[n, i] (sq None: of X[n, i]), transposed (observations contiguous), one power-of-two scale per feature."""
     lib = _cabi.require_cuda()
@@ -204,7 +201,7 @@ def ozaki_slice_t(X, sq, nslices=OZAKI_SLICES, integer_variant=False):
     out = torch.zeros((nslices, cols, ld), dtype=torch.int8, device=X.device)
     scale = torch.empty(cols, dtype=torch.float64, device=X.device)
     check(lib.vt_ozaki_slice_t(ptr(X), _ld(X), rows, cols, ptr(sq), ptr(cmax), ptr(out), ld, cols * ld, nslices,
-                               ptr(scale), 1 if integer_variant else 0, stream()))
+                               ptr(scale), stream()))
     return out, scale
 
 
