@@ -94,11 +94,21 @@ def glm_objective(X, y, family='logistic', l2=0.0):
     return f
 
 
+def _sigmoid_pair(z):
+    """(sigma(z), sigma(-z), b''(z) = sigma(z) sigma(-z)), all from e = exp(-|z|): 1 - sigma(z) is never formed, so
+    nothing cancels in either tail (p (1 - p) loses e^z of its relative accuracy for z > 0)."""
+    z = np.asarray(z, dtype=np.float64)
+    e = np.exp(-np.abs(z))
+    d = 1.0 + e
+    pos = z >= 0
+    return np.where(pos, 1.0 / d, e / d), np.where(pos, e / d, 1.0 / d), e / (d * d)
+
+
 def glm_mean_var(z, family):
     """b'(z), b''(z)."""
     if family == 'logistic':
-        p = 1.0 / (1.0 + np.exp(-z))
-        return p, p * (1.0 - p)
+        p, _, var = _sigmoid_pair(z)
+        return p, var
     if family == 'poisson':
         e = np.exp(z)
         return e, e
@@ -107,13 +117,22 @@ def glm_mean_var(z, family):
     raise ValueError(family)
 
 
+def glm_resid(z, y, family):
+    """b'(z) - y.  Logistic: (1 - y) sigma(z) - y sigma(-z), equal for every y and free of the cancellation of
+    sigma(z) - 1 at y = 1."""
+    if family == 'logistic':
+        p, q, _ = _sigmoid_pair(z)
+        return (1.0 - y) * p - y * q
+    return glm_mean_var(z, family)[0] - y
+
+
 def glm_closed_form(X, y, theta, w, family='logistic', l2=0.0):
     """Closed forms the CUDA kernels implement: gradient, Hessian
     ``X^T diag(w b''(z)) X`` and the (D, N) cross-Hessian whose column n is
     ``(b'(z_n) - y_n) x_n`` (the per-observation gradient)."""
     z = X @ theta
-    mu, var = glm_mean_var(z, family)
-    r = mu - y
+    var = glm_mean_var(z, family)[1]
+    r = glm_resid(z, y, family)
     grad = X.T @ (w * r) + l2 * theta
     H = X.T @ ((w * var)[:, None] * X) + l2 * np.eye(X.shape[1])
     cross = (X * r[:, None]).T

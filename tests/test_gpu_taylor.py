@@ -110,14 +110,33 @@ def test_dirderiv_and_hvp_kernels_vs_oracle(vt, n, d):
     eps = np.array([0.3, -0.1])
     obj = vt.objectives.GLMPriorObjective(X, y)
     g_torch = torch.func.grad(models.hier_glm_objective(X, y), argnums=0)
-    dirs = [rng.normal(size=d) / np.sqrt(d) * 3 for _ in range(3)]
+    dirs = [rng.normal(size=d) / np.sqrt(d) * 3 for _ in range(4)]
     de = [np.array([0.2, 0.5]), np.array([-0.4, 0.1])]
-    for m, ne in [(0, 0), (1, 0), (2, 0), (3, 0), (0, 1), (0, 2), (1, 1), (1, 2), (2, 1)]:
+    for m, ne in [(0, 0), (1, 0), (2, 0), (3, 0), (4, 0), (0, 1), (0, 2), (1, 1), (1, 2), (2, 1)]:
         ours = obj.vt_directional_derivative(theta, eps, dirs[:m], de[:ne])
         ref = osens.directional_derivative(g_torch, theta, eps, dirs[:m], de[:ne])
         assert_close(ours, ref, rtol=1e-8, atol_scale=1e-11, what='m={} n={}'.format(m, ne))
     hv = obj.vt_hvp_fn(theta, eps)(dirs[0])
     assert_close(hv, osens.directional_derivative(g_torch, theta, eps, dirs[:1], []), rtol=1e-9, atol_scale=1e-12)
+
+
+def test_poisson_dirderiv_vs_oracle(vt):
+    """The Poisson family's fused directional derivatives of orders 3-5 (q = 2..4 directions: b^(k) = exp for every
+    k) against the oracle's nested forward-mode JVPs."""
+    from oracle import models, sensitivity as osens
+    n, d = 2000, 48
+    rng = np.random.RandomState(4)
+    X = models.synth_design(6, 0, n, d)
+    theta = 0.7 * rng.normal(size=d)
+    y = rng.poisson(np.exp(X @ theta)).astype(np.float64)
+    eps = np.array([0.3, -0.1])
+    obj = vt.objectives.GLMPriorObjective(X, y, family='poisson')
+    g_torch = torch.func.grad(models.hier_glm_objective(X, y, family='poisson'), argnums=0)
+    dirs = [rng.normal(size=d) / np.sqrt(d) * 3 for _ in range(4)]
+    for m in (2, 3, 4):
+        ours = obj.vt_directional_derivative(theta, eps, dirs[:m], [])
+        ref = osens.directional_derivative(g_torch, theta, eps, dirs[:m], [])
+        assert_close(ours, ref, rtol=1e-8, atol_scale=1e-11, what='poisson m={}'.format(m))
 
 
 def test_weights_taylor_wls(vt):

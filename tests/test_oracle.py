@@ -266,3 +266,69 @@ def test_integer_designs_are_exact_in_float64_and_in_the_int8_model():
         dH, sH = slicing.slice_rows(Hinv, 7)
         dX, sX = slicing.slice_rows(X, 7)
         assert np.array_equal(-slicing.digits_gemm(dH, sH, dX, sX * r), S)
+
+
+# ------------------------------------------------------------------ the GLM family functions in both tails ----
+EPS = np.finfo(np.float64).eps
+TINY = 2.0 ** -1073                     # two units of the last subnormal place
+
+
+def _assert_f64(actual, ref, rtol, what, scale=None):
+    """|actual - ref| <= rtol * scale + 2^-1073 elementwise (scale = |ref| by default); infinities and NaNs equal."""
+    actual, ref = np.asarray(actual, dtype=np.float64), np.asarray(ref, dtype=np.float64)
+    finite = np.isfinite(ref)
+    assert np.array_equal(actual[~finite], ref[~finite], equal_nan=True), what + ': non-finite entries differ'
+    scale = np.abs(ref) if scale is None else np.broadcast_to(scale, ref.shape)
+    err = np.abs(actual[finite] - ref[finite])
+    tol = rtol * scale[finite] + TINY
+    bad = ~(err <= tol)
+    assert not bad.any(), '{}: {} entries off, worst err/tol {:.3g}'.format(what, int(bad.sum()),
+                                                                             float(np.max(err / tol)))
+
+
+def test_logistic_closed_form_is_the_derivative_of_softplus():
+    """The oracle's closed form b^(k) = P_k(sigma) (the identity the logistic kernels evaluate) against mpmath's
+    numerical differentiation of log1p(exp(t)), k = 2 .. 5, at 40 points of [-40, 40]."""
+    import mpmath
+    from oracle import highprec
+    zs = np.concatenate([np.linspace(-40.0, 40.0, 37), [-2.29, 1.32, 0.0]])
+    ref = {k: [] for k in range(2, 6)}
+    with mpmath.workdps(70):
+        for z in zs:
+            for k in range(2, 6):
+                closed = highprec._bderiv(z, k, 'logistic')
+                diff = mpmath.diff(lambda t: mpmath.log1p(mpmath.exp(t)), mpmath.mpf(z), k)
+                assert abs(closed - diff) <= mpmath.mpf(10) ** -30 * max(abs(diff), mpmath.mpf(10) ** -20), (z, k)
+                ref[k].append(float(diff))
+    for k in range(2, 6):                          # and its rounding to float64
+        r = np.array(ref[k])                       # (an exact zero of b^(k) comes out of diff as ~1e-70)
+        _assert_f64(highprec.glm_bderiv_mp(zs, k, 'logistic'), r, EPS, 'b^({})'.format(k), np.maximum(np.abs(r), 1e-40))
+
+
+def _tail_grid():
+    z = np.linspace(0.0, 745.0, 746)
+    z = np.concatenate([z, [1e-300, 0.5, 2.29, 36.7, 37.0, 708.4, 709.78, 745.13, 745.2]])
+    return np.concatenate([z, -z])
+
+
+def test_float64_oracles_are_accurate_in_both_tails():
+    """models.glm_mean_var / glm_resid (float64) and highprec.logistic_stats_ld (longdouble, rounded to float64)
+    against the mpmath functions over z in [-745, 745]: 4 eps everywhere.  Forming p (1 - p) or p - 1 loses e^z of the
+    relative accuracy for z > 0 (b''(z) would be 0 from z = 37 on)."""
+    from oracle import highprec
+    z = _tail_grid()
+    for fam in ('logistic', 'poisson', 'gaussian'):
+        zf = z[z < 709.78] if fam == 'poisson' else z
+        mu, var = models.glm_mean_var(zf, fam)
+        _assert_f64(mu, highprec.glm_bderiv_mp(zf, 1, fam), 4 * EPS, fam + " b'")
+        _assert_f64(var, highprec.glm_bderiv_mp(zf, 2, fam), 4 * EPS, fam + " b''")
+        for yv in (0.0, 1.0, 0.3):
+            ref = highprec.glm_resid_mp(zf, yv, fam)
+            scale = np.abs(ref) if (fam == 'logistic' and yv != 0.3) else np.abs(mu) + yv
+            _assert_f64(models.glm_resid(zf, yv, fam), ref, 4 * EPS, '{} resid y={}'.format(fam, yv), scale)
+    w = 0.37
+    for yv in (0.0, 1.0):
+        r_ld, s_ld = highprec.logistic_stats_ld(z, np.full_like(z, yv), np.full_like(z, w))
+        _assert_f64(r_ld.astype(np.float64), highprec.glm_resid_mp(z, yv, 'logistic'), 4 * EPS,
+                    'longdouble resid y={}'.format(yv))
+        _assert_f64(s_ld.astype(np.float64), highprec.glm_weight_mp(z, w, 'logistic'), 4 * EPS, 'longdouble s')

@@ -63,13 +63,15 @@ __device__ __forceinline__ double sigmoid(double z) {
   return e / (1.0 + e);
 }
 
-// k-th derivative of b at z (k >= 1)
+// k-th derivative of b at z (k >= 1).  Logistic, k >= 2: b^(k) has parity (-1)^k, so it is evaluated at -|z|, where
+// sigma <= 1/2 and P_k(sigma) does not cancel (at sigma(z) -> 1 the relative error of P_k(sigma(z)) grows like e^z).
 __device__ __forceinline__ double b_deriv(int family, int k, double z, const Poly& poly) {
   if (family == GLM_LOGISTIC) {
-    const double s = sigmoid(z);
+    if (k == 1) return sigmoid(z);
+    const double s = sigmoid(-fabs(z));
     double r = poly.c[poly.deg];
     for (int i = poly.deg - 1; i >= 0; --i) r = fma(r, s, poly.c[i]);
-    return r;
+    return (z > 0 && (k & 1)) ? -r : r;
   }
   if (family == GLM_POISSON) return exp(z);
   return k == 1 ? z : (k == 2 ? 1.0 : 0.0);
@@ -84,11 +86,21 @@ struct StatsOp {
   __device__ Aux load(long n) const { return Aux{y[n], w ? w[n] : 1.0}; }
   __device__ double eval(long n, const double* t, const Aux& a, double* s_out) const {
     const double zz = t[0];
-    double mu, var;
-    if (family == GLM_LOGISTIC) { mu = sigmoid(zz); var = mu * (1.0 - mu); }
-    else if (family == GLM_POISSON) { mu = exp(zz); var = mu; }
-    else { mu = zz; var = 1.0; }
-    const double r = mu - a.y;
+    double r, var;
+    if (family == GLM_LOGISTIC) {
+      // everything from e = exp(-|z|): 1 - sigma(z) is never formed, so neither tail cancels.
+      // var = sigma(z) sigma(-z);  resid = (1 - y) sigma(z) - y sigma(-z)  (= sigma(z) - y for every y)
+      const double e = exp(-fabs(zz));
+      const double big = 1.0 / (1.0 + e);          // sigma(|z|)
+      const double small = e * big;                // sigma(-|z|)
+      const bool pos = zz >= 0;
+      var = small * big;
+      r = fma(1.0 - a.y, pos ? big : small, -a.y * (pos ? small : big));
+    } else {
+      const double mu = family == GLM_POISSON ? exp(zz) : zz;
+      var = family == GLM_POISSON ? mu : 1.0;
+      r = mu - a.y;
+    }
     if (z) z[n] = zz;
     if (resid) resid[n] = r;
     const double sv = a.w * var;
