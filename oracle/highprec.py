@@ -41,6 +41,51 @@ def solve_lower_ld(L, B, transpose=False):
     return X
 
 
+def cholesky_ld_batched(B):
+    """Lower Cholesky factors of a stack (G, M, M) of small SPD matrices in longdouble, column by column."""
+    B = np.asarray(B, dtype=LD)
+    M = B.shape[-1]
+    L = np.zeros_like(B)
+    for j in range(M):
+        v = B[:, j:, j] - np.einsum('gik,gk->gi', L[:, j:, :j], L[:, j, :j])
+        L[:, j:, j] = v / np.sqrt(v[:, :1])
+    return L
+
+
+def solve_lower_ld_batched(L, B, transpose=False):
+    """L_g^{-1} B_g or L_g^{-T} B_g for stacks L (G, M, M) and B (G, M, K) by substitution in longdouble."""
+    L = np.asarray(L, dtype=LD)
+    X = np.array(B, dtype=LD)
+    M = L.shape[-1]
+    for i in (range(M - 1, -1, -1) if transpose else range(M)):
+        s = (np.einsum('gk,gkc->gc', L[:, i + 1:, i], X[:, i + 1:]) if transpose else
+             np.einsum('gk,gkc->gc', L[:, i, :i], X[:, :i]))
+        X[:, i] = (X[:, i] - s) / L[:, i, i, None]
+    return X
+
+
+def block_arrow_residual_ld(sa, gi, blocks, cross, hgg, x, b, chunk_entries=1 << 23):
+    """b - H x in longdouble for the block-arrow matrix H = [blockdiag(B_g) C; C^T Hgg] placed by the index arrays
+    sa (G, M) and gi (Dg,), all float64 numpy arrays; x and b are (d, K).  The cross blocks are converted a chunk of
+    blocks at a time, so a C of several GB needs no longdouble copy of itself."""
+    x = np.asarray(x, dtype=LD)
+    r = np.array(b, dtype=LD)
+    G, M = sa.shape
+    Dg = gi.shape[0]
+    xl, xg = x[sa], x[gi]
+    loc = np.empty(xl.shape, dtype=LD)
+    glob = np.asarray(hgg, dtype=LD) @ xg
+    step = max(1, chunk_entries // (M * max(Dg, 1)))
+    for g0 in range(0, G, step):
+        sl = slice(g0, g0 + step)
+        Cc = np.asarray(cross[sl], dtype=LD)
+        loc[sl] = np.asarray(blocks[sl], dtype=LD) @ xl[sl] + Cc @ xg
+        glob += Cc.reshape(-1, Dg).T @ xl[sl].reshape(-1, x.shape[1])
+    r[sa] -= loc
+    r[gi] -= glob
+    return r
+
+
 def logistic_stats_ld(z, y, w):
     """(resid, s) = (sigma(z) - y, w sigma(z) sigma(-z)) of the logistic family in longdouble.  Both are evaluated at
     -|z|, where nothing cancels: 1 - sigma(z) is never formed, so the relative error does not grow like e^z."""

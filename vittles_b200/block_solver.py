@@ -46,9 +46,11 @@ class CudaBlockKernels:
 
     @staticmethod
     def gram(Z2):
-        """Z^T Z on the tensor cores: the FP64 DMMA engine, or for large Z the FP64-grade INT8 slicing engine
-        ('auto', same parity bar)."""
-        return ops.syrk_weighted(Z2, precision='auto')
+        """Z^T Z on the FP64 DMMA engine, at every size.  The Schur complement Hgg - Z^T Z is a difference of large
+        terms, and the INT8 slicing engine's error is relative to the column maxima of Z: with a few O(1) cross
+        blocks among 1e-3 ones and S a thousandfold cancellation, its S misses the parity bar
+        (tests/test_gpu_block_arrow.py), so 'auto' is not used here."""
+        return ops.syrk_weighted(Z2, precision='f64')
 
     @staticmethod
     def dense_factor(S):

@@ -574,6 +574,27 @@ def synth_bernoulli(seed, row0, z):
 
 
 # ------------------------------------------------------- block-arrow path ----
+# The block kernels take no leading dimension and no strides: every operand is read as a packed array of the shape
+# the other arguments imply.  A view that is not packed, or an operand of the wrong size, would be read at the wrong
+# addresses or past its end, so it is refused here.  Nothing is copied: Z and the cross blocks can be many GB.
+def _packed(t, name, shape):
+    _f64(t, name)
+    if tuple(t.shape) != tuple(shape):
+        raise ValueError('{} has shape {}, expected {}'.format(name, tuple(t.shape), tuple(shape)))
+    if not t.is_contiguous():
+        raise ValueError('{} must be contiguous (the block kernels take no leading dimension), got strides {}'.format(
+            name, tuple(t.stride())))
+    return t
+
+
+def _vec(t, name, n):
+    """A read-only vector of exactly n entries (a packed copy of a strided one: these are short)."""
+    _f64(t, name)
+    if t.dim() != 1 or t.numel() != n:
+        raise ValueError('{} has shape {}, expected ({},)'.format(name, tuple(t.shape), n))
+    return t.contiguous()
+
+
 def block_potrf(blocks, check_pd=True):
     """In-place lower Cholesky of (G, M, M) blocks; returns the same tensor."""
     lib = _cabi.require_cuda()
@@ -593,63 +614,84 @@ def block_potrf(blocks, check_pd=True):
 def block_trsm(Lb, C, transpose=False):
     """C[g] <- L[g]^{-1} C[g] (or L[g]^{-T} C[g]) in place, C of shape (G, M, Dg)."""
     lib = _cabi.require_cuda()
+    _f64(C, 'C')
+    if C.dim() != 3:
+        raise ValueError('C must have shape (G, M, Dg), got {}'.format(tuple(C.shape)))
     G, M, Dg = C.shape
-    if not C.is_contiguous():
-        raise ValueError('C must be contiguous')
+    _packed(C, 'C', (G, M, Dg))
+    _packed(Lb, 'Lb', (G, M, M))
     fn = lib.vt_block_trsmt_batched if transpose else lib.vt_block_trsm_batched
-    check(fn(ptr(_f64(Lb, 'Lb')), ptr(_f64(C, 'C')), G, M, Dg, stream()))
+    check(fn(ptr(Lb), ptr(C), G, M, Dg, stream()))
     return C
 
 
 def block_solve(Lb, b, transpose=False):
     """b[g] <- L[g]^{-1} b[g] (or L[g]^{-T} b[g]) in place, b of shape (G, M)."""
     lib = _cabi.require_cuda()
+    _f64(b, 'b')
+    if b.dim() != 2:
+        raise ValueError('b must have shape (G, M), got {}'.format(tuple(b.shape)))
     G, M = b.shape
-    check(lib.vt_block_solve_batched(ptr(_f64(Lb, 'Lb')), ptr(_f64(b, 'b')), G, M, 1 if transpose else 0, stream()))
+    _packed(b, 'b', (G, M))
+    _packed(Lb, 'Lb', (G, M, M))
+    check(lib.vt_block_solve_batched(ptr(Lb), ptr(b), G, M, 1 if transpose else 0, stream()))
     return b
 
 
 def tall_gemv(Z, x, alpha=1.0, y=None, beta=0.0):
-    """y = beta*y + alpha * Z @ x for a (R, Dg) matrix with R very long."""
+    """y = beta*y + alpha * Z @ x for a contiguous (R, Dg) matrix with R very long; y (R,) is updated in place."""
     lib = _cabi.require_cuda()
     _mat(Z, 'Z')
     R, Dg = Z.shape
+    _packed(Z, 'Z', (R, Dg))
+    x = _vec(x, 'x', Dg)
     if y is None:
         y = torch.empty(R, dtype=torch.float64, device=Z.device)
         beta = 0.0
-    check(lib.vt_tall_gemv(ptr(Z), R, Dg, ptr(_f64(x, 'x').contiguous()), float(alpha), ptr(y), float(beta), stream()))
+    _packed(y, 'y', (R,))
+    check(lib.vt_tall_gemv(ptr(Z), R, Dg, ptr(x), float(alpha), ptr(y), float(beta), stream()))
     return y
 
 
 def tall_colsum(Z, u, alpha=1.0, y0=None, beta=1.0):
-    """alpha * Z.T @ u + beta * y0 for a (R, Dg) matrix with R very long."""
+    """alpha * Z.T @ u + beta * y0 for a contiguous (R, Dg) matrix with R very long."""
     lib = _cabi.require_cuda()
     _mat(Z, 'Z')
     R, Dg = Z.shape
+    _packed(Z, 'Z', (R, Dg))
+    u = _vec(u, 'u', R)
+    y0 = None if y0 is None else _vec(y0, 'y0', Dg)
     out = torch.empty(Dg, dtype=torch.float64, device=Z.device)
     ws, wsb = _ws('colsum', lib.vt_tall_colsum_workspace_bytes(Dg), Z.device)
-    check(lib.vt_tall_colsum(ptr(Z), R, Dg, ptr(_f64(u, 'u').contiguous()), float(alpha), ptr(y0), float(beta),
-                             ptr(out), ptr(ws), wsb, stream()))
+    check(lib.vt_tall_colsum(ptr(Z), R, Dg, ptr(u), float(alpha), ptr(y0), float(beta), ptr(out), ptr(ws), wsb,
+                             stream()))
     return out
 
 
 def gmm_blocks(X, m, rho, log_pi, want_blocks=True, want_cross=True):
-    """Closed-form pieces of the GMM-VB objective: local Hessian blocks
-    (N, K-1, K-1), cross blocks (N, K-1, K*d), responsibilities (N, K), local
+    """Closed-form pieces of the GMM-VB objective for a contiguous X (N, d), means m (K, d), logits rho (N, K-1) and
+    log_pi (K,): local Hessian blocks (N, K-1, K-1), cross blocks (N, K-1, K*d), responsibilities (N, K), local
     gradient (N, K-1) and per-observation objective terms (N,)."""
     lib = _cabi.require_cuda()
     _mat(X, 'X')
     N, d = X.shape
-    K = m.shape[0]
+    _packed(X, 'X', (N, d))
+    _f64(m, 'm')
+    K = m.shape[0] if m.dim() == 2 else -1
+    if tuple(m.shape) != (K, d):
+        raise ValueError('m has shape {}, expected (K, {})'.format(tuple(m.shape), d))
+    _f64(rho, 'rho')
+    if tuple(rho.shape) != (N, K - 1):
+        raise ValueError('rho has shape {}, expected ({}, {})'.format(tuple(rho.shape), N, K - 1))
+    log_pi = _vec(log_pi, 'log_pi', K)
     dev = X.device
     blocks = torch.empty((N, K - 1, K - 1), dtype=torch.float64, device=dev) if want_blocks else None
     cross = torch.empty((N, K - 1, K * d), dtype=torch.float64, device=dev) if want_cross else None
     rmat = torch.empty((N, K), dtype=torch.float64, device=dev)
     grad_rho = torch.empty((N, K - 1), dtype=torch.float64, device=dev)
     obj = torch.empty(N, dtype=torch.float64, device=dev)
-    check(lib.vt_gmm_blocks(ptr(X), N, d, K, ptr(_f64(m, 'm').contiguous()), ptr(_f64(rho, 'rho').contiguous()),
-                            ptr(_f64(log_pi, 'log_pi').contiguous()), ptr(blocks), ptr(cross), ptr(rmat),
-                            ptr(grad_rho), ptr(obj), stream()))
+    check(lib.vt_gmm_blocks(ptr(X), N, d, K, ptr(m.contiguous()), ptr(rho.contiguous()), ptr(log_pi), ptr(blocks),
+                            ptr(cross), ptr(rmat), ptr(grad_rho), ptr(obj), stream()))
     return dict(blocks=blocks, cross=cross, r=rmat, grad_rho=grad_rho, obj_terms=obj)
 
 
