@@ -137,6 +137,27 @@ int vt_glm_influence(const double* X, int64_t ldx, int64_t N, int D, const doubl
 size_t vt_potrf_dinv_doubles(int D);
 int vt_potrf(double* A, int64_t lda, int D, double* dinv, int32_t* info, void* stream);
 int vt_potrs(const double* L, int64_t ldl, int D, const double* dinv, double* B, int64_t ldb, int K, void* stream);
+/* One half of vt_potrs, in place: B <- L^{-1} B (transpose = 0) or L^{-T} B
+ * (transpose = 1).  Forward then backward gives the bits of vt_potrs.        */
+int vt_trsm_lower(const double* L, int64_t ldl, int D, const double* dinv, double* B, int64_t ldb, int K, int transpose,
+                  void* stream);
+
+/* ---- Quadratic forms of the inverse Hessian ---------------------------------
+ * out[n] = |Linv x_n|^2 = x_n^T H^{-1} x_n for H = L L^T, Linv = L^{-1} (D x D,
+ * lower triangular: zero above the diagonal), x_n the rows of X (N x D): the
+ * leverage terms of approximate leave-one-out cross-validation.  A sum of
+ * squares, so no cancellation; nothing of size D x N is written.
+ * vt_quad_forms runs on the FP64 DMMA engine (U = X_c Linv^T per chunk of rows,
+ * then the row sums of squares); vt_quad_forms_ozaki on the INT8 slicing
+ * engine (the chunks of vt_ij_apply_ozaki, squares summed in the GEMM's
+ * epilogue, row block tm of Linv meeting its k-blocks 0 .. tm only).  Both sum
+ * in a fixed order: two calls give the same bits.                           */
+size_t vt_quad_forms_workspace_bytes(int64_t N, int D);
+int vt_quad_forms(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D, double* out,
+                  void* workspace, size_t workspace_bytes, void* stream);
+size_t vt_quad_forms_ozaki_workspace_bytes(int64_t N, int D, int nslices);
+int vt_quad_forms_ozaki(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D, double* out,
+                        int nslices, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- Infinitesimal-jackknife apply ----------------------------------------
  * S (D x N) = -Hinv (D x D) * G^T, column n of G^T being resid[n] * x_n, fused

@@ -10,7 +10,7 @@ from .sensitivity_lib import \
 
 from .sparse_hessian_lib import SparseBlockHessian
 from .lr_cov_lib import LinearResponseCovariances
-from .influence_lib import ObservationInfluence, AMIPResult
+from .influence_lib import ObservationInfluence, AMIPResult, ApproximateCVResult
 from . import influence_lib
 from . import solver_lib
 from . import bivariate_sensitivity_lib

@@ -46,6 +46,9 @@ SIGNATURES = {
     'vt_potrf_dinv_doubles': (_SZ, [_I]),
     'vt_potrf': (_I, [_P, _I64, _I, _P, _P, _P]),
     'vt_potrs': (_I, [_P, _I64, _I, _P, _P, _I64, _I, _P]),
+    'vt_trsm_lower': (_I, [_P, _I64, _I, _P, _P, _I64, _I, _I, _P]),
+    'vt_quad_forms_workspace_bytes': (_SZ, [_I64, _I]),
+    'vt_quad_forms': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _P, _SZ, _P]),
     'vt_ij_apply': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _P, _I64, _P]),
     'vt_tf32_gemm_workspace_bytes': (_SZ, [_I, _I, _I64, _I]),
     'vt_tf32_convert': (_I, [_P, _I64, _I64, _I, _P, _I, _P, _P, _I64, _P]),
@@ -61,6 +64,8 @@ SIGNATURES = {
     'vt_syrk_ozaki': (_I, [_P, _I64, _I64, _I, _P, _D, _P, _I64, _I, _P, _P, _P, _SZ, _P]),
     'vt_ij_apply_ozaki_workspace_bytes': (_SZ, [_I64, _I, _I]),
     'vt_ij_apply_ozaki': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _P, _I64, _I, _P, _SZ, _P]),
+    'vt_quad_forms_ozaki_workspace_bytes': (_SZ, [_I64, _I, _I]),
+    'vt_quad_forms_ozaki': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _I, _P, _SZ, _P]),
     'vt_gemv_workspace_bytes': (_SZ, [_I, _I64]),
     'vt_gemv': (_I, [_P, _I64, _I, _I64, _P, _D, _P, _D, _P, _P, _SZ, _P]),
     'vt_cg_batch_init': (_I, [_I, _I, _P, _P, _P, _P, _D, _D, _I, _P]),

@@ -196,6 +196,18 @@ int vt_potrs(const double* L, int64_t ldl, int D, const double* dinv, double* B,
   return chol_potrs(L, ldl, D, dinv, B, ldb, K, S(stream));
 }
 
+int vt_trsm_lower(const double* L, int64_t ldl, int D, const double* dinv, double* B, int64_t ldb, int K, int transpose,
+                  void* stream) {
+  return chol_trsm_lower(L, ldl, D, dinv, B, ldb, K, transpose, S(stream));
+}
+
+size_t vt_quad_forms_workspace_bytes(int64_t N, int D) { return quad_forms_workspace_bytes(N, D); }
+
+int vt_quad_forms(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D, double* out,
+                  void* workspace, size_t workspace_bytes, void* stream) {
+  return quad_forms(Linv, ldl, X, ldx, N, D, out, workspace, workspace_bytes, S(stream));
+}
+
 int vt_ij_apply(const double* Hinv, int64_t ldh, const double* X, int64_t ldx, int64_t N, int D,
                 const double* resid, double* Sout, int64_t lds, void* stream) {
   VT_REQUIRE(Hinv && X && resid && Sout, "ij_apply: null pointer");
@@ -283,6 +295,15 @@ int vt_ij_apply_ozaki(const double* Hinv, int64_t ldh, const double* X, int64_t 
                       const double* resid, double* Sout, int64_t lds, int nslices, void* workspace,
                       size_t workspace_bytes, void* stream) {
   return ij_apply_ozaki(Hinv, ldh, X, ldx, N, D, resid, Sout, lds, nslices, workspace, workspace_bytes, S(stream));
+}
+
+size_t vt_quad_forms_ozaki_workspace_bytes(int64_t N, int D, int nslices) {
+  return quad_forms_ozaki_workspace_bytes(N, D, nslices);
+}
+
+int vt_quad_forms_ozaki(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D, double* out,
+                        int nslices, void* workspace, size_t workspace_bytes, void* stream) {
+  return quad_forms_ozaki(Linv, ldl, X, ldx, N, D, out, nslices, workspace, workspace_bytes, S(stream));
 }
 
 size_t vt_syrk_ozaki_workspace_bytes(int64_t N, int D, int nslices) { return syrk_ozaki_workspace_bytes(N, D, nslices); }

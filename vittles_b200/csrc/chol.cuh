@@ -16,5 +16,8 @@ int chol_potrf(double* A, long lda, int D, double* dinv, int* info, cudaStream_t
 
 // Solve (L L^T) X = B in place for the row-major D x K right-hand side B.
 int chol_potrs(const double* L, long ldl, int D, const double* dinv, double* B, long ldb, int K, cudaStream_t stream);
+// One pass of that solve, in place: B <- L^{-1} B (transpose = 0) or B <- L^{-T} B (transpose = 1).
+int chol_trsm_lower(const double* L, long ldl, int D, const double* dinv, double* B, long ldb, int K, int transpose,
+                    cudaStream_t stream);
 
 }  // namespace vt

@@ -467,4 +467,58 @@ int gemm_launch(GemmParams p, cudaStream_t stream) {
   return VT_OK;
 }
 
+// ---- out[n] = |Linv x_n|^2 on the DMMA engine -------------------------------
+namespace {
+constexpr size_t QF_CHUNK_BYTES = (size_t)256 << 20;          // U of one chunk of rows
+
+long quad_forms_chunk_rows(long N, int D) {
+  long rows = (long)(QF_CHUNK_BYTES / ((size_t)D * 8));
+  if (rows < 1) rows = 1;
+  if (rows > 2147483647L) rows = 2147483647L;
+  return rows < N ? rows : N;
+}
+
+// out[r] = sum_i U[r][i]^2: a warp per row, lane-strided partial sums and a fixed shuffle tree.
+__global__ void __launch_bounds__(256) row_sumsq_kernel(const double* __restrict__ U, long ldu, long rows, int D,
+                                                        double* __restrict__ out) {
+  const long r = ((long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= rows) return;
+  const double* u = U + r * ldu;
+  double acc = 0.0;
+  for (int i = lane; i < D; i += 32) acc = fma(u[i], u[i], acc);
+  acc = warp_sum(acc);
+  if (lane == 0) out[r] = acc;
+}
+}  // namespace
+
+size_t quad_forms_workspace_bytes(long N, int D) {
+  return N > 0 && D > 0 ? (size_t)quad_forms_chunk_rows(N, D) * D * 8 : 0;
+}
+
+int quad_forms(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, void* workspace,
+               size_t workspace_bytes, cudaStream_t stream) {
+  VT_REQUIRE(Linv && X && out, "quad_forms: null pointer");
+  VT_REQUIRE(D >= 1 && N >= 0 && ldl >= D && ldx >= D, "quad_forms: bad shape");
+  if (N == 0) return VT_OK;
+  VT_REQUIRE(workspace && workspace_bytes >= quad_forms_workspace_bytes(N, D), "quad_forms: workspace too small");
+  const long ch = quad_forms_chunk_rows(N, D);
+  double* U = static_cast<double*>(workspace);
+  for (long r0 = 0; r0 < N; r0 += ch) {
+    const long rows = (N - r0 < ch) ? N - r0 : ch;
+    GemmParams p{};                                              // U = X_c Linv^T  (rows x D)
+    p.M = (int)rows; p.N = D; p.K = D;
+    p.A = X + r0 * ldx; p.lda = ldx; p.amode = KC;
+    p.B = Linv; p.ldb = ldl; p.bmode = KC;
+    p.C = U; p.ldc = D;
+    p.alpha = 1.0; p.beta = 0.0;
+    p.parts = 1;
+    int st = gemm_launch(p, stream);
+    if (st != VT_OK) return st;
+    row_sumsq_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, stream>>>(U, D, rows, D, out + r0);
+    VT_LAUNCH_CHECK();
+  }
+  return VT_OK;
+}
+
 }  // namespace vt

@@ -64,4 +64,10 @@ int gemm_pick_tile(int M, int N, int K, int lower);
 int gemm_pick_parts(int ntiles, int kiters, int tile, size_t workspace_bytes);
 int gemm_ctas_per_sm(int tile);
 
+// out[n] = |Linv x_n|^2 for the rows of X (N x D): per chunk of rows U = X_c Linv^T on this engine, then the sum of
+// squares of every row of U in a fixed order.
+size_t quad_forms_workspace_bytes(long N, int D);
+int quad_forms(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, void* workspace,
+               size_t workspace_bytes, cudaStream_t stream);
+
 }  // namespace vt

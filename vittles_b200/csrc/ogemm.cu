@@ -51,7 +51,13 @@ struct OKernelArgs {
   int c_vec;
   SliceJob next;                // rows to slice during this launch (X == nullptr: none; cols <= 1024)
   unsigned long long* timing;   // development aid (VT_OGEMM_TIMING=1): clocks the MMA thread waits, summed over CTAs
+  int tri;                      // A lower triangular (OBM == OBK): row block tm needs the k-blocks 0 .. tm only
+                                // (honoured by the EPI_QUAD instances)
 };
+
+// Epilogue of ogemm_kernel: EPI_STORE writes C; EPI_QUAD writes, for every column n, the partial sums of squares
+// of the 32 rows of each warp, P[4 tm + quarter][n] (C = P, ldc = its pitch): no tile of C is stored.
+constexpr int EPI_STORE = 0, EPI_QUAD = 1;
 
 // lower: row block tm keeps the column blocks 0 .. (tm*OBM + OBM-1) / OBN
 __host__ __device__ inline int o_lower_cols(int tm, int tiles_n) {
@@ -61,8 +67,33 @@ __host__ __device__ inline int o_lower_cols(int tm, int tiles_n) {
 struct OUnit {
   int m0, n0, kb0, nkb, part;
 };
+template <int EPI>
 __device__ __forceinline__ OUnit o_decode(const OKernelArgs& a, long u) {
   OUnit r;
+  if constexpr (EPI == EPI_QUAD) {
+    if (a.tri) {
+      // Row block tm costs tm + 1 k-blocks.  Units stay in the order "row blocks fastest" (the CTAs running together
+      // share the B slices in L2) with the heaviest row block first, and every other wave of gridDim.x units is
+      // dealt to the CTAs in reverse: the CTA that drew a heavy tile in one wave draws a light one in the next.
+      // (When 2 gridDim.x is a multiple of tiles_m, the two row blocks a CTA draws in a pair of waves add up to
+      // tiles_m - 1, and the static round-robin is balanced exactly.)
+#ifndef VT_QF_NAIVE_ORDER
+      const long G = gridDim.x, wave = u / G, p = u % G;
+      const long len = (a.units - wave * G < G) ? a.units - wave * G : G;
+      const long tile = wave * G + ((wave & 1) ? len - 1 - p : p);
+      const int tm = a.tiles_m - 1 - (int)(tile % a.tiles_m);
+#else   // measurement aid (tools/loo_probe.py): the order of the rectangular product, lightest row block first
+      const long tile = u;
+      const int tm = (int)(tile % a.tiles_m);
+#endif
+      r.part = 0;
+      r.m0 = tm * OBM;
+      r.n0 = (int)(tile / a.tiles_m) * OBN;
+      r.kb0 = 0;
+      r.nkb = (tm + 1 < a.kblocks) ? tm + 1 : a.kblocks;
+      return r;
+    }
+  }
   const long tile = u % a.ntiles;
   r.part = (int)(u / a.ntiles);
   int tm, tn;
@@ -322,7 +353,7 @@ __device__ __forceinline__ double exact_double(long long u) {
 }
 __device__ __forceinline__ double pair_double(int hi, int lo) { return exact_double((long long)hi * 256 + (long long)lo); }
 
-template <int S>
+template <int S, int EPI>
 __global__ void __launch_bounds__(O_THREADS, 1)
 ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const OKernelArgs a) {
   constexpr int B_BUF_BYTES = OCfg<S>::B_BUF_BYTES;
@@ -364,7 +395,7 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
       int bs = 0, as = 0;
       uint32_t bph = 0, aph = 0;
       for (long u = blockIdx.x; u < a.units; u += gridDim.x) {
-        const OUnit U = o_decode(a, u);
+        const OUnit U = o_decode<EPI>(a, u);
         const int m0 = U.m0, n0 = U.n0;
         for (int kb = U.kb0; kb < U.kb0 + U.nkb; ++kb) {
           mbar_wait_(bempty(bs), bph ^ 1u);
@@ -395,7 +426,7 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
       long long w_t = 0, w_b = 0, w_a = 0;
       const long long t_begin = clock64();
       for (long u = blockIdx.x; u < a.units; u += gridDim.x) {
-        const OUnit U = o_decode(a, u);
+        const OUnit U = o_decode<EPI>(a, u);
         if (U.nkb == 0) continue;              // every role skips an empty unit
         long long c0 = clock64();
         mbar_wait_(tempty, tph ^ 1u);          // the epilogue has drained the accumulators of the previous tile
@@ -464,7 +495,7 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
     const int row_local = quarter * 32 + lane;
     uint32_t tph = 0;
     for (long u = blockIdx.x; u < a.units; u += gridDim.x) {
-      const OUnit U = o_decode(a, u);
+      const OUnit U = o_decode<EPI>(a, u);
       if (U.nkb == 0) continue;
       const int m0 = U.m0, n0 = U.n0;
       const int grow = m0 + row_local;
@@ -511,7 +542,30 @@ ogemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ C
           for (g -= 2; g >= 0; g -= 2) t = fma(t, 1.0 / 65536.0, pair_double((int)v[g][j], (int)v[g + 1][j]));
           out[j] = t * (rs * __shfl_sync(0xffffffffu, cs_lane, c + j));      // t = 256 sum_l P_l 2^-8l
         }
-        if (grow < a.M) {
+        if constexpr (EPI == EPI_QUAD) {
+          // sum over the warp's 32 rows (lanes) of the squares of its 8 columns: a transpose-reduce in a fixed tree
+          // (each step halves the columns a lane keeps and sums them with the partner's; a + b == b + a, so the
+          // result does not depend on which lane forms it), then the last two steps over the lanes that share a
+          // column.  Rows past M have rs = 0 and add zeros.
+          double q[8];
+#pragma unroll
+          for (int j = 0; j < 8; ++j) q[j] = out[j] * out[j];
+#pragma unroll
+          for (int w = 4; w >= 1; w >>= 1) {             // lane bit 4, 3, 2 -> keep the upper or lower w columns
+            const bool up = (lane & (w << 2)) != 0;
+#pragma unroll
+            for (int j = 0; j < w; ++j) {
+              const double send = up ? q[j] : q[j + w];
+              const double keep = up ? q[j + w] : q[j];
+              q[j] = keep + __shfl_xor_sync(0xffffffffu, send, w << 2);
+            }
+          }
+          double v = q[0];                               // column (lane >> 2) of the 8, summed over 8 lanes so far
+          v += __shfl_xor_sync(0xffffffffu, v, 2);
+          v += __shfl_xor_sync(0xffffffffu, v, 1);
+          const int gcol = n0 + chalf * (OBN / 2) + c + (lane >> 2);
+          if ((lane & 3) == 0 && gcol < a.N) Cpart[(long)(m0 / OBM * 4 + quarter) * a.ldc + gcol] = v;
+        } else if (grow < a.M) {
           const int gcol = n0 + chalf * (OBN / 2) + c;
           double* cp = Cpart + (long)grow * a.ldc + gcol;
           if (a.c_vec && gcol + 8 <= a.N) {
@@ -663,9 +717,9 @@ unsigned long long* ogemm_timing_buffer() {
   return buf;
 }
 
-template <int S>
+template <int S, int EPI>
 int launch_s(const CUtensorMap& mA, const CUtensorMap& mB, const OKernelArgs& a, cudaStream_t stream) {
-  auto kern = ogemm_kernel<S>;
+  auto kern = ogemm_kernel<S, EPI>;
   VT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OCfg<S>::SMEM_BYTES));
   VT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   const long slots = num_sms();
@@ -740,6 +794,7 @@ int ozaki_slice_t(const double* X, long ldx, long rows, int cols, const double* 
 namespace {
 struct OLaunchOpts {
   int lower = 0, parts = 1, accumulate = 0;
+  int epi = EPI_STORE, tri = 0;
   long part_stride = 0;
   SliceJob next{};              // rows sliced by the converter warps of this launch (X == nullptr: none)
 };
@@ -758,6 +813,7 @@ int ogemm_launch_opts(int M, int N, int K, const int8_t* A, long lda, long a_sli
   VT_REQUIRE(reinterpret_cast<uintptr_t>(A) % 16 == 0 && reinterpret_cast<uintptr_t>(B) % 16 == 0,
              "ogemm: operands must be 16-byte aligned");
   if (o.lower) VT_REQUIRE(M == N, "ogemm: lower-only output must be square");
+  VT_REQUIRE(!o.tri || (o.epi == EPI_QUAD && !o.lower && o.parts == 1), "ogemm: triangular K range: quadratic forms only");
   CUtensorMap mA, mB;
   int st = make_slice_map(&mA, A, M, K, lda, a_slice_stride, nslices, OBM, 1);
   if (st != VT_OK) return st;
@@ -788,10 +844,18 @@ int ogemm_launch_opts(int M, int N, int K, const int8_t* A, long lda, long a_sli
     VT_REQUIRE((a.next.colmax || a.next.cols <= 1024) && a.next.ldo % 16 == 0,
                "ogemm: in-kernel slicing takes rows of at most 1024 elements");
   a.timing = ogemm_timing_buffer();
+  a.tri = o.tri;
+  if (o.epi == EPI_QUAD) {
+    switch (nslices) {
+      case 5: return launch_s<5, EPI_QUAD>(mA, mB, a, stream);
+      case 6: return launch_s<6, EPI_QUAD>(mA, mB, a, stream);
+      default: return launch_s<7, EPI_QUAD>(mA, mB, a, stream);
+    }
+  }
   switch (nslices) {
-    case 5: return launch_s<5>(mA, mB, a, stream);
-    case 6: return launch_s<6>(mA, mB, a, stream);
-    default: return launch_s<7>(mA, mB, a, stream);
+    case 5: return launch_s<5, EPI_STORE>(mA, mB, a, stream);
+    case 6: return launch_s<6, EPI_STORE>(mA, mB, a, stream);
+    default: return launch_s<7, EPI_STORE>(mA, mB, a, stream);
   }
 }
 }  // namespace
@@ -919,12 +983,77 @@ int ogemm_launch(int M, int N, int K, const int8_t* A, long lda, long a_slice_st
                            ldc, OLaunchOpts{}, stream);
 }
 
-size_t ij_apply_ozaki_workspace_bytes(long N, int D, int nslices) {
-  const long ld = (D + 15) / 16 * 16;
-  const long ch = ozaki_chunk_rows(N, D, nslices);
-  return align_up((size_t)nslices * D * ld, 256) + align_up((size_t)D * 8, 256) +
-         2 * (align_up((size_t)nslices * ch * ld, 256) + align_up((size_t)ch * 8, 256));
+namespace {
+// Rows of X (N x D) against a D x D matrix A on the INT8 engine, chunk by chunk: A is sliced once, chunk c of X
+// (ozaki_chunk_rows rows, scale tau_n * fold[n]; fold == nullptr: tau_n) into one of two digit buffers, and
+// product(r0, rows, Bs, tau, o) runs the GEMM of the chunk with the slicing job `o.next` of the chunk after it.
+// Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (rows of up to 1024 elements; longer rows:
+// a separate slicing launch per chunk).
+struct RowChunks {
+  long ld, ch;
+  size_t a_bytes, sigma_bytes, b_bytes, tau_bytes;
+  RowChunks(long N, int D, int nslices)
+      : ld((D + 15) / 16 * 16), ch(ozaki_chunk_rows(N, D, nslices)), a_bytes(align_up((size_t)nslices * D * ld, 256)),
+        sigma_bytes(align_up((size_t)D * 8, 256)), b_bytes(align_up((size_t)nslices * ch * ld, 256)),
+        tau_bytes(align_up((size_t)ch * 8, 256)) {}
+  size_t bytes() const { return a_bytes + sigma_bytes + 2 * (b_bytes + tau_bytes); }
+};
+
+template <class Product>
+int ozaki_row_chunks(const double* A, long lda, const double* X, long ldx, long N, int D, const double* fold,
+                     int nslices, void* workspace, cudaStream_t stream, Product&& product) {
+  const RowChunks rc(N, D, nslices);
+  const long ld = rc.ld, ch = rc.ch;
+  char* w = static_cast<char*>(workspace);
+  int8_t* As = reinterpret_cast<int8_t*>(w);
+  w += rc.a_bytes;
+  double* sigma = reinterpret_cast<double*>(w);
+  w += rc.sigma_bytes;
+  int8_t* Bs[2];
+  double* tau[2];
+  for (int b = 0; b < 2; ++b) {
+    Bs[b] = reinterpret_cast<int8_t*>(w);
+    w += rc.b_bytes;
+    tau[b] = reinterpret_cast<double*>(w);
+    w += rc.tau_bytes;
+  }
+  int st = ozaki_slice(A, lda, D, D, As, ld, (long)D * ld, nslices, sigma, nullptr, stream);
+  if (st != VT_OK) return st;
+  const bool fuse = D <= 1024;
+  long c = 0;
+  for (long r0 = 0; r0 < N; r0 += ch, ++c) {
+    const int b = (int)(c & 1);
+    const long rows = (N - r0 < ch) ? N - r0 : ch;
+    if (!fuse || c == 0) {
+      st = ozaki_slice(X + r0 * ldx, ldx, rows, D, Bs[b], ld, ch * ld, nslices, tau[b], fold ? fold + r0 : nullptr, stream);
+      if (st != VT_OK) return st;
+    }
+    OLaunchOpts o;
+    const long n0 = r0 + ch;
+    if (fuse && n0 < N) {
+      const long nrows = (N - n0 < ch) ? N - n0 : ch;
+      o.next = SliceJob{X + n0 * ldx, ldx, nrows, D, Bs[b ^ 1], ld, ch * ld, tau[b ^ 1], fold ? fold + n0 : nullptr,
+                        nullptr, nullptr};
+    }
+    st = product(r0, rows, As, sigma, Bs[b], tau[b], ld, ch, o);
+    if (st != VT_OK) return st;
+  }
+  return VT_OK;
 }
+
+// out[n] = sum of the 4 tiles_m partial sums of squares of column n, in a fixed order (no atomics: two calls give
+// the same bits).
+__global__ void __launch_bounds__(256) quad_forms_finish_kernel(const double* __restrict__ P, int nparts, long ldp,
+                                                                long rows, double* __restrict__ out) {
+  const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= rows) return;
+  double v = 0.0;
+  for (int p = 0; p < nparts; ++p) v += P[(long)p * ldp + n];
+  out[n] = v;
+}
+}  // namespace
+
+size_t ij_apply_ozaki_workspace_bytes(long N, int D, int nslices) { return RowChunks(N, D, nslices).bytes(); }
 
 int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long N, int D, const double* resid,
                    double* S, long lds, int nslices, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
@@ -933,45 +1062,44 @@ int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long
   VT_REQUIRE(nslices >= OZAKI_MIN_SLICES && nslices <= OZAKI_MAX_SLICES, "ij_apply_ozaki: 5, 6 or 7 slices");
   VT_REQUIRE(workspace_bytes >= ij_apply_ozaki_workspace_bytes(N, D, nslices), "ij_apply_ozaki: workspace too small");
   if (N == 0) return VT_OK;
-  const long ld = (D + 15) / 16 * 16;
-  const long ch = ozaki_chunk_rows(N, D, nslices);
-  char* w = static_cast<char*>(workspace);
-  int8_t* As = reinterpret_cast<int8_t*>(w);
-  w += align_up((size_t)nslices * D * ld, 256);
-  double* sigma = reinterpret_cast<double*>(w);
-  w += align_up((size_t)D * 8, 256);
-  int8_t* Bs[2];
-  double* tau[2];
-  for (int b = 0; b < 2; ++b) {
-    Bs[b] = reinterpret_cast<int8_t*>(w);
-    w += align_up((size_t)nslices * ch * ld, 256);
-    tau[b] = reinterpret_cast<double*>(w);
-    w += align_up((size_t)ch * 8, 256);
-  }
-  int st = ozaki_slice(Hinv, ldh, D, D, As, ld, (long)D * ld, nslices, sigma, nullptr, stream);
-  if (st != VT_OK) return st;
-  // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (rows of up to 1024 elements; longer rows:
-  // a separate slicing launch per chunk).
-  const bool fuse = D <= 1024;
-  long c = 0;
-  for (long r0 = 0; r0 < N; r0 += ch, ++c) {
-    const int b = (int)(c & 1);
-    const long rows = (N - r0 < ch) ? N - r0 : ch;
-    if (!fuse || c == 0) {
-      st = ozaki_slice(X + r0 * ldx, ldx, rows, D, Bs[b], ld, ch * ld, nslices, tau[b], resid + r0, stream);   // tau_n resid_n
-      if (st != VT_OK) return st;
-    }
-    OLaunchOpts o;
-    const long n0 = r0 + ch;
-    if (fuse && n0 < N) {
-      const long nrows = (N - n0 < ch) ? N - n0 : ch;
-      o.next = SliceJob{X + n0 * ldx, ldx, nrows, D, Bs[b ^ 1], ld, ch * ld, tau[b ^ 1], resid + n0, nullptr, nullptr};
-    }
-    st = ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs[b], ld, ch * ld, nslices, -1.0, sigma, tau[b], S + r0, lds,
-                           o, stream);
-    if (st != VT_OK) return st;
-  }
-  return VT_OK;
+  // tau_n resid_n: the residual is folded into the column scale
+  return ozaki_row_chunks(Hinv, ldh, X, ldx, N, D, resid, nslices, workspace, stream,
+                          [&](long r0, long rows, const int8_t* As, const double* sigma, const int8_t* Bs,
+                              const double* tau, long ld, long ch, const OLaunchOpts& o) {
+                            return ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs, ld, ch * ld, nslices,
+                                                     -1.0, sigma, tau, S + r0, lds, o, stream);
+                          });
+}
+
+// ---- out[n] = |Linv x_n|^2 ---------------------------------------------------
+size_t quad_forms_ozaki_workspace_bytes(long N, int D, int nslices) {
+  const RowChunks rc(N, D, nslices);
+  return rc.bytes() + align_up((size_t)4 * ((D + OBM - 1) / OBM) * rc.ch * 8, 256);
+}
+
+int quad_forms_ozaki(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, int nslices,
+                     void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  VT_REQUIRE(Linv && X && out && workspace, "quad_forms_ozaki: null pointer");
+  VT_REQUIRE(D >= 1 && D <= OZAKI_MAX_K && N >= 0 && ldl >= D && ldx >= D, "quad_forms_ozaki: bad shape");
+  VT_REQUIRE(nslices >= OZAKI_MIN_SLICES && nslices <= OZAKI_MAX_SLICES, "quad_forms_ozaki: 5, 6 or 7 slices");
+  VT_REQUIRE(workspace_bytes >= quad_forms_ozaki_workspace_bytes(N, D, nslices), "quad_forms_ozaki: workspace too small");
+  if (N == 0) return VT_OK;
+  const RowChunks rc(N, D, nslices);
+  double* P = reinterpret_cast<double*>(static_cast<char*>(workspace) + rc.bytes());    // (4 tiles_m) x ch partials
+  const int nparts = 4 * ((D + OBM - 1) / OBM);
+  return ozaki_row_chunks(Linv, ldl, X, ldx, N, D, nullptr, nslices, workspace, stream,
+                          [&](long r0, long rows, const int8_t* As, const double* sigma, const int8_t* Bs,
+                              const double* tau, long ld, long ch, OLaunchOpts o) {
+                            o.epi = EPI_QUAD;
+                            o.tri = 1;          // Linv is lower triangular (the caller's contract)
+                            int st = ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs, ld, ch * ld, nslices,
+                                                       1.0, sigma, tau, P, ch, o, stream);
+                            if (st != VT_OK) return st;
+                            quad_forms_finish_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, stream>>>(P, nparts, ch,
+                                                                                                          rows, out + r0);
+                            VT_LAUNCH_CHECK();
+                            return VT_OK;
+                          });
 }
 
 // ---- H = X^T diag(s) X -----------------------------------------------------

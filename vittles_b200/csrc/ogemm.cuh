@@ -48,6 +48,14 @@ size_t ij_apply_ozaki_workspace_bytes(long N, int D, int nslices);
 int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long N, int D, const double* resid,
                    double* S, long lds, int nslices, void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
+// out[n] = |Linv x_n|^2 for every row x_n of X (N x D), Linv (D x D) lower triangular (zero above the diagonal:
+// row block tm of Linv meets the k-blocks 0 .. tm only).  The chunks of ij_apply_ozaki; the epilogue squares each
+// element of Linv X_c^T and sums the squares of every column over the rows of a warp, and a finish kernel adds
+// the 4 ceil(D / 128) partials of a column in a fixed order.  Nothing of size D x N is written.
+size_t quad_forms_ozaki_workspace_bytes(long N, int D, int nslices);
+int quad_forms_ozaki(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, int nslices,
+                     void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 // H (D x D) = X^T diag(s) X (s >= 0) with FP64-grade accuracy on the INT8 tensor cores: per chunk of
 // observations the digits of sqrt(s_n) x_ni are written transposed with one power-of-two scale per
 // feature, the lower tiles of the chunk's Gram matrix run as split-K parts of at most 16384

@@ -10,6 +10,16 @@ That is K solves against the Cholesky factor of H and one pass over X that write
 (``ops.glm_influence``); nothing of size D x N is formed, so the (D, N) matrix of
 ``HyperparameterSensitivityLinearApproximation`` and its memory are never needed.
 
+Approximate leave-one-out cross-validation (:meth:`ObservationInfluence.approximate_cv`) needs one scalar per
+observation, h_n = x_n^T H^{-1} x_n = |L^{-1} x_n|^2 (``ops.quad_forms``: a sum of squares, N D^2 / 2 multiply-adds
+on the tensor cores).  With the statistics r_n = b'(z_n) - y_n and s_n = w_n b''(z_n) at theta_hat:
+
+    leverage_n = s_n h_n
+    z_n^IJ = z_n + w_n r_n h_n                          (x_n^T of predict_opt_par_without([n]))
+    z_n^NS = z_n + w_n r_n h_n / (1 - s_n h_n)          (one Newton step from theta_hat without row n)
+
+The Newton-step ("ALO") form equals the exact leave-one-out prediction for the Gaussian family.
+
 On top of psi, :meth:`ObservationInfluence.amip` computes the Approximate Maximum Influence Perturbation of
 Broderick, Giordano & Meager: the smallest set of observations whose removal is predicted to move a quantity of
 interest to a target (zero: a sign change), and :meth:`ObservationInfluence.refit` re-optimises without that set to
@@ -147,6 +157,70 @@ class AMIPResult:
     target: float
 
 
+@dataclass
+class ApproximateCVResult:
+    """Outcome of :meth:`ObservationInfluence.approximate_cv`.
+
+    Per local row, in the array kind of the weights: ``z_loo``, the leave-one-out linear predictor of ``method``
+    ('ns' or 'ij'); ``loss``, the family's negative log-likelihood of y_n at z_loo (up to terms in y only);
+    ``leverage``, s_n h_n.  Over all ranks: ``mean_loss`` = sum w_n loss_n / sum w_n over the rows with a nonzero
+    weight and a defined prediction, and ``n_invalid``, the rows whose Newton step is not defined (NaN in z_loo and
+    loss: without row n the Hessian is singular to working accuracy)."""
+    method: str
+    z_loo: object
+    loss: object
+    leverage: object
+    mean_loss: float
+    n_invalid: int
+
+
+LOO_METHODS = ('ns', 'ij')
+# s_n h_n at or above this: H - s_n x_n x_n^T is singular to working accuracy (an exactly singular case computes
+# s_n h_n only to within a few ulps of 1)
+NS_SINGULAR = 1.0 - 2.0 ** -40
+
+
+def check_loo_method(method):
+    if method not in LOO_METHODS:
+        raise ValueError("method must be 'ns' (Newton step) or 'ij' (infinitesimal jackknife), not {!r}".format(method))
+    return method
+
+
+def loo_predictor(z, resid, s, w, h, method):
+    """z_n^NS (NaN where s_n h_n >= 1 - 2^-40) or z_n^IJ from the statistics at theta_hat and h_n."""
+    step = w * resid * h
+    if method == 'ij':
+        return z + step
+    lev = s * h
+    return torch.where(lev < NS_SINGULAR, z + step / (1.0 - lev), torch.full_like(z, float('nan')))
+
+
+def glm_loss(z, y, family):
+    """The family's negative log-likelihood of y at the linear predictor z, up to terms in y only."""
+    if family == 'logistic':
+        return torch.clamp(z, min=0.0) + torch.log1p(torch.exp(-torch.abs(z))) - y * z
+    if family == 'poisson':
+        return torch.exp(z) - y * z
+    if family == 'gaussian':
+        return 0.5 * (y - z) ** 2
+    raise ValueError('unknown GLM family {!r}'.format(family))
+
+
+def cv_totals(loss, w, invalid, group=None):
+    """(mean_loss, n_invalid) over all ranks: sum w_n loss_n / sum w_n over the rows with w_n != 0 that are not
+    ``invalid`` (bool mask of the rows without a prediction), and the number of invalid rows.  One all-reduce of
+    three numbers, on the device for NCCL and on the host otherwise."""
+    keep = (w != 0) & ~invalid
+    t = torch.stack([torch.where(keep, w * loss, torch.zeros_like(loss)).sum(),
+                     torch.where(keep, w, torch.zeros_like(w)).sum(),
+                     invalid.sum().to(loss.dtype)])
+    if _world(group) > 1:
+        t = t if _nccl(group) else t.cpu()
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    num, den, nbad = (float(v) for v in t.cpu())
+    return (num / den if den != 0 else float('nan')), int(nbad)
+
+
 def amip_from_scores(score, value, target, max_drop, offset=0, group=None):
     """AMIP selection from the per-observation scores w_n psi_n of this rank (dropping a set A changes phi by about
     -sum_{n in A} w_n psi_n).  Pure torch over the N_local scores and the candidate lists, so it runs on any device
@@ -217,6 +291,7 @@ class ObservationInfluence:
                                  '||grad|| = {} > {} = grad_tol'.format(g, grad_tol))
         self.factor = solver_lib.get_cholesky_solver(H).factor
         self.offset, self.n_total = row_offset(n, objective.group, dev if _nccl(objective.group) else None)
+        self._h = None
 
     # -- influence ------------------------------------------------------------
     def _influence_device(self, A):
@@ -274,6 +349,51 @@ class ObservationInfluence:
                           UserWarning)
         return as_kind(theta, self._theta_kind)
 
+    # -- approximate leave-one-out ---------------------------------------------
+    def _quad_forms(self):
+        """h_n = x_n^T H^{-1} x_n = |L^{-1} x_n|^2 for this rank's rows, computed once.  The engine follows the
+        objective's precision; a TF32 objective gets 'auto' (the quadratic forms are always FP64-grade)."""
+        if getattr(self, '_h', None) is None:
+            precision = self._obj.precision
+            if precision in ('tf32', 'tf32x3'):
+                precision = 'auto'
+            self._obj._wait_resident()
+            Linv = self.factor.inverse_factor()
+            self._h = ops.quad_forms(Linv, self._obj.X, precision=precision)
+            del Linv
+        return self._h
+
+    def _loo(self, method):
+        st = self._stats
+        return loo_predictor(st['z'], st['resid'], st['s'], self._w, self._quad_forms(), method)
+
+    def leverage(self):
+        """s_n h_n (the diagonal of the GLM hat matrix) for this rank's observations, shape (N_local,)."""
+        return as_kind(self._stats['s'] * self._quad_forms(), self._kind)
+
+    def loo_linear_predictor(self, method='ns'):
+        """The approximate leave-one-out linear predictor x_n^T theta_hat_{-n} of this rank's rows, (N_local,):
+        'ns' one Newton step without row n (NaN, with a UserWarning, where that step is not defined), 'ij' the
+        infinitesimal jackknife x_n^T predict_opt_par_without([n])."""
+        check_loo_method(method)
+        z = self._loo(method)
+        if method == 'ns':
+            _warn_invalid(int(torch.isnan(z).sum()))
+        return as_kind(z, self._kind)
+
+    def approximate_cv(self, method='ns'):
+        """Approximate leave-one-out cross-validation: the held-out loss of every observation at its approximate
+        leave-one-out prediction, and their weighted mean over all ranks (:class:`ApproximateCVResult`)."""
+        check_loo_method(method)
+        z = self._loo(method)
+        loss = glm_loss(z, self._obj.y, self._obj.family)
+        invalid = torch.isnan(z) if method == 'ns' else torch.zeros_like(z, dtype=torch.bool)
+        mean_loss, n_invalid = cv_totals(loss, self._w, invalid, self._obj.group)
+        _warn_invalid(n_invalid)
+        return ApproximateCVResult(method=method, z_loo=as_kind(z, self._kind), loss=as_kind(loss, self._kind),
+                                   leverage=as_kind(self._stats['s'] * self._quad_forms(), self._kind),
+                                   mean_loss=mean_loss, n_invalid=n_invalid)
+
     # -- AMIP -----------------------------------------------------------------
     def amip(self, qoi, target=0.0, max_drop=0.01):
         """Approximate Maximum Influence Perturbation: the fewest observations whose removal is predicted to move
@@ -299,6 +419,13 @@ class ObservationInfluence:
         A, _ = qoi_matrix(a, self.dim)
         psi = self._influence_device(to_device(A, self._theta.device))[0]
         return amip_from_scores(self._w * psi, value, target, m, self.offset, self._obj.group)
+
+
+def _warn_invalid(n):
+    if n:
+        warnings.warn('approximate leave-one-out: the Newton step is not defined for {} observation(s) (s_n h_n >= '
+                      '1 - 2^-40: the Hessian without the row is singular); their prediction and loss are NaN and they '
+                      'are left out of mean_loss'.format(n), UserWarning)
 
 
 def _nccl(group):

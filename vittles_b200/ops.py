@@ -437,11 +437,8 @@ class CholeskyFactor:
         self.dinv = dinv
         self.dim = L.shape[0]
 
-    def solve(self, B, overwrite=False):
-        """(L L^T)^{-1} B for B of shape (D,) or (D, K); float64 CUDA tensor."""
-        lib = _cabi.require_cuda()
+    def _rhs(self, B, overwrite):
         _f64(B, 'B')
-        vec = B.dim() == 1
         if B.shape[0] != self.dim or B.dim() > 2:
             raise ValueError('right-hand side has shape {}, expected ({},) or ({}, K)'.format(
                 tuple(B.shape), self.dim, self.dim))
@@ -450,8 +447,29 @@ class CholeskyFactor:
             X = X.contiguous()
             if X.data_ptr() == B.data_ptr():
                 X = X.clone()
+        return X
+
+    def solve(self, B, overwrite=False):
+        """(L L^T)^{-1} B for B of shape (D,) or (D, K); float64 CUDA tensor."""
+        lib = _cabi.require_cuda()
+        X = self._rhs(B, overwrite)
         check(lib.vt_potrs(ptr(self.L), _ld(self.L), self.dim, ptr(self.dinv), ptr(X), _ld(X), X.shape[1], stream()))
-        return X.reshape(-1) if vec else X
+        return X.reshape(-1) if B.dim() == 1 else X
+
+    def solve_lower(self, B, transpose=False, overwrite=False):
+        """L^{-1} B (or L^{-T} B with ``transpose``) for B of shape (D,) or (D, K): one of the two passes of
+        :meth:`solve`, which is solve_lower(solve_lower(B), transpose=True) bit for bit."""
+        lib = _cabi.require_cuda()
+        X = self._rhs(B, overwrite)
+        check(lib.vt_trsm_lower(ptr(self.L), _ld(self.L), self.dim, ptr(self.dinv), ptr(X), _ld(X), X.shape[1],
+                                1 if transpose else 0, stream()))
+        return X.reshape(-1) if B.dim() == 1 else X
+
+    def inverse_factor(self):
+        """L^{-1} (D, D), lower triangular with the strict upper triangle exactly zero (``quad_forms`` relies on
+        it)."""
+        eye = torch.eye(self.dim, dtype=torch.float64, device=self.L.device)
+        return self.solve_lower(eye, overwrite=True).tril_()
 
     def inverse(self):
         eye = torch.eye(self.dim, dtype=torch.float64, device=self.L.device)
@@ -514,6 +532,38 @@ def ij_apply(Hinv, X, resid, out=None, precision='f64'):
         return out
     check(lib.vt_ij_apply(ptr(Hinv), _ld(Hinv), ptr(X), _ld(X), N, D, ptr(_f64(resid, 'resid')), ptr(out), _ld(out),
                           stream()))
+    return out
+
+
+# ------------------------------------------------------ quadratic forms ----
+def quad_forms(Linv, X, precision='auto', out=None):
+    """out (N,) = |Linv x_n|^2 for the rows x_n of X: x_n^T H^{-1} x_n when Linv = L^{-1} for H = L L^T
+    (``CholeskyFactor.inverse_factor``).  Linv must be lower triangular (zero above the diagonal): the INT8 engine
+    skips the blocks above it.  ``precision``: 'f64' (DMMA engine), 'f64_ozaki' (INT8 error-free slicing), or 'auto'
+    (one of the two by size, as ``resolve_precision``); both are FP64-grade, and there is no TF32 form.  X may be a
+    row-major view with padded rows or an offset base."""
+    lib = _cabi.require_cuda()
+    _mat(Linv, 'Linv'); _mat(X, 'X')
+    N, D = X.shape
+    if precision in ('tf32', 'tf32x3'):
+        raise ValueError("quad_forms: precision {!r} is not offered; use 'auto', 'f64' or 'f64_ozaki'".format(precision))
+    precision = resolve_precision(precision, N, D)
+    if tuple(Linv.shape) != (D, D):
+        raise ValueError('Linv must have shape ({}, {}), got {}'.format(D, D, tuple(Linv.shape)))
+    if bool(torch.triu(Linv, diagonal=1).any()):
+        raise ValueError('Linv must be lower triangular (zero above the diagonal)')
+    if out is None:
+        out = torch.empty(N, dtype=torch.float64, device=X.device)
+    _f64(out, 'out')
+    if out.dim() != 1 or out.numel() != N or (N > 1 and out.stride(0) != 1):
+        raise ValueError('out must be a contiguous ({},) tensor, got shape {}'.format(N, tuple(out.shape)))
+    if precision == 'f64_ozaki':
+        ws, wsb = _ws('qf_ozaki', lib.vt_quad_forms_ozaki_workspace_bytes(N, D, OZAKI_SLICES), X.device)
+        check(lib.vt_quad_forms_ozaki(ptr(Linv), _ld(Linv), ptr(X), _ld(X), N, D, ptr(out), OZAKI_SLICES, ptr(ws), wsb,
+                                      stream()))
+        return out
+    ws, wsb = _ws('qf', lib.vt_quad_forms_workspace_bytes(N, D), X.device)
+    check(lib.vt_quad_forms(ptr(Linv), _ld(Linv), ptr(X), _ld(X), N, D, ptr(out), ptr(ws), wsb, stream()))
     return out
 
 
@@ -729,10 +779,12 @@ def _device_scoped(fn):
 
 
 for _name in ('gemm', 'tf32_convert', 'tf32_gemm', 'ozaki_slice', 'ozaki_gemm', 'syrk_weighted', 'glm_stats', 'glm_hvp',
-              'glm_hvp_multi', 'glm_dirderiv', 'glm_influence', 'potrf', 'ij_apply', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
+              'glm_hvp_multi', 'glm_dirderiv', 'glm_influence', 'potrf', 'ij_apply', 'quad_forms', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
               'synth_design',
               'synth_theta', 'synth_bernoulli', 'block_potrf', 'block_trsm', 'block_solve', 'tall_gemv', 'tall_colsum',
               'gmm_blocks'):
     globals()[_name] = _device_scoped(globals()[_name])
 CholeskyFactor.solve = _device_scoped(CholeskyFactor.solve)
+CholeskyFactor.solve_lower = _device_scoped(CholeskyFactor.solve_lower)
+CholeskyFactor.inverse_factor = _device_scoped(CholeskyFactor.inverse_factor)
 del _name
