@@ -157,3 +157,62 @@ def wls_fixture(n_obs=10, dim=2, seed=7):
         xty = torch.einsum('n,ni,n->i', w, xt, yt)
         return torch.linalg.solve(xtx, xty)
     return objective, run_regression, x, y
+
+
+# --------------------------------------------------------------------------
+# GMM-VB observations assigned with confidence (the regime of a fitted mixture
+# whose clusters are separated)
+# --------------------------------------------------------------------------
+
+GMM_GAPS = (0, 1, 20, 36, 37, 38, 60, 300, 700, 740, 800)
+
+
+def gmm_confident(seed, N, K, d, spacing=48.0):
+    """X (N, d), m (K, d), rho (N, K-1), log_pi (K,) and, per observation, the component built to dominate (``dom``)
+    and the gap between its logit and the runner-up's (``gap``); ``vb`` marks the observations with logits at the
+    VB optimum.
+
+    Centers are ``spacing`` apart: m_k = spacing / sqrt(2) e_k when d >= K, else m_k = spacing k e_0 (on a line).
+    Observation n takes in turn a dominant component (the first, the last free logit or the implicit K-th), a gap
+    from GMM_GAPS and whether two logits tie at the top.
+      * even n (``vb``): x_n lies on the segment from m_dom to a runner-up m_b where c_b - c_dom = gap, plus unit
+        noise in the directions no center spans; rho_j = -(c_j - c_K), so that a_k = c_k + log r_k is the same for
+        every k and only the complements 1 - r carry the local block.  A tie is the midpoint (gap 0).
+      * odd n: top logit T, runner-up T - gap (T for a tie, which may be the implicit 0), the others T - gap - U(0, 8).
+    Gaps >= 745 underflow the runner-up's responsibility."""
+    rng = np.random.default_rng(seed)
+    lp = 0.3 * rng.normal(size=K)
+    log_pi = lp - np.log(np.sum(np.exp(lp)))
+    m = np.zeros((K, d))
+    if d >= K:
+        m[np.arange(K), np.arange(K)] = spacing / np.sqrt(2.0)
+        free_axes = np.arange(K, d)
+    else:
+        m[:, 0] = spacing * np.arange(K)
+        free_axes = np.arange(1, d)
+    positions = sorted({0, K - 2, K - 1})
+    combos = [(p, g, tie) for p in positions for g in GMM_GAPS for tie in (False, True)]
+    dom = np.empty(N, dtype=np.int64)
+    gap = np.empty(N)
+    vb = np.arange(N) % 2 == 0
+    X = np.zeros((N, d))
+    offsets = np.zeros((N, K))
+    for n in range(N):
+        a, g, tie = combos[(n // 2 + 7 * (n % 2)) % len(combos)]
+        g = 0.0 if tie else float(g)
+        others = [k for k in range(K) if k != a]
+        if vb[n]:
+            b = (a + 1 if a + 1 < K else a - 1) if d < K else others[rng.integers(K - 1)]
+            u = (m[b] - m[a]) / spacing
+            t = (0.5 * spacing ** 2 + (log_pi[a] - log_pi[b]) - g) / spacing
+            X[n] = m[a] + t * u
+            X[n, free_axes] = rng.normal(size=len(free_axes))
+        else:
+            b = others[rng.integers(K - 1)]
+            offsets[n] = g + rng.uniform(0.0, 8.0, size=K)
+            offsets[n, a] = 0.0
+            offsets[n, b] = g
+        dom[n], gap[n] = a, g
+    c = 0.5 * ((X[:, None, :] - m[None]) ** 2).sum(-1) - log_pi[None]
+    logits = np.where(vb[:, None], -(c - c[:, -1:]), offsets[:, -1:] - offsets)
+    return X, m, logits[:, :K - 1].copy(), log_pi, dict(dom=dom, gap=gap, vb=vb)

@@ -181,3 +181,139 @@ def glm_resid_mp(z, y, family):
 def glm_weight_mp(z, w, family):
     """s = w b''(z), correctly rounded to float64."""
     return _elementwise(lambda zz, ww: mpmath.mpf(ww) * _bderiv(zz, 2, family), z, w)
+
+
+# ----------------------------------------------------------------------------------------------------------------
+# The per-observation GMM-VB assembly of ``gmm_blocks`` (csrc/blockchol.cu).  Observation n, logits l = [rho_n, 0],
+# r = softmax(l), c_k = |x_n - m_k|^2 / 2 - log pi_k, a_k = c_k + log r_k, abar = sum_k r_k a_k, delta_k = a_k - abar:
+#   B[j][l] = r_j d_jl (delta_j + 1) - r_j r_l (delta_j + delta_l + 1)      j, l < K-1
+#   coef[j][k] = r_j (d_jk - r_k)       (the cross block is coef[j][k] (m_k[t] - x_n[t]))
+#   grad_rho_j = r_j delta_j,  obj = abar
+# When one responsibility r_dom is close to 1, B_dom,dom, coef_dom,dom and delta_dom are (1 - r_dom)-small, but
+# these formulas form them as differences of O(1) numbers: in float64 every digit is lost once the gap between the
+# two largest logits passes ~37 (longdouble: ~44).  gmm_blocks_mp evaluates the formulas as written at a precision
+# that absorbs the cancellation; gmm_blocks_stable_ld uses forms that do not cancel.
+# ----------------------------------------------------------------------------------------------------------------
+def _gmm_logits(rho):
+    rho = np.asarray(rho, dtype=np.float64)
+    return np.concatenate([rho, np.zeros((rho.shape[0], 1))], axis=1)
+
+
+def gmm_blocks_mp(X, m, rho, log_pi, rows):
+    """r, grad_rho, obj_terms, blocks and coef of the observations ``rows`` from the definition, in mpmath, each
+    rounded once to float64.  The inputs are taken as the exact float64 values.  The working precision is 50 digits
+    plus what the cancellation of 1 - r_dom costs, (top-two logit gap + log(1 + max|c|)) / ln 10."""
+    X, m, log_pi = (np.asarray(a, dtype=np.float64) for a in (X, m, log_pi))
+    logits = _gmm_logits(rho)
+    K, d = m.shape
+    M = K - 1
+    out = dict(r=np.empty((len(rows), K)), grad_rho=np.empty((len(rows), M)), obj_terms=np.empty(len(rows)),
+               blocks=np.empty((len(rows), M, M)), coef=np.empty((len(rows), M, K)))
+    for i, n in enumerate(rows):
+        top2 = np.sort(logits[n])[-2:]
+        csize = float(np.max(np.abs(0.5 * ((X[n] - m) ** 2).sum(1) - log_pi)))
+        digits = 50 + int((top2[1] - top2[0] + math.log1p(csize)) / math.log(10)) + 1
+        with mpmath.workdps(digits):
+            mpf = mpmath.mpf
+            lg = [mpf(float(v)) for v in logits[n]]
+            mx = max(lg)
+            e = [mpmath.exp(v - mx) for v in lg]
+            tot = mpmath.fsum(e)
+            r = [v / tot for v in e]
+            c = [mpmath.fsum((mpf(float(X[n, t])) - mpf(float(m[k, t]))) ** 2 for t in range(d)) / 2
+                 - mpf(float(log_pi[k])) for k in range(K)]
+            a = [c[k] + (lg[k] - mx - mpmath.log(tot)) for k in range(K)]
+            abar = mpmath.fsum(r[k] * a[k] for k in range(K))
+            dev = [a[k] - abar for k in range(K)]
+            out['r'][i] = [_to_f64(v) for v in r]
+            out['grad_rho'][i] = [_to_f64(r[j] * dev[j]) for j in range(M)]
+            out['obj_terms'][i] = _to_f64(abar)
+            for j in range(M):
+                for l in range(M):
+                    v = -r[j] * r[l] * (dev[j] + dev[l] + 1)
+                    out['blocks'][i, j, l] = _to_f64(v + r[j] * (dev[j] + 1) if j == l else v)
+                for k in range(K):
+                    out['coef'][i, j, k] = _to_f64(r[j] * ((1 if j == k else 0) - r[k]))
+    return out
+
+
+def gmm_blocks_stable_ld(X, m, rho, log_pi):
+    """The same quantities for every observation, in longdouble, in forms that do not cancel (dom = the first
+    largest logit; every sum skips the term that is exactly zero):
+        q_k = 1 - r_k = sum_{i != k} r_i
+        delta_j = sum_i r_i [(c_j - c_i) + (l_j - l_i)]
+        B_jj = r_j q_j + r_j delta_j (q_j - r_j),   B_jl = -r_j r_l (1 + delta_j + delta_l)
+        coef_jk = r_j q_j (j = k),  -r_j r_k (j != k)
+    Longdouble's exponent range also keeps e^-800 normal.  Returns float64 arrays of the outputs of gmm_blocks
+    (coef in place of the cross blocks) and, for the error bars, the longdouble c, logits, q and delta."""
+    X, m, log_pi = (np.asarray(a, dtype=np.float64) for a in (X, m, log_pi))
+    lg = _gmm_logits(rho).astype(LD)
+    N, K = lg.shape
+    M = K - 1
+    off = 1 - np.eye(K, dtype=LD)
+    e = np.exp(lg - lg.max(1, keepdims=True))
+    tot = e.sum(1, keepdims=True)
+    r = e / tot
+    q = (e @ off) / tot
+    c = np.empty((N, K), dtype=LD)
+    for k in range(K):
+        c[:, k] = 0.5 * ((X.astype(LD) - m[k].astype(LD)) ** 2).sum(1) - LD(log_pi[k])
+    diff = (c[:, :, None] - c[:, None, :]) + (lg[:, :, None] - lg[:, None, :])      # [n, j, i] = a_j - a_i
+    delta = np.einsum('ni,nji->nj', r, diff)
+    obj = (r * (c + lg - lg.max(1, keepdims=True) - np.log(tot))).sum(1)
+    rj, qj, dj = r[:, :M], q[:, :M], delta[:, :M]
+    blocks = -(rj[:, :, None] * rj[:, None, :]) * (1 + dj[:, :, None] + dj[:, None, :])
+    idx = np.arange(M)
+    blocks[:, idx, idx] = rj * qj + rj * dj * (qj - rj)
+    coef = -(rj[:, :, None] * r[:, None, :])
+    coef[:, idx, idx] = rj * qj
+    f64 = lambda a: np.asarray(a, dtype=np.float64)                  # noqa: E731
+    return dict(r=f64(r), grad_rho=f64(rj * dj), obj_terms=f64(obj), blocks=f64(blocks), coef=f64(coef),
+                c=c, logits=lg, q=q, delta=delta)
+
+
+GMM_EPS = 2.0 ** -53
+GMM_FLOOR = 2.0 ** -1060
+
+
+def gmm_error_bars(ref, d):
+    """Per-entry error bars for gmm_blocks from a first-order error analysis (eps = 2^-53), given the output of
+    gmm_blocks_stable_ld for data of dimension d:
+        A_n = 1 + max_k |c_k| + max_k |l_k - max l|,   tau_n = 16 (d + K) eps A_n
+        floors phi = 2^-1060,  phi_n = 4 phi A_n
+        r_k: (8K + |l_k - max l|) eps r_k + phi    (exp amplifies the rounding of its argument l_k - max l)
+        grad_rho_j: tau_n r_j q_j + phi_n,   obj: tau_n
+        B_jj: tau_n r_j q_j (1 + |delta_j|) + phi_n,   B_jl: tau_n r_j r_l (1 + |delta_j| + |delta_l|) + phi_n
+        coef_jk: tau_n |coef_jk| + phi_n     (times |m_k[t] - x_n[t]| for the cross block entry (j, k, t))
+    Every bar scales with the entry's own size (r_j q_j, r_j r_l), never with the block's largest entry: a bar
+    relative to max |B| is met by formulas that lose every digit of the (1 - r)-small entries.  Only the floors are
+    absolute: a responsibility that underflowed to a subnormal or 0 is off by up to 2^-1074, and it is multiplied by
+    deviations a_i - a_j of up to 2 A_n.  phi_n stays below 2^-1030, far under every (1 - r) of a gap up to 700."""
+    c, lg = np.asarray(ref['c'], dtype=np.float64), np.asarray(ref['logits'], dtype=np.float64)
+    r, q, dl = (np.asarray(ref[k], dtype=np.float64) for k in ('r', 'q', 'delta'))
+    N, K = r.shape
+    M = K - 1
+    gap = lg.max(1, keepdims=True) - lg
+    A = 1 + np.abs(c).max(1) + gap.max(1)
+    tau = 16 * (d + K) * GMM_EPS * A
+    t2 = tau[:, None, None]
+    rj, qj, dj = r[:, :M], q[:, :M], np.abs(dl[:, :M])
+    phi = 4 * GMM_FLOOR * A
+    assert np.all(phi < 2.0 ** -1030), 'the underflow floor would cover (1 - r)-small entries'
+    p2 = phi[:, None, None]
+    blocks = t2 * (rj[:, :, None] * rj[:, None, :]) * (1 + dj[:, :, None] + dj[:, None, :]) + p2
+    idx = np.arange(M)
+    blocks[:, idx, idx] = tau[:, None] * rj * qj * (1 + dj) + phi[:, None]
+    return dict(r=(8 * K + gap) * GMM_EPS * r + GMM_FLOOR, grad_rho=tau[:, None] * rj * qj + phi[:, None],
+                obj_terms=tau, blocks=blocks, coef=t2 * np.abs(ref['coef']) + p2, tau=tau, floor=phi)
+
+
+def gmm_bar_ratios(got, ref, bars, keys=('r', 'grad_rho', 'obj_terms', 'blocks', 'coef')):
+    """Per observation, max |got - ref| / bar over the entries of each key (NaN in got gives inf)."""
+    out = {}
+    for k in keys:
+        g = np.asarray(got[k], dtype=np.float64)
+        ratio = np.abs(g - ref[k]) / bars[k]
+        ratio = np.where(np.isnan(ratio), np.inf, ratio).reshape(g.shape[0], -1)
+        out[k] = ratio.max(1)
+    return out

@@ -219,21 +219,32 @@ __global__ void colsum_finish_kernel(const double* partial, int ncta, int Dg, do
 }
 
 // -------------------------------------------------------------- GMM-VB ----
-// One CTA per observation.  x = (m (K x d), rho_n (K-1 free logits)):
-//   r = softmax([rho_n, 0]),  a_k = 0.5 |x_n - m_k|^2 - log pi_k + log r_k,  abar = sum r_k a_k
-//   B[j][l] = r_j d_jl (a_j - abar + 1) - r_j r_l ((a_j - abar) + (a_l - abar) + 1)     j,l < K-1
+// One CTA per observation.  x = (m (K x d), rho_n (K-1 free logits)), logits l = [rho_n, 0]:
+//   r = softmax(l),  c_k = 0.5 |x_n - m_k|^2 - log pi_k,  a_k = c_k + log r_k,  abar = sum r_k a_k
+//   q_k = 1 - r_k,  delta_k = a_k - abar
+//   B[j][l] = r_j d_jl (delta_j + 1) - r_j r_l (delta_j + delta_l + 1)                   j,l < K-1
 //   C[j][k*d + t] = r_j (d_jk - r_k) (m_k[t] - x_n[t])                                   j < K-1, k < K
 //   rsum[k] += r_k  (diagonal of the global block; reduced by the caller)
-//   grad_rho[j] = r_j (a_j - abar),  obj = abar
-__global__ void __launch_bounds__(256) gmm_blocks_kernel(const double* __restrict__ X, long N, int d, int K,
+//   grad_rho[j] = r_j delta_j,  obj = abar
+// A fitted mixture with separated clusters has logit gaps of tens to hundreds, so r_dom ~ 1 for the dominant
+// component dom (the lowest lane holding the largest logit), and B_dom,dom, r_dom (1 - r_dom) and delta_dom are
+// (1 - r_dom)-small.  Formed as written they are differences of O(1) numbers (1 - r rounds to 0 past a gap of ~37)
+// and B comes out indefinite.  They are formed instead from sums over the other components, which do not cancel:
+//   q_dom = r_dom sum_{i != dom} e_i  (e_k = e^(l_k - l_dom), r_dom = 1 / tot),  q_k = 1 - r_k for k != dom
+//   (r_k <= 1/2 there),  delta_j = (a_j - a_dom) - sum_{i != dom} r_i (a_i - a_dom),
+//   a_i - a_dom = (c_i - c_dom) + (l_i - l_dom),
+//   B_jj = r_j q_j + r_j delta_j (q_j - r_j),  B_jl = -r_j r_l (delta_j + delta_l + 1),  C coefficient r_j q_j at j = k
+// 8 CTAs per SM (the grid cap of gmm_blocks) need <= 32 registers a thread.
+__global__ void __launch_bounds__(256, 8) gmm_blocks_kernel(const double* __restrict__ X, long N, int d, int K,
                                                          const double* __restrict__ m, const double* __restrict__ rho,
                                                          const double* __restrict__ log_pi, double* blocks,
                                                          double* cross, double* rmat, double* grad_rho,
                                                          double* obj_terms) {
   extern __shared__ double sm[];
-  double* sr = sm;            // K
-  double* sa = sm + K;        // K
-  double* sx = sm + 2 * K;    // d
+  double* sr = sm;            // K: r
+  double* sq = sm + K;        // K: q = 1 - r
+  double* sa = sm + 2 * K;    // K: c, then delta
+  double* sx = sm + 3 * K;    // d
   const int M = K - 1;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (long n = blockIdx.x; n < N; n += gridDim.x) {
@@ -249,27 +260,35 @@ __global__ void __launch_bounds__(256) gmm_blocks_kernel(const double* __restric
     }
     __syncthreads();
     if (warp == 0) {
-      // softmax over [rho, 0] and a_k, by one warp (K <= 32)
-      const double logit = lane < M ? rho[n * M + lane] : (lane == M ? 0.0 : -1e300);
-      double mx = logit;
+      // softmax over [rho, 0], q and delta, by one warp (K <= 32)
+      double z = lane < M ? rho[n * M + lane] : (lane == M ? 0.0 : -1e300);
+      double mx = z;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-      const double e = lane < K ? exp(logit - mx) : 0.0;
+      z -= mx;                                                          // l - l_dom
+      const double e = lane < K ? exp(z) : 0.0;
+      const int dom = __ffs(__ballot_sync(0xffffffffu, z == 0.0)) - 1;
       const double tot = warp_sum(e);
-      const double r = e / tot;
-      const double logr = (logit - mx) - log(tot);
-      const double a = lane < K ? sa[lane] + logr : 0.0;
-      const double abar = warp_sum(lane < K ? r * a : 0.0);
-      if (lane < K) { sr[lane] = r; sa[lane] = a - abar; }
+      const double rest = warp_sum(lane == dom ? 0.0 : e);
+      if (lane < K) { const double r = e / tot; sr[lane] = r; sq[lane] = lane == dom ? rest * r : 1.0 - r; }
+      const double logr = z - log(tot);
+      __syncwarp();
+      const double r = lane < K ? sr[lane] : 0.0;
       if (lane < K && rmat) rmat[n * K + lane] = r;
-      if (lane < M && grad_rho) grad_rho[n * M + lane] = r * (a - abar);
+      const double c = lane < K ? sa[lane] : 0.0;
+      const double abar = warp_sum(r * (c + logr));
+      const double da = (c - __shfl_sync(0xffffffffu, c, dom)) + z;     // a - a_dom
+      const double dev = da - warp_sum(lane != dom ? r * da : 0.0);
+      if (lane < K) sa[lane] = dev;
+      if (lane < M && grad_rho) grad_rho[n * M + lane] = r * dev;
       if (lane == 0 && obj_terms) obj_terms[n] = abar;
     }
     __syncthreads();
     if (blocks) {
       for (int e = threadIdx.x; e < M * M; e += blockDim.x) {
         const int j = e / M, l = e % M;
-        const double v = (j == l ? sr[j] * (sa[j] + 1.0) : 0.0) - sr[j] * sr[l] * (sa[j] + sa[l] + 1.0);
+        const double v = j == l ? sr[j] * sq[j] + sr[j] * sa[j] * (sq[j] - sr[j])
+                                : -sr[j] * sr[l] * (sa[j] + sa[l] + 1.0);
         blocks[n * (long)M * M + e] = v;
       }
     }
@@ -280,8 +299,9 @@ __global__ void __launch_bounds__(256) gmm_blocks_kernel(const double* __restric
       for (int c = threadIdx.x; c < Dg; c += blockDim.x) {
         const int k = c / d, t = c - k * d;
         const double dm = m[(long)k * d + t] - sx[t];
-        const double rk = sr[k];
-        for (int j = 0; j < M; ++j) Cn[(long)j * Dg + c] = sr[j] * ((j == k ? 1.0 : 0.0) - rk) * dm;
+        const double diag = sr[k] * sq[k] * dm, off = -sr[k] * dm;      // r_k q_k dm at j = k, -r_j r_k dm elsewhere
+        double* p = Cn + c;
+        for (int j = 0; j < M; ++j, p += Dg) *p = j == k ? diag : sr[j] * off;
       }
     }
   }
@@ -360,7 +380,7 @@ int gmm_blocks(const double* X, long N, int d, int K, const double* m, const dou
                double* blocks, double* cross, double* rmat, double* grad_rho, double* obj_terms,
                cudaStream_t stream) {
   VT_REQUIRE(X && m && rho && log_pi && N >= 1 && d >= 1 && K >= 2 && K <= 32, "gmm_blocks: need 2 <= K <= 32");
-  const size_t smem = (size_t)(2 * K + d) * 8;
+  const size_t smem = (size_t)(3 * K + d) * 8;
   gmm_blocks_kernel<<<grid_for(N, 1, 8), 256, smem, stream>>>(X, N, d, K, m, rho, log_pi, blocks, cross, rmat,
                                                                grad_rho, obj_terms);
   VT_LAUNCH_CHECK();
