@@ -159,6 +159,30 @@ size_t vt_quad_forms_ozaki_workspace_bytes(int64_t N, int D, int nslices);
 int vt_quad_forms_ozaki(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D, double* out,
                         int nslices, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Leave-one-group-out predictors -----------------------------------------
+ * Groups are runs of consecutive rows: group g is rows starts[g] .. starts[g+1]-1
+ * (starts: G + 1 int64, strictly increasing from 0 to N, consecutive entries at
+ * most 32 apart; the caller checks this).  For a group R, Q = X_R H^{-1} X_R^T
+ * = U_R^T U_R with U = Linv X^T (Linv as for vt_quad_forms), t = Q u_R, and
+ *   h[n]     = Q_nn = x_n^T H^{-1} x_n
+ *   method 0 (IJ):          zpred_R = z_R + t
+ *   method 1 (Newton step): zpred_R = z_R + t + Q S^1/2 M^{-1} S^1/2 t,
+ *                           M = I - S^1/2 Q S^1/2, S = diag(s_R)
+ * NaN on every row of a group when a pivot of the Cholesky factor of M, squared,
+ * is <= 2^-40.  vt_group_loo runs U on the DMMA engine (rows x D per chunk),
+ * vt_group_loo_ozaki on the INT8 slicing engine (the chunks of
+ * vt_ij_apply_ozaki); both then form each group's Q in one kernel.  Chunks
+ * overlap by 32 rows, so no group is split; nothing of size D x N is written.
+ * Both sum in a fixed order: two calls give the same bits.                   */
+size_t vt_group_loo_workspace_bytes(int64_t N, int D);
+int vt_group_loo(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D,
+                 const int64_t* starts, int64_t G, const double* s, const double* u, const double* z, int method,
+                 double* zpred, double* h, void* workspace, size_t workspace_bytes, void* stream);
+size_t vt_group_loo_ozaki_workspace_bytes(int64_t N, int D, int nslices);
+int vt_group_loo_ozaki(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D,
+                       const int64_t* starts, int64_t G, const double* s, const double* u, const double* z, int method,
+                       double* zpred, double* h, int nslices, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- Infinitesimal-jackknife apply ----------------------------------------
  * S (D x N) = -Hinv (D x D) * G^T, column n of G^T being resid[n] * x_n, fused
  * so that the cross-Hessian G^T is never materialised.  Replaces

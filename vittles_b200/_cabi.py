@@ -66,6 +66,10 @@ SIGNATURES = {
     'vt_ij_apply_ozaki': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _P, _I64, _I, _P, _SZ, _P]),
     'vt_quad_forms_ozaki_workspace_bytes': (_SZ, [_I64, _I, _I]),
     'vt_quad_forms_ozaki': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _I, _P, _SZ, _P]),
+    'vt_group_loo_workspace_bytes': (_SZ, [_I64, _I]),
+    'vt_group_loo': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _I64, _P, _P, _P, _I, _P, _P, _P, _SZ, _P]),
+    'vt_group_loo_ozaki_workspace_bytes': (_SZ, [_I64, _I, _I]),
+    'vt_group_loo_ozaki': (_I, [_P, _I64, _P, _I64, _I64, _I, _P, _I64, _P, _P, _P, _I, _P, _P, _I, _P, _SZ, _P]),
     'vt_gemv_workspace_bytes': (_SZ, [_I, _I64]),
     'vt_gemv': (_I, [_P, _I64, _I, _I64, _P, _D, _P, _D, _P, _P, _SZ, _P]),
     'vt_cg_batch_init': (_I, [_I, _I, _P, _P, _P, _P, _D, _D, _I, _P]),

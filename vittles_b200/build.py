@@ -19,7 +19,7 @@ CSRC = os.path.join(PKG, 'csrc')
 LIBDIR = os.path.join(PKG, 'lib')
 LIB = os.path.join(LIBDIR, 'libvittles_b200.so')
 OBJDIR = os.path.join(PKG, 'build')
-SOURCES = ['common.cu', 'dgemm.cu', 'glm.cu', 'chol.cu', 'synth.cu', 'blockchol.cu', 'tgemm.cu', 'ogemm.cu', 'abi.cu']
+SOURCES = ['common.cu', 'dgemm.cu', 'glm.cu', 'chol.cu', 'synth.cu', 'blockchol.cu', 'tgemm.cu', 'ogemm.cu', 'grouploo.cu', 'abi.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC'] + os.environ.get('VT_NVCC_EXTRA', '').split()
 

@@ -306,6 +306,26 @@ int vt_quad_forms_ozaki(const double* Linv, int64_t ldl, const double* X, int64_
   return quad_forms_ozaki(Linv, ldl, X, ldx, N, D, out, nslices, workspace, workspace_bytes, S(stream));
 }
 
+size_t vt_group_loo_workspace_bytes(int64_t N, int D) { return group_loo_workspace_bytes(N, D); }
+
+int vt_group_loo(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D,
+                 const int64_t* starts, int64_t G, const double* s, const double* u, const double* z, int method,
+                 double* zpred, double* h, void* workspace, size_t workspace_bytes, void* stream) {
+  return group_loo(Linv, ldl, X, ldx, N, D, starts, G, s, u, z, method, zpred, h, workspace, workspace_bytes,
+                   S(stream));
+}
+
+size_t vt_group_loo_ozaki_workspace_bytes(int64_t N, int D, int nslices) {
+  return group_loo_ozaki_workspace_bytes(N, D, nslices);
+}
+
+int vt_group_loo_ozaki(const double* Linv, int64_t ldl, const double* X, int64_t ldx, int64_t N, int D,
+                       const int64_t* starts, int64_t G, const double* s, const double* u, const double* z, int method,
+                       double* zpred, double* h, int nslices, void* workspace, size_t workspace_bytes, void* stream) {
+  return group_loo_ozaki(Linv, ldl, X, ldx, N, D, starts, G, s, u, z, method, zpred, h, nslices, workspace,
+                         workspace_bytes, S(stream));
+}
+
 size_t vt_syrk_ozaki_workspace_bytes(int64_t N, int D, int nslices) { return syrk_ozaki_workspace_bytes(N, D, nslices); }
 
 int vt_syrk_ozaki(const double* X, int64_t ldx, int64_t N, int D, const double* s, double l2, double* H, int64_t ldh,

@@ -1,5 +1,6 @@
 // FP64 DMMA GEMM engine - see dgemm.cuh for the design notes.
 #include "dgemm.cuh"
+#include "grouploo.cuh"
 #include <cstdlib>
 
 namespace vt {
@@ -517,6 +518,41 @@ int quad_forms(const double* Linv, long ldl, const double* X, long ldx, long N, 
     if (st != VT_OK) return st;
     row_sumsq_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, stream>>>(U, D, rows, D, out + r0);
     VT_LAUNCH_CHECK();
+  }
+  return VT_OK;
+}
+
+// ---- leave-one-group-out on the DMMA engine ----------------------------------
+size_t group_loo_workspace_bytes(long N, int D) { return quad_forms_workspace_bytes(N, D); }
+
+int group_loo(const double* Linv, long ldl, const double* X, long ldx, long N, int D, const int64_t* starts, long G,
+              const double* s, const double* u, const double* z, int method, double* zpred, double* h, void* workspace,
+              size_t workspace_bytes, cudaStream_t stream) {
+  VT_REQUIRE(Linv && X && starts && s && u && z && zpred && h, "group_loo: null pointer");
+  VT_REQUIRE(D >= 1 && N >= 0 && G >= 0 && G <= N && ldl >= D && ldx >= D, "group_loo: bad shape");
+  VT_REQUIRE(method == GROUP_LOO_IJ || method == GROUP_LOO_NS, "group_loo: method 0 (IJ) or 1 (Newton step)");
+  if (N == 0) return VT_OK;
+  VT_REQUIRE(workspace && workspace_bytes >= group_loo_workspace_bytes(N, D), "group_loo: workspace too small");
+  const long ch = quad_forms_chunk_rows(N, D);
+  VT_REQUIRE(ch == N || ch > GROUP_LOO_OVERLAP, "group_loo: D = %d leaves no room for whole groups in a chunk", D);
+  const long stride = ch - GROUP_LOO_OVERLAP;
+  double* U = static_cast<double*>(workspace);
+  for (long r0 = 0;; r0 += stride) {
+    const long rows = (N - r0 < ch) ? N - r0 : ch;
+    const bool last = r0 + ch >= N;
+    GemmParams p{};                                              // U = X_c Linv^T  (rows x D)
+    p.M = (int)rows; p.N = D; p.K = D;
+    p.A = X + r0 * ldx; p.lda = ldx; p.amode = KC;
+    p.B = Linv; p.ldb = ldl; p.bmode = KC;
+    p.C = U; p.ldc = D;
+    p.alpha = 1.0; p.beta = 0.0;
+    p.parts = 1;
+    int st = gemm_launch(p, stream);
+    if (st != VT_OK) return st;
+    st = group_loo_chunk(GroupLooChunk{U, D, 1, r0, rows, D, starts, G, r0, last ? N : r0 + stride, s, u, z, method,
+                                       zpred, h}, stream);
+    if (st != VT_OK) return st;
+    if (last) break;
   }
   return VT_OK;
 }

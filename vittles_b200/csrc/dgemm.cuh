@@ -70,4 +70,11 @@ size_t quad_forms_workspace_bytes(long N, int D);
 int quad_forms(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, void* workspace,
                size_t workspace_bytes, cudaStream_t stream);
 
+// Leave-one-group-out predictors and h_n (grouploo.cuh) with U = X_c Linv^T per chunk of rows on this engine; the
+// chunks overlap by GROUP_LOO_OVERLAP rows so that every group lies whole in one of them.
+size_t group_loo_workspace_bytes(long N, int D);
+int group_loo(const double* Linv, long ldl, const double* X, long ldx, long N, int D, const int64_t* starts, long G,
+              const double* s, const double* u, const double* z, int method, double* zpred, double* h, void* workspace,
+              size_t workspace_bytes, cudaStream_t stream);
+
 }  // namespace vt

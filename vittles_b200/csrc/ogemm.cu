@@ -1,5 +1,6 @@
 // FP64-grade GEMM on the INT8 tensor cores by error-free slicing - see ogemm.cuh.
 #include "ogemm.cuh"
+#include "grouploo.cuh"
 #include "tc05.cuh"
 #include <cstdlib>
 
@@ -985,8 +986,9 @@ int ogemm_launch(int M, int N, int K, const int8_t* A, long lda, long a_slice_st
 
 namespace {
 // Rows of X (N x D) against a D x D matrix A on the INT8 engine, chunk by chunk: A is sliced once, chunk c of X
-// (ozaki_chunk_rows rows, scale tau_n * fold[n]; fold == nullptr: tau_n) into one of two digit buffers, and
-// product(r0, rows, Bs, tau, o) runs the GEMM of the chunk with the slicing job `o.next` of the chunk after it.
+// (ozaki_chunk_rows rows from row c (ch - overlap), scale tau_n * fold[n]; fold == nullptr: tau_n) into one of two
+// digit buffers, and product(r0, rows, Bs, tau, o) runs the GEMM of the chunk with the slicing job `o.next` of the
+// chunk after it.  The last chunk is the first that reaches row N.
 // Chunk c + 1 is sliced by the converter warps of the GEMM of chunk c (rows of up to 1024 elements; longer rows:
 // a separate slicing launch per chunk).
 struct RowChunks {
@@ -1001,9 +1003,10 @@ struct RowChunks {
 
 template <class Product>
 int ozaki_row_chunks(const double* A, long lda, const double* X, long ldx, long N, int D, const double* fold,
-                     int nslices, void* workspace, cudaStream_t stream, Product&& product) {
+                     int nslices, long overlap, void* workspace, cudaStream_t stream, Product&& product) {
   const RowChunks rc(N, D, nslices);
-  const long ld = rc.ld, ch = rc.ch;
+  const long ld = rc.ld, ch = rc.ch, stride = ch - overlap;
+  VT_REQUIRE(ch == N || stride > 0, "ozaki_row_chunks: chunks of %ld rows cannot overlap by %ld", ch, overlap);
   char* w = static_cast<char*>(workspace);
   int8_t* As = reinterpret_cast<int8_t*>(w);
   w += rc.a_bytes;
@@ -1021,22 +1024,24 @@ int ozaki_row_chunks(const double* A, long lda, const double* X, long ldx, long 
   if (st != VT_OK) return st;
   const bool fuse = D <= 1024;
   long c = 0;
-  for (long r0 = 0; r0 < N; r0 += ch, ++c) {
+  for (long r0 = 0;; r0 += stride, ++c) {
     const int b = (int)(c & 1);
     const long rows = (N - r0 < ch) ? N - r0 : ch;
+    const bool last = r0 + ch >= N;
     if (!fuse || c == 0) {
       st = ozaki_slice(X + r0 * ldx, ldx, rows, D, Bs[b], ld, ch * ld, nslices, tau[b], fold ? fold + r0 : nullptr, stream);
       if (st != VT_OK) return st;
     }
     OLaunchOpts o;
-    const long n0 = r0 + ch;
-    if (fuse && n0 < N) {
+    const long n0 = r0 + stride;
+    if (fuse && !last) {
       const long nrows = (N - n0 < ch) ? N - n0 : ch;
       o.next = SliceJob{X + n0 * ldx, ldx, nrows, D, Bs[b ^ 1], ld, ch * ld, tau[b ^ 1], fold ? fold + n0 : nullptr,
                         nullptr, nullptr};
     }
     st = product(r0, rows, As, sigma, Bs[b], tau[b], ld, ch, o);
     if (st != VT_OK) return st;
+    if (last) break;
   }
   return VT_OK;
 }
@@ -1063,7 +1068,7 @@ int ij_apply_ozaki(const double* Hinv, long ldh, const double* X, long ldx, long
   VT_REQUIRE(workspace_bytes >= ij_apply_ozaki_workspace_bytes(N, D, nslices), "ij_apply_ozaki: workspace too small");
   if (N == 0) return VT_OK;
   // tau_n resid_n: the residual is folded into the column scale
-  return ozaki_row_chunks(Hinv, ldh, X, ldx, N, D, resid, nslices, workspace, stream,
+  return ozaki_row_chunks(Hinv, ldh, X, ldx, N, D, resid, nslices, 0, workspace, stream,
                           [&](long r0, long rows, const int8_t* As, const double* sigma, const int8_t* Bs,
                               const double* tau, long ld, long ch, const OLaunchOpts& o) {
                             return ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs, ld, ch * ld, nslices,
@@ -1087,7 +1092,7 @@ int quad_forms_ozaki(const double* Linv, long ldl, const double* X, long ldx, lo
   const RowChunks rc(N, D, nslices);
   double* P = reinterpret_cast<double*>(static_cast<char*>(workspace) + rc.bytes());    // (4 tiles_m) x ch partials
   const int nparts = 4 * ((D + OBM - 1) / OBM);
-  return ozaki_row_chunks(Linv, ldl, X, ldx, N, D, nullptr, nslices, workspace, stream,
+  return ozaki_row_chunks(Linv, ldl, X, ldx, N, D, nullptr, nslices, 0, workspace, stream,
                           [&](long r0, long rows, const int8_t* As, const double* sigma, const int8_t* Bs,
                               const double* tau, long ld, long ch, OLaunchOpts o) {
                             o.epi = EPI_QUAD;
@@ -1099,6 +1104,37 @@ int quad_forms_ozaki(const double* Linv, long ldl, const double* X, long ldx, lo
                                                                                                           rows, out + r0);
                             VT_LAUNCH_CHECK();
                             return VT_OK;
+                          });
+}
+
+// ---- leave-one-group-out -------------------------------------------------------
+size_t group_loo_ozaki_workspace_bytes(long N, int D, int nslices) {
+  const RowChunks rc(N, D, nslices);
+  return rc.bytes() + align_up((size_t)D * rc.ch * 8, 256);
+}
+
+int group_loo_ozaki(const double* Linv, long ldl, const double* X, long ldx, long N, int D, const int64_t* starts,
+                    long G, const double* s, const double* u, const double* z, int method, double* zpred, double* h,
+                    int nslices, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  VT_REQUIRE(Linv && X && starts && s && u && z && zpred && h && workspace, "group_loo_ozaki: null pointer");
+  VT_REQUIRE(D >= 1 && D <= OZAKI_MAX_K && N >= 0 && G >= 0 && G <= N && ldl >= D && ldx >= D,
+             "group_loo_ozaki: bad shape");
+  VT_REQUIRE(nslices >= OZAKI_MIN_SLICES && nslices <= OZAKI_MAX_SLICES, "group_loo_ozaki: 5, 6 or 7 slices");
+  VT_REQUIRE(method == GROUP_LOO_IJ || method == GROUP_LOO_NS, "group_loo_ozaki: method 0 (IJ) or 1 (Newton step)");
+  VT_REQUIRE(workspace_bytes >= group_loo_ozaki_workspace_bytes(N, D, nslices), "group_loo_ozaki: workspace too small");
+  if (N == 0) return VT_OK;
+  const RowChunks rc(N, D, nslices);
+  double* U = reinterpret_cast<double*>(static_cast<char*>(workspace) + rc.bytes());    // D x ch: U = Linv X_c^T
+  return ozaki_row_chunks(Linv, ldl, X, ldx, N, D, nullptr, nslices, GROUP_LOO_OVERLAP, workspace, stream,
+                          [&](long r0, long rows, const int8_t* As, const double* sigma, const int8_t* Bs,
+                              const double* tau, long ld, long ch, const OLaunchOpts& o) {
+                            int st = ogemm_launch_opts(D, (int)rows, D, As, ld, (long)D * ld, Bs, ld, ch * ld, nslices,
+                                                       1.0, sigma, tau, U, ch, o, stream);
+                            if (st != VT_OK) return st;
+                            const long stride = ch - GROUP_LOO_OVERLAP;
+                            const long hi = (r0 + ch >= N) ? N : r0 + stride;
+                            return group_loo_chunk(GroupLooChunk{U, 1, ch, r0, rows, D, starts, G, r0, hi, s, u, z,
+                                                                 method, zpred, h}, stream);
                           });
 }
 

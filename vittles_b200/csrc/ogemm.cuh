@@ -56,6 +56,14 @@ size_t quad_forms_ozaki_workspace_bytes(long N, int D, int nslices);
 int quad_forms_ozaki(const double* Linv, long ldl, const double* X, long ldx, long N, int D, double* out, int nslices,
                      void* workspace, size_t workspace_bytes, cudaStream_t stream);
 
+// Leave-one-group-out predictors and h_n (grouploo.cuh): per chunk of ij_apply_ozaki rows U = Linv X_c^T (D x ch,
+// stored by the GEMM) over the full K range, then the per-group Gram and solve.  The chunks overlap by
+// GROUP_LOO_OVERLAP rows so that every group lies whole in one of them.
+size_t group_loo_ozaki_workspace_bytes(long N, int D, int nslices);
+int group_loo_ozaki(const double* Linv, long ldl, const double* X, long ldx, long N, int D, const int64_t* starts,
+                    long G, const double* s, const double* u, const double* z, int method, double* zpred, double* h,
+                    int nslices, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 // H (D x D) = X^T diag(s) X (s >= 0) with FP64-grade accuracy on the INT8 tensor cores: per chunk of
 // observations the digits of sqrt(s_n) x_ni are written transposed with one power-of-two scale per
 // feature, the lower tiles of the chunk's Gram matrix run as split-K parts of at most 16384

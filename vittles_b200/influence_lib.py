@@ -20,6 +20,16 @@ on the tensor cores).  With the statistics r_n = b'(z_n) - y_n and s_n = w_n b''
 
 The Newton-step ("ALO") form equals the exact leave-one-out prediction for the Gaussian family.
 
+With ``groups`` (one integer label per row, non-decreasing; a group is one label of at most 32 rows, all on one
+rank), the same methods leave out whole groups.  For the rows R of a group, Q = X_R H^{-1} X_R^T, u = (w r)_R and
+S = diag(s_R) (``ops.group_loo``: the rows of U = L^{-1} X^T as for h_n, then a per-group Gram and solve):
+
+    z_R^IJ = z_R + Q u                                  (X_R of predict_opt_par_without(R))
+    z_R^NS = z_R + t + Q S^1/2 M^{-1} S^1/2 t,  t = Q u,  M = I - S^1/2 Q S^1/2
+
+which is z_R + X_R H_{-R}^{-1} X_R^T u by Woodbury (one Newton step without the group; exact for the Gaussian
+family).  At groups of one row both reduce to the leave-one-out forms.
+
 On top of psi, :meth:`ObservationInfluence.amip` computes the Approximate Maximum Influence Perturbation of
 Broderick, Giordano & Meager: the smallest set of observations whose removal is predicted to move a quantity of
 interest to a target (zero: a sign change), and :meth:`ObservationInfluence.refit` re-optimises without that set to
@@ -195,6 +205,65 @@ def loo_predictor(z, resid, s, w, h, method):
     return torch.where(lev < NS_SINGULAR, z + step / (1.0 - lev), torch.full_like(z, float('nan')))
 
 
+GROUP_MAX_ROWS = ops.GROUP_LOO_MAX_ROWS
+
+
+def group_starts(groups, n_local, group=None, device=None):
+    """(starts, labels): the int64 group starts (G + 1 entries, 0 .. n_local) of this rank's rows and the labels as
+    an int64 tensor (both on the labels' device), from one integer label per local row in any array kind.  Labels must be non-decreasing (a group
+    is one label), no group may have more than GROUP_MAX_ROWS rows, and no label may continue on the next rank: the
+    last label of rank r must be less than the first label of rank r + 1.  One all-gather of each rank's first and
+    last label (and of whether its labels are well formed, so that every rank raises the same ValueError instead of
+    leaving the others in the collective; ``device`` carries it for NCCL)."""
+    err, labels, starts = None, None, None
+    try:
+        lab = groups.detach() if isinstance(groups, torch.Tensor) else torch.as_tensor(np.asarray(groups))
+    except (TypeError, ValueError, RuntimeError) as e:
+        lab, err = None, 'groups cannot be read as integer labels ({})'.format(e)
+    if err is None:
+        if lab.dim() != 1 or lab.numel() != n_local:
+            err = 'groups has shape {}, this rank holds {} observations'.format(tuple(lab.shape), n_local)
+        elif lab.dtype == torch.bool or lab.dtype.is_floating_point or lab.dtype.is_complex:
+            err = 'groups must hold integer labels, not {}'.format(lab.dtype)
+    if err is None:
+        labels = lab.to(dtype=torch.int64)
+        step = labels[1:] - labels[:-1]
+        if bool((step < 0).any()):
+            err = 'group labels must be non-decreasing (each group a run of consecutive rows)'
+        else:
+            cut = torch.nonzero(step).reshape(-1) + 1
+            ends = [cut, torch.full((1,), n_local, dtype=torch.int64, device=labels.device)] if n_local else []
+            starts = torch.cat([torch.zeros(1, dtype=torch.int64, device=labels.device)] + ends)
+            size = starts[1:] - starts[:-1]
+            if size.numel() and int(size.max()) > GROUP_MAX_ROWS:
+                g = int(torch.argmax(size))
+                err = 'group {} has {} rows; at most {} are supported'.format(int(labels[starts[g]]), int(size[g]),
+                                                                             GROUP_MAX_ROWS)
+    if _world(group) > 1:
+        dev = device if _nccl(group) else None
+        mine = torch.tensor([err is None, n_local > 0 if err is None else 0,
+                             int(labels[0]) if err is None and n_local else 0,
+                             int(labels[-1]) if err is None and n_local else 0], dtype=torch.int64, device=dev)
+        every = [t.cpu().tolist() for t in _all_gather(mine, group)]
+        if err is None:
+            bad = [r for r, e in enumerate(every) if not e[0]]
+            if bad:
+                err = 'the group labels of rank(s) {} are malformed'.format(bad)
+        if err is None:
+            prev = None
+            for r, (_, nonempty, first, last) in enumerate(every):
+                if not nonempty:
+                    continue
+                if prev is not None and not prev[1] < first:
+                    err = ('group {} straddles ranks {} and {}: a group must lie on one rank (labels increasing '
+                           'across ranks)'.format(first, prev[0], r))
+                    break
+                prev = (r, last)
+    if err is not None:
+        raise ValueError(err)
+    return starts, labels
+
+
 def glm_loss(z, y, family):
     """The family's negative log-likelihood of y at the linear predictor z, up to terms in y only."""
     if family == 'logistic':
@@ -367,31 +436,65 @@ class ObservationInfluence:
         st = self._stats
         return loo_predictor(st['z'], st['resid'], st['s'], self._w, self._quad_forms(), method)
 
+    def _group_loo(self, method, groups):
+        """(z, h, labels) of leaving out each group; the labels are checked (:func:`group_starts`) before any
+        device work.  The engine follows the objective's precision as for :meth:`_quad_forms`."""
+        group = self._obj.group
+        starts, labels = group_starts(groups, self._obj.n_obs, group, self._obj.device if _nccl(group) else None)
+        dev = self._obj.X.device
+        starts, labels = starts.to(dev), labels.to(dev)
+        precision = self._obj.precision
+        if precision in ('tf32', 'tf32x3'):
+            precision = 'auto'
+        self._obj._wait_resident()
+        Linv = self.factor.inverse_factor()
+        st = self._stats
+        z, h = ops.group_loo(Linv, self._obj.X, starts, st['s'], self._w * st['resid'], st['z'], method,
+                             precision=precision)
+        del Linv
+        return z, h, labels
+
     def leverage(self):
         """s_n h_n (the diagonal of the GLM hat matrix) for this rank's observations, shape (N_local,)."""
         return as_kind(self._stats['s'] * self._quad_forms(), self._kind)
 
-    def loo_linear_predictor(self, method='ns'):
+    def loo_linear_predictor(self, method='ns', groups=None):
         """The approximate leave-one-out linear predictor x_n^T theta_hat_{-n} of this rank's rows, (N_local,):
         'ns' one Newton step without row n (NaN, with a UserWarning, where that step is not defined), 'ij' the
-        infinitesimal jackknife x_n^T predict_opt_par_without([n])."""
+        infinitesimal jackknife x_n^T predict_opt_par_without([n]).  With ``groups`` (one integer label per local
+        row, see :func:`group_starts`), row n's predictor leaves out its whole group instead."""
         check_loo_method(method)
-        z = self._loo(method)
+        if groups is None:
+            z = self._loo(method)
+            if method == 'ns':
+                _warn_invalid(int(torch.isnan(z).sum()))
+            return as_kind(z, self._kind)
+        z, _, labels = self._group_loo(method, groups)
         if method == 'ns':
-            _warn_invalid(int(torch.isnan(z).sum()))
+            _warn_invalid_groups(int(torch.isnan(z).sum()), labels[torch.isnan(z)])
         return as_kind(z, self._kind)
 
-    def approximate_cv(self, method='ns'):
+    def approximate_cv(self, method='ns', groups=None):
         """Approximate leave-one-out cross-validation: the held-out loss of every observation at its approximate
-        leave-one-out prediction, and their weighted mean over all ranks (:class:`ApproximateCVResult`)."""
+        leave-one-out prediction, and their weighted mean over all ranks (:class:`ApproximateCVResult`).  With
+        ``groups`` (one integer label per local row, non-decreasing, groups of at most 32 rows on one rank; see
+        :func:`group_starts`), leave-one-group-out: each row is predicted without its whole group, and
+        ``n_invalid`` counts the rows of the groups whose Newton step is not defined."""
         check_loo_method(method)
-        z = self._loo(method)
+        if groups is None:
+            z = self._loo(method)
+            h = self._quad_forms()
+        else:
+            z, h, labels = self._group_loo(method, groups)
         loss = glm_loss(z, self._obj.y, self._obj.family)
         invalid = torch.isnan(z) if method == 'ns' else torch.zeros_like(z, dtype=torch.bool)
         mean_loss, n_invalid = cv_totals(loss, self._w, invalid, self._obj.group)
-        _warn_invalid(n_invalid)
+        if groups is None:
+            _warn_invalid(n_invalid)
+        else:
+            _warn_invalid_groups(n_invalid, labels[invalid])
         return ApproximateCVResult(method=method, z_loo=as_kind(z, self._kind), loss=as_kind(loss, self._kind),
-                                   leverage=as_kind(self._stats['s'] * self._quad_forms(), self._kind),
+                                   leverage=as_kind(self._stats['s'] * h, self._kind),
                                    mean_loss=mean_loss, n_invalid=n_invalid)
 
     # -- AMIP -----------------------------------------------------------------
@@ -426,6 +529,17 @@ def _warn_invalid(n):
         warnings.warn('approximate leave-one-out: the Newton step is not defined for {} observation(s) (s_n h_n >= '
                       '1 - 2^-40: the Hessian without the row is singular); their prediction and loss are NaN and they '
                       'are left out of mean_loss'.format(n), UserWarning)
+
+
+def _warn_invalid_groups(n, labels):
+    """n rows over all ranks without a prediction; ``labels`` of this rank's such rows name the groups."""
+    if n:
+        names = torch.unique(labels).cpu().tolist()
+        shown = ', '.join(str(v) for v in names[:10]) + (', ...' if len(names) > 10 else '')
+        warnings.warn('approximate leave-one-group-out: the Newton step is not defined for {} observation(s) (the '
+                      'Hessian without the group is singular to working accuracy: a squared Cholesky pivot of '
+                      'I - S^1/2 Q S^1/2 <= 2^-40); their prediction and loss are NaN and they are left out of '
+                      'mean_loss.  Groups on this rank: {}'.format(n, shown or 'none'), UserWarning)
 
 
 def _nccl(group):

@@ -567,6 +567,58 @@ def quad_forms(Linv, X, precision='auto', out=None):
     return out
 
 
+# ------------------------------------------------------ leave one group out ----
+GROUP_LOO_MAX_ROWS = 32
+GROUP_LOO_METHODS = {'ij': 0, 'ns': 1}
+
+
+def group_loo(Linv, X, starts, s, u, z, method, precision='auto'):
+    """(zpred, h), both (N,), for groups of consecutive rows: group g is rows starts[g] .. starts[g+1]-1 (``starts``
+    an int64 CUDA tensor of G + 1 entries, strictly increasing from 0 to N, at most 32 apart).  With Q = X_R L^{-T}
+    L^{-1} X_R^T for the rows R of a group (``Linv`` = L^{-1}, lower triangular), t = Q u_R:
+
+        h_n = Q_nn;  'ij': zpred_R = z_R + t;  'ns': zpred_R = z_R + t + Q S^1/2 M^{-1} S^1/2 t,  M = I - S^1/2 Q S^1/2
+
+    (S = diag(s_R)); 'ns' is NaN on every row of a group whose M has a squared Cholesky pivot <= 2^-40.
+    ``precision``: 'f64' (DMMA engine), 'f64_ozaki' (INT8 error-free slicing) or 'auto' (as ``quad_forms``).
+    Everything is checked before any launch."""
+    lib = _cabi.require_cuda()
+    _mat(Linv, 'Linv'); _mat(X, 'X')
+    N, D = X.shape
+    if method not in GROUP_LOO_METHODS:
+        raise ValueError("group_loo: method must be 'ns' or 'ij', not {!r}".format(method))
+    if precision in ('tf32', 'tf32x3'):
+        raise ValueError("group_loo: precision {!r} is not offered; use 'auto', 'f64' or 'f64_ozaki'".format(precision))
+    precision = resolve_precision(precision, N, D)
+    if tuple(Linv.shape) != (D, D):
+        raise ValueError('Linv must have shape ({}, {}), got {}'.format(D, D, tuple(Linv.shape)))
+    if bool(torch.triu(Linv, diagonal=1).any()):
+        raise ValueError('Linv must be lower triangular (zero above the diagonal)')
+    if (not isinstance(starts, torch.Tensor) or not starts.is_cuda or starts.dtype != torch.int64 or starts.dim() != 1
+            or starts.numel() < 1):
+        raise TypeError('starts must be a 1-d int64 CUDA tensor of G + 1 group starts')
+    starts = starts.contiguous()
+    size = starts[1:] - starts[:-1]
+    if int(starts[0]) != 0 or int(starts[-1]) != N:
+        raise ValueError('starts must begin at 0 and end at N = {}'.format(N))
+    if size.numel() and (bool((size <= 0).any()) or int(size.max()) > GROUP_LOO_MAX_ROWS):
+        raise ValueError('starts must be strictly increasing, with groups of at most {} rows'.format(
+            GROUP_LOO_MAX_ROWS))
+    s, u, z = (_vec(v, name, N) for v, name in ((s, 's'), (u, 'u'), (z, 'z')))
+    zpred = torch.empty(N, dtype=torch.float64, device=X.device)
+    h = torch.empty(N, dtype=torch.float64, device=X.device)
+    G = starts.numel() - 1
+    args = (ptr(Linv), _ld(Linv), ptr(X), _ld(X), N, D, ptr(starts), G, ptr(s), ptr(u), ptr(z),
+            GROUP_LOO_METHODS[method], ptr(zpred), ptr(h))
+    if precision == 'f64_ozaki':
+        ws, wsb = _ws('glo_ozaki', lib.vt_group_loo_ozaki_workspace_bytes(N, D, OZAKI_SLICES), X.device)
+        check(lib.vt_group_loo_ozaki(*args, OZAKI_SLICES, ptr(ws), wsb, stream()))
+    else:
+        ws, wsb = _ws('glo', lib.vt_group_loo_workspace_bytes(N, D), X.device)
+        check(lib.vt_group_loo(*args, ptr(ws), wsb, stream()))
+    return zpred, h
+
+
 def gemv(A, x, alpha=1.0, y0=None, beta=1.0):
     """alpha * A @ x + beta * y0 for a row-major (M, N) matrix with N long."""
     lib = _cabi.require_cuda()
@@ -779,7 +831,7 @@ def _device_scoped(fn):
 
 
 for _name in ('gemm', 'tf32_convert', 'tf32_gemm', 'ozaki_slice', 'ozaki_gemm', 'syrk_weighted', 'glm_stats', 'glm_hvp',
-              'glm_hvp_multi', 'glm_dirderiv', 'glm_influence', 'potrf', 'ij_apply', 'quad_forms', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
+              'glm_hvp_multi', 'glm_dirderiv', 'glm_influence', 'potrf', 'ij_apply', 'quad_forms', 'group_loo', 'gemv', 'cg_batch_init', 'cg_batch_update_p', 'cg_batch_update_xr',
               'synth_design',
               'synth_theta', 'synth_bernoulli', 'block_potrf', 'block_trsm', 'block_solve', 'tall_gemv', 'tall_colsum',
               'gmm_blocks'):
