@@ -344,7 +344,7 @@ __global__ void __launch_bounds__(256) tf32_convert_kernel(const double* __restr
     }
     if (rowscale) {
       double sc = rowscale[r];
-      if (sqrt_scale) sc = sqrt(sc > 0.0 ? sc : 0.0);
+      if (sqrt_scale) sc = (sc == sc) ? sqrt(fmax(sc, 0.0)) : sc;     // a NaN weight stays NaN (fmax would drop it)
 #pragma unroll
       for (int j = 0; j < 4; ++j) x[j] *= sc;
     }
@@ -586,11 +586,14 @@ int tf32_convert(const double* X, long ldx, long rows, int cols, const double* r
 }
 
 // ---- S = -Hinv diag(resid) X^T --------------------------------------------
+// Workspace: Hinv hi [lo], one chunk of X hi [lo], and - once D > 4096 (more than one FP32 accumulation segment
+// along k = D) - the FP64 partial tiles of one chunk's GEMM.
 size_t ij_apply_tf32_workspace_bytes(long N, int D, int split) {
   const long ld = (D + 3) / 4 * 4;
   const int nops = split == 3 ? 2 : 1;
   const long ch = chunk_rows(N, D, split, split == 3 ? CfgT3::BN : CfgT1::BN, (D + TBM - 1) / TBM);
-  return align_up((size_t)D * ld * 4, 256) * nops + align_up((size_t)ch * ld * 4, 256) * nops;
+  return align_up((size_t)D * ld * 4, 256) * nops + align_up((size_t)ch * ld * 4, 256) * nops +
+         ws_bytes_for(D, (int)ch, D, split, 0, 1);
 }
 
 int ij_apply_tf32(const double* Hinv, long ldh, const double* X, long ldx, long N, int D, const double* resid,
@@ -609,6 +612,8 @@ int ij_apply_tf32(const double* Hinv, long ldh, const double* X, long ldx, long 
   float* Hl = nops == 2 ? reinterpret_cast<float*>(w + hbytes) : nullptr;
   float* Xh = reinterpret_cast<float*>(w + hbytes * nops);
   float* Xl = nops == 2 ? reinterpret_cast<float*>(w + hbytes * nops + xbytes) : nullptr;
+  double* ws = reinterpret_cast<double*>(w + (hbytes + xbytes) * nops);
+  const size_t ws_bytes = ws_bytes_for(D, (int)ch, D, split, 0, 1);
   int st = tf32_convert(Hinv, ldh, D, D, nullptr, 0, Hh, Hl, ld, stream);
   if (st != VT_OK) return st;
   for (long r0 = 0; r0 < N; r0 += ch) {
@@ -624,6 +629,8 @@ int ij_apply_tf32(const double* Hinv, long ldh, const double* X, long ldx, long 
     p.colscale = resid + r0;
     p.rowscale = nullptr;
     p.parts = 1;
+    p.workspace = ws_bytes ? ws : nullptr;
+    p.workspace_bytes = ws_bytes;
     st = tgemm_launch(p, stream);
     if (st != VT_OK) return st;
   }
